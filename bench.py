@@ -453,6 +453,24 @@ def leg_cli(cols, rank, world, local_rank, torch, n_files=4):
     return out
 
 
+DUMP_LIMIT = 64 << 20
+DUMP_SAMPLE = 1 << 21
+
+
+def dump_outputs(outdir: str, arrays: dict) -> None:
+    """Writes each 1-D float64 device tensor as outdir/<name>.npy.  When the arrays together exceed DUMP_LIMIT bytes, each one is
+    cut to DUMP_SAMPLE positions drawn (sorted, without replacement) from a generator seeded with 0, so that two runs with the same
+    arguments write the same positions and can be compared element for element."""
+    import torch
+    os.makedirs(outdir, exist_ok=True)
+    full = sum(a.numel() * a.element_size() for a in arrays.values()) <= DUMP_LIMIT
+    for name, a in arrays.items():
+        if not full and a.numel() > DUMP_SAMPLE:
+            idx = np.sort(np.random.default_rng(0).choice(a.numel(), DUMP_SAMPLE, replace=False))
+            a = a[torch.from_numpy(idx).to(a.device)]
+        np.save(os.path.join(outdir, name + ".npy"), a.cpu().numpy().astype(np.float64))
+
+
 # ------------------------------------------------------------------------------------------------ main
 def main():
     ap = argparse.ArgumentParser()
@@ -473,7 +491,12 @@ def main():
     ap.add_argument("--precision", default="tc5", choices=["f64", "tc5"],
                     help="tc5: tcgen05/TMEM split-TF32 path (fastest path inside the 1e-3 deciban contract); "
                          "f64: FP64 DMMA path (parity anchor, byte-identical wig text)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write what the last timed step computed on rank 0 (plus / minus decibans per window, bls per column) as "
+                         "DIR/<name>.npy, float64; above 64 MiB in all, the same seeded sample of positions of every array")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the b200 arm")
 
     # stdout carries exactly one JSON line: libraries that write to fd 1 (NCCL prints its version banner there at
     # communicator creation) are sent to stderr instead
@@ -594,6 +617,8 @@ def main():
     ms_max = float(t_ms.item())
     value = world * B * args.steps / (ms_max / 1e3)
     checksum = float(plus[::4097].sum().item() + minus[::4099].sum().item() + bls[::4111].sum().item())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"plus": plus, "minus": minus, "bls": bls})
 
     # ---- e2e through the host-buffer C-ABI call (pinned host memory, H2D + D2H inside the timed region)
     h_seqs = torch.empty((nl, ld), dtype=torch.uint8, pin_memory=True)

@@ -1,15 +1,21 @@
 """The reference itself as the checker.
 
-oracle/_ref/phylocsf_ref is the reference's UNMODIFIED build-tracks / score-msa compiled where the sources lie under
-/root/reference with oracle/ref/gsl standing in for the absent GSL (oracle/ref/Makefile).  Three layers:
+oracle/_ref/phylocsf_ref is the reference's UNMODIFIED build-tracks / score-msa compiled where the sources lie in a PhyloCSF++
+checkout with oracle/ref/gsl standing in for the absent GSL (oracle/ref/Makefile).  Three layers:
 
   1. (CPU, needs the binary) the shim-built reference reproduces the reference's own golden files -> the shim is sound;
   2. (CPU) the oracle restatement + the Python reader mirror reproduce what the reference wrote for the synthetic inputs of
      tests/golden/ref-generated/ (made by tests/golden/make_ref_fixtures.py): a chain crossing the 1 Mb breakpoint, holes,
      reference gaps, unknown species, --species reduction, single-block alignments;
   3. (GPU) the product (C++ host over the C-ABI over the CUDA kernels) reproduces the same files.
+
+The differential runs (4.) feed fresh synthetic MAFs to the oracle and to the product and compare what they write with what the
+reference binary writes for the same input, stored as sha256 digests in tests/golden/ref-generated/digests.json
+(tests/golden/make_ref_digests.py), so that they need no binary outside the repository.
 """
 import gzip
+import hashlib
+import json
 import os
 import shutil
 import subprocess
@@ -27,6 +33,7 @@ from tests.util import read_lines
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 REF = os.path.join(ROOT, "oracle", "_ref", "phylocsf_ref")
 BIN = os.path.join(ROOT, "phylocsfpp_b200", "bin", "phylocsf_b200")
+DIGESTS = os.path.join(ROOT, "tests", "golden", "ref-generated", "digests.json")
 SPECIES29 = "Human,Chimp,Mouse,Dog,Cow,Horse,Elephant,Armadillo,Rat,Rabbit,Cat,Megabat"
 WIGS = ["PhyloCSFpower.wig"] + [f"PhyloCSFRaw{s}{f}.wig" for s in "+-" for f in (1, 2, 3)]
 
@@ -43,7 +50,17 @@ def _rows(path):
 
 def _need_ref():
     if not os.path.exists(REF):
-        pytest.skip("oracle/_ref/phylocsf_ref not built (needs /root/reference; `make -C oracle/ref`)")
+        pytest.skip("oracle/_ref/phylocsf_ref not built (needs the reference's sources: `make -C oracle/ref REF=<PhyloCSF++ checkout>`)")
+
+
+def _sha(data: bytes) -> str:
+    return hashlib.sha256(data).hexdigest()
+
+
+def _ref_digest(group: str, key: str):
+    """What the reference binary wrote for one input: sha256 per output (tests/golden/make_ref_digests.py)."""
+    with open(DIGESTS) as fh:
+        return json.load(fh)[group][key]
 
 
 # ------------------------------------------------------------------------------------------------ 1. the shim is sound
@@ -254,36 +271,47 @@ def _oracle_build_tracks(model_name, maf, threshold=0.1, species=""):
     return out
 
 
-@pytest.mark.parametrize("model_name,cols,seed,extra", [("7yeast", 2500, 21, []), ("20flies", 1800, 22, []),
-                                                        ("12flies", 2200, 23, ["--power-threshold", "1"]),
-                                                        ("12flies", 2200, 24, ["--power-threshold", "0.5"]),
-                                                        ("29mammals", 900, 25, ["--species", SPECIES29])])
-def test_differential_build_tracks_oracle_vs_reference_binary(tmp_path, model_name, cols, seed, extra):
-    """Fresh synthetic MAFs (holes, reference gaps, unknown species) through the reference binary and through the oracle + reader
-    mirror: byte-identical wig files.  Includes the --power-threshold quirk (read with get_bool, build_tracks.hpp:416-417: "1" gives 1.0,
-    anything else 0.0) and a --species reduction."""
-    _need_ref()
-    import sys
-    sys.path.insert(0, os.path.join(ROOT, "tools"))
-    os.environ["PCSF_SYNTH_CPU"] = "1"
-    from make_synth_maf import write_synth_maf
-    maf = os.path.join(str(tmp_path), "d.maf")
-    write_synth_maf(maf, load_model(model_name), cols, seed=seed, mean_block=70, hole_p=1 / 15.0, ref_gap=0.03, alien_p=0.1)
-    out = os.path.join(str(tmp_path), "ref")
-    subprocess.run([REF, "build-tracks", "--threads", "4", "--output", out] + extra + [model_name, maf], check=True,
-                   stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
+def oracle_build_tracks_for(model_name, maf, extra):
+    """_oracle_build_tracks with the options of a build-tracks command line: dict file name -> file contents (bytes)."""
     threshold = 0.1
     species = ""
     if "--power-threshold" in extra:
         threshold = 1.0 if extra[extra.index("--power-threshold") + 1] in ("1", "true", "one") else 0.0
     if "--species" in extra:
         species = extra[extra.index("--species") + 1]
-    ours = _oracle_build_tracks(model_name, maf, threshold, species)
+    return {n: "".join(ln + "\n" for ln in lines).encode() for n, lines in _oracle_build_tracks(model_name, maf, threshold, species).items()}
+
+
+def write_differential_maf(kind, path, model_name, cols, seed):
+    """The synthetic MAF of one differential case (CPU generator: the same bytes on every machine)."""
+    import sys
+    sys.path.insert(0, os.path.join(ROOT, "tools"))
+    os.environ["PCSF_SYNTH_CPU"] = "1"
+    from make_synth_maf import write_synth_maf
+    kw = {"oracle": dict(mean_block=70, hole_p=1 / 15.0, ref_gap=0.03, alien_p=0.1),
+          "cli": dict(mean_block=80, hole_p=1 / 20.0, ref_gap=0.03, alien_p=0.1),
+          "acceptance": dict(mean_block=120, hole_p=1 / 40.0, ref_gap=0.02, alien_p=0.05, start0=1000000 - cols // 2)}[kind]
+    write_synth_maf(path, load_model(model_name), cols, seed=seed, **kw)
+
+
+ORACLE_CASES = [("7yeast", 2500, 21, []), ("20flies", 1800, 22, []), ("12flies", 2200, 23, ["--power-threshold", "1"]),
+                ("12flies", 2200, 24, ["--power-threshold", "0.5"]), ("29mammals", 900, 25, ["--species", SPECIES29])]
+CLI_CASES = [("20flies", 6000, 41, []), ("53birds", 4000, 42, ["--power-threshold", "1"]), ("29mammals", 5000, 43, ["--species", SPECIES29])]
+ACCEPTANCE_CASES = [("58mammals", 60000, 51), ("100vertebrates", 50000, 52)]
+MODEL_INFO_MODELS = ["100vertebrates", "53birds", "23flies", "7yeast"]
+
+
+@pytest.mark.parametrize("model_name,cols,seed,extra", ORACLE_CASES)
+def test_differential_build_tracks_oracle_vs_reference_binary(tmp_path, model_name, cols, seed, extra):
+    """Fresh synthetic MAFs (holes, reference gaps, unknown species) through the oracle + reader mirror: byte for byte the wig files
+    the reference binary writes for them.  Includes the --power-threshold quirk (read with get_bool, build_tracks.hpp:416-417: "1"
+    gives 1.0, anything else 0.0) and a --species reduction."""
+    maf = os.path.join(str(tmp_path), "d.maf")
+    write_differential_maf("oracle", maf, model_name, cols, seed)
+    ours = oracle_build_tracks_for(model_name, maf, extra)
+    gold = _ref_digest("build_tracks", f"{model_name}-{seed}")
     for n in WIGS:
-        ref_lines = open(os.path.join(out, n)).read().split("\n")
-        if ref_lines and ref_lines[-1] == "":
-            ref_lines.pop()
-        assert ours[n] == ref_lines, n
+        assert _sha(ours[n]) == gold[n], n
 
 
 @pytest.mark.parametrize("model_name,seed", [("7yeast", 31), ("12flies", 32)])
@@ -322,24 +350,17 @@ def test_differential_score_msa_oracle_vs_reference_binary(tmp_path, model_name,
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("model_name,cols,seed,extra", [("20flies", 6000, 41, []), ("53birds", 4000, 42, ["--power-threshold", "1"]),
-                                                        ("29mammals", 5000, 43, ["--species", SPECIES29])])
+@pytest.mark.parametrize("model_name,cols,seed,extra", CLI_CASES)
 def test_differential_cli_vs_reference_binary(tmp_path, model_name, cols, seed, extra):
-    """The product's command line and the reference binary side by side on a fresh synthetic MAF (the binary travels to the GPU box
-    with the repository snapshot): seven wig files byte-identical on the FP64 path."""
-    _need_ref()
-    import sys
-    sys.path.insert(0, os.path.join(ROOT, "tools"))
-    os.environ["PCSF_SYNTH_CPU"] = "1"
-    from make_synth_maf import write_synth_maf
+    """The product's command line on a fresh synthetic MAF: on the FP64 path, byte for byte the seven wig files the reference binary
+    writes for it."""
     maf = os.path.join(str(tmp_path), "d.maf")
-    write_synth_maf(maf, load_model(model_name), cols, seed=seed, mean_block=80, hole_p=1 / 20.0, ref_gap=0.03, alien_p=0.1)
-    ref_out, our_out = os.path.join(str(tmp_path), "ref"), os.path.join(str(tmp_path), "ours")
-    subprocess.run([REF, "build-tracks", "--threads", "8", "--output", ref_out] + extra + [model_name, maf], check=True,
-                   stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
+    write_differential_maf("cli", maf, model_name, cols, seed)
+    our_out = os.path.join(str(tmp_path), "ours")
     subprocess.run([BIN, "build-tracks", "--threads", "3", "--output", our_out] + extra + [model_name, maf], check=True, capture_output=True)
+    gold = _ref_digest("build_tracks", f"{model_name}-{seed}")
     for n in WIGS:
-        assert open(os.path.join(our_out, n), "rb").read() == open(os.path.join(ref_out, n), "rb").read(), n
+        assert _sha(open(os.path.join(our_out, n), "rb").read()) == gold[n], n
 
 
 def test_differential_omega_oracle_vs_reference_binary(tmp_path):
@@ -368,14 +389,13 @@ def test_differential_omega_oracle_vs_reference_binary(tmp_path):
     assert sorted(d)[len(d) // 2] <= 0.02, d
 
 
-@pytest.mark.parametrize("model_name", ["100vertebrates", "53birds", "23flies", "7yeast"])
+@pytest.mark.parametrize("model_name", MODEL_INFO_MODELS)
 def test_model_info_matches_reference_binary(model_name):
-    """--model-info (run.hpp:213-232): species and alternative names, identical text from both tools and both sub-commands."""
-    _need_ref()
+    """--model-info (run.hpp:213-232): species and alternative names, the text the reference binary writes, from both sub-commands."""
     for tool in ("build-tracks", "score-msa"):
         ours = subprocess.run([BIN, tool, "--model-info", model_name], capture_output=True, text=True, check=True).stdout
-        ref = subprocess.run([REF, tool, "--model-info", model_name], capture_output=True, text=True, check=True).stdout
-        assert ours == ref and model_name in ours and len(ours.splitlines()) > 5
+        assert _sha(ours.encode()) == _ref_digest("model_info", f"{tool} {model_name}")
+        assert model_name in ours and len(ours.splitlines()) > 5
 
 
 def _wig_values(path):
@@ -391,28 +411,21 @@ def _wig_values(path):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("model_name,cols,seed", [("58mammals", 60000, 51), ("100vertebrates", 50000, 52)])
+@pytest.mark.parametrize("model_name,cols,seed", ACCEPTANCE_CASES)
 def test_acceptance_baseline_models_vs_reference_binary(tmp_path, model_name, cols, seed):
     """North-star acceptance at BASELINE model size: build-tracks of the product against what the reference binary itself writes
     for the same synthetic MAF (58mammals = config 3's model, 100vertebrates = config 4's; holes, reference gaps, unknown species
-    and a chain through the 1 Mb breakpoint).  FP64 path: seven wig files byte-identical.  tcgen05 path: identical fixedStep
-    headers at identical line numbers (gap / missing-species handling and wig positions are bit-exact), power track identical,
-    every PhyloCSF value within 1e-3 decibans (one unit of the last printed digit)."""
-    _need_ref()
-    import sys
-    sys.path.insert(0, os.path.join(ROOT, "tools"))
-    os.environ["PCSF_SYNTH_CPU"] = "1"
-    from make_synth_maf import write_synth_maf
+    and a chain through the 1 Mb breakpoint).  FP64 path: seven wig files byte-identical.  tcgen05 path, against those same files:
+    identical fixedStep headers at identical line numbers (gap / missing-species handling and wig positions are bit-exact), power
+    track identical, every PhyloCSF value within 1e-3 decibans (one unit of the last printed digit)."""
     maf = os.path.join(str(tmp_path), "acc.maf")
-    write_synth_maf(maf, load_model(model_name), cols, seed=seed, mean_block=120, hole_p=1 / 40.0, ref_gap=0.02, alien_p=0.05,
-                    start0=1000000 - cols // 2)
-    ref_out = os.path.join(str(tmp_path), "ref")
-    subprocess.run([REF, "build-tracks", "--threads", str(os.cpu_count() or 8), "--output", ref_out, model_name, maf], check=True,
-                   stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
+    write_differential_maf("acceptance", maf, model_name, cols, seed)
     out64 = os.path.join(str(tmp_path), "f64")
     subprocess.run([BIN, "build-tracks", "--threads", "4", "--output", out64, model_name, maf], check=True, capture_output=True)
+    gold = _ref_digest("build_tracks", f"{model_name}-{seed}")
     for n in WIGS:
-        assert open(os.path.join(out64, n), "rb").read() == open(os.path.join(ref_out, n), "rb").read(), n
+        assert _sha(open(os.path.join(out64, n), "rb").read()) == gold[n], n
+    ref_out = out64                 # byte for byte what the reference writes (checked just above)
     out5 = os.path.join(str(tmp_path), "tc5")
     subprocess.run([BIN, "build-tracks", "--threads", "4", "--precision", "tc5", "--output", out5, model_name, maf], check=True,
                    capture_output=True)
