@@ -151,6 +151,41 @@ typedef enum { PCSF_STRATEGY_MLE = 0, PCSF_STRATEGY_FIXED = 1, PCSF_STRATEGY_OME
 pcsf_status pcsf_score_msa(pcsf_model *m, pcsf_strategy strategy, int32_t n_aln, const uint8_t *seqs,
                            const int64_t *offset, const int64_t *len, float *phylo, float *anc, float *bls);
 
+/* ---- six-frame / open-reading-frame scoring (score-msa --frames, --orf) --------------------------- */
+
+typedef enum { PCSF_ORF_ASIS = 0, PCSF_ORF_STOPSTOP = 1, PCSF_ORF_ATGSTOP = 2 } pcsf_orf_mode;
+
+/* One scored region.  strand +1/-1 and frame 1..3 name the reading frame (0 and 0: the "none" record of an alignment without a
+ * region in best-only mode, with columns -1 and NaN scores).  [col_begin, col_end) are columns of the input alignment; codons counts
+ * the region's full codons (for PCSF_ORF_ATGSTOP / STOPSTOP including the closing stop). */
+typedef struct {
+    int32_t aln;
+    int8_t strand;
+    int8_t frame;
+    int16_t pad;
+    int64_t col_begin, col_end, codons;
+    float phylo, anc, bls;
+} pcsf_region;
+
+/*
+ * Scores the reading frames, or the open reading frames, of n_aln alignments (the inputs of pcsf_score_msa) on the device.
+ *   ref_row     [n_aln] model row of each alignment's reference species: its codons define stops (TAA TAG TGA) and starts (ATG)
+ *   frames      1 (+1), 3 (+1 +2 +3) or 6 (+1 +2 +3 -1 -2 -3); a '-' frame reads the reverse complement of the whole alignment
+ *   orf         ASIS: one region per frame, from the frame's offset to the alignment's end (frame +1 = the whole alignment);
+ *               STOPSTOP: every stop-delimited segment of a frame (closing stop included) and its non-empty open tail;
+ *               ATGSTOP: per segment, its first ATG through its stop (the open tail never yields one)
+ *   min_codons  >= 1; the ORF modes keep regions of at least this many codons
+ *   best_only   0: every region, by alignment, frame (+1 +2 +3 -1 -2 -3) and codon; 1: one region per alignment, the largest phylo
+ *               (NaN never wins, ties go to the earlier region; all NaN: the first; none: the "none" record)
+ * A region's (phylo, anc, bls) are bit for bit what pcsf_score_msa returns for its sub-alignment extracted on the host (reverse
+ * complemented for '-').  anc / bls are NaN unless want_anc / want_bls.  FP64 throughout.  *n_regions receives the number of
+ * records; pcsf_score_regions_get copies the first n of them (n <= *n_regions) from the handle.
+ */
+pcsf_status pcsf_score_regions(pcsf_model *m, pcsf_strategy strategy, int32_t n_aln, const uint8_t *seqs, const int64_t *offset,
+                               const int64_t *len, const int32_t *ref_row, int32_t frames, pcsf_orf_mode orf, int32_t min_codons,
+                               int32_t best_only, int32_t want_anc, int32_t want_bls, int64_t *n_regions);
+pcsf_status pcsf_score_regions_get(const pcsf_model *m, pcsf_region *out, int64_t n);   /* results of the last call on this handle */
+
 /* ---- introspection (used by the parity tests) -------------------------------------------------- */
 
 /* What the last pcsf_score_msa call with PCSF_STRATEGY_MLE did on this handle: `evaluations` counts lpr_leaves calls — (alignment,

@@ -32,10 +32,20 @@ STRATEGY_MLE = 0
 STRATEGY_FIXED = 1
 STRATEGY_OMEGA = 2
 
+ORF_ASIS = 0
+ORF_STOPSTOP = 1
+ORF_ATGSTOP = 2
+
+# pcsf_region (include/phylocsf_b200.h), 48 bytes
+REGION_DTYPE = np.dtype([("aln", np.int32), ("strand", np.int8), ("frame", np.int8), ("pad", np.int16), ("col_begin", np.int64),
+                         ("col_end", np.int64), ("codons", np.int64), ("phylo", np.float32), ("anc", np.float32),
+                         ("bls", np.float32)], align=True)
+
 EXPORTS = [
     "pcsf_model_create", "pcsf_model_destroy", "pcsf_last_error", "pcsf_abi_version", "pcsf_tracks",
     "pcsf_tracks_device", "pcsf_tracks_device_finish", "pcsf_set_chunk_columns", "pcsf_set_timing",
     "pcsf_score_msa", "pcsf_model_get", "pcsf_alloc_pinned", "pcsf_free_pinned", "pcsf_device_count", "pcsf_score_msa_stats", "pcsf_register_host", "pcsf_unregister_host",
+    "pcsf_score_regions", "pcsf_score_regions_get",
 ]
 
 
@@ -101,6 +111,9 @@ def load():
     L.pcsf_model_get.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]
     L.pcsf_score_msa_stats.argtypes = [C.c_void_p, C.POINTER(MsaStats)]
     L.pcsf_device_count.restype = C.c_int
+    L.pcsf_score_regions.argtypes = [C.c_void_p, C.c_int, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32,
+                                     C.c_int, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.POINTER(C.c_int64)]
+    L.pcsf_score_regions_get.argtypes = [C.c_void_p, C.c_void_p, C.c_int64]
     _lib = L
     return L
 
@@ -188,8 +201,7 @@ class DeviceModel:
         _check(load().pcsf_score_msa_stats(self.h, C.byref(st)))
         return st.as_dict()
 
-    def score_msa(self, alignments, strategy: int = STRATEGY_FIXED, comp_anc: bool = True, comp_bls: bool = True):
-        """alignments: list of uint8 ASCII [nl, L_i] matrices.  Returns (phylo, anc, bls) float32 arrays."""
+    def _batch(self, alignments):
         n = len(alignments)
         lens = np.array([a.shape[1] for a in alignments], np.int64)
         offs = np.zeros(n, np.int64)
@@ -198,9 +210,33 @@ class DeviceModel:
         blob = np.concatenate([np.ascontiguousarray(a, np.uint8).reshape(-1) for a in alignments]) if n else np.zeros(1, np.uint8)
         if blob.size == 0:
             blob = np.zeros(1, np.uint8)
+        return n, lens, offs, blob
+
+    def score_msa(self, alignments, strategy: int = STRATEGY_FIXED, comp_anc: bool = True, comp_bls: bool = True):
+        """alignments: list of uint8 ASCII [nl, L_i] matrices.  Returns (phylo, anc, bls) float32 arrays."""
+        n, lens, offs, blob = self._batch(alignments)
         phylo = np.full(n, np.nan, np.float32)
         anc = np.full(n, np.nan, np.float32) if comp_anc else None
         b = np.full(n, np.nan, np.float32) if comp_bls else None
         _check(load().pcsf_score_msa(self.h, strategy, n, blob.ctypes.data, offs.ctypes.data, lens.ctypes.data,
                                      phylo.ctypes.data, _ptr(anc), _ptr(b)))
         return phylo, anc, b
+
+    def score_regions(self, alignments, ref_rows, strategy: int = STRATEGY_FIXED, frames: int = 6, orf: int = ORF_ATGSTOP,
+                      min_codons: int = 25, best_only: bool = False, comp_anc: bool = True, comp_bls: bool = True) -> np.ndarray:
+        """Reading frames / ORFs of every alignment, scored on the device (pcsf_score_regions).  ref_rows: model row of each
+        alignment's reference species.  Returns a structured array of REGION_DTYPE records (phylocsfpp_b200.orf mirrors the
+        enumeration and the best-only rule)."""
+        n, lens, offs, blob = self._batch(alignments)
+        refs = np.ascontiguousarray(np.asarray(ref_rows, np.int32).reshape(-1))
+        if refs.size != n:
+            raise ValueError("one reference row per alignment")
+        if refs.size == 0:
+            refs = np.zeros(1, np.int32)
+        L = load()
+        nreg = C.c_int64(0)
+        _check(L.pcsf_score_regions(self.h, strategy, n, blob.ctypes.data, offs.ctypes.data, lens.ctypes.data, refs.ctypes.data,
+                                    frames, orf, min_codons, int(best_only), int(comp_anc), int(comp_bls), C.byref(nreg)))
+        out = np.zeros(nreg.value, REGION_DTYPE)
+        _check(L.pcsf_score_regions_get(self.h, out.ctypes.data if out.size else None, nreg.value))
+        return out

@@ -97,7 +97,8 @@ __global__ void k_pack(const uint8_t *__restrict__ seqs, int64_t L, int64_t ld_i
 
 // ---------------------------------------------------------------------------------------------------
 // Window enumeration.  mode 0 (tracks): local window lw of a chunk starting at column c0 is
-// (o = c0 + lw/2, strand = lw&1).  mode 1 (score-msa): o = win_off[lw], strand '+'.
+// (o = c0 + lw/2, strand = lw&1).  mode 1 (score-msa): o = win_off[lw], strand = win_strand[lw] (0 '+', 1 '-'), or '+' for every
+// window when win_strand is null.  A '-' window at o is the codon comp(x[o+2]) comp(x[o+1]) comp(x[o]) (codon_minus).
 struct WinSpace {
     const uint8_t *codes;
     int64_t ld;
@@ -105,7 +106,15 @@ struct WinSpace {
     int mode;
     int64_t c0;
     const uint32_t *win_off;
+    const uint8_t *win_strand;   // mode 1 only, nullable
 };
+
+// (column offset, strand) of local window lw
+__device__ __forceinline__ int64_t win_column(const WinSpace &ws, uint32_t lw, uint32_t *strand) {
+    if (ws.mode == 0) { *strand = lw & 1; return ws.c0 + (lw >> 1); }
+    *strand = ws.win_strand ? ws.win_strand[lw] : 0u;
+    return ws.win_off[lw];
+}
 
 __device__ __forceinline__ uint32_t codon_plus(uint32_t b0, uint32_t b1, uint32_t b2) {
     return ((b0 | b1 | b2) & 4u) ? 64u : 16u * b0 + 4u * b1 + b2;
@@ -185,14 +194,15 @@ __global__ void k_keys_tracks_unaligned(WinSpace ws, int64_t ncols, ulonglong2 *
     khi[t] = make_ulonglong2(fmix64(hp.h2), fmix64(hm.h2));
 }
 
-// k_keys mode 1: one thread per listed window, '+' strand only.
+// k_keys mode 1: one thread per listed window (the '-' codon id for a '-' window).
 __global__ void k_keys_list(WinSpace ws, int64_t nwin, uint64_t *__restrict__ klo, uint64_t *__restrict__ khi) {
     const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= nwin) return;
+    const bool minus = ws.win_strand && ws.win_strand[t];
     const uint8_t *p = ws.codes + ws.win_off[t];
     uint64_t a1 = 0x9E3779B97F4A7C15ULL, a2 = 0xC2B2AE3D27D4EB4FULL;
     for (int s = 0; s < ws.nl; ++s, p += ws.ld) {
-        const uint64_t cp = codon_plus(p[0], p[1], p[2]);
+        const uint64_t cp = minus ? codon_minus(p[0], p[1], p[2]) : codon_plus(p[0], p[1], p[2]);
         a1 = (a1 ^ cp) * 0x100000001B3ULL;
         a2 = (a2 + cp + 1) * 0xFF51AFD7ED558CCDULL; a2 ^= a2 >> 29;
     }
@@ -207,10 +217,8 @@ constexpr uint32_t EMPTY = 0xFFFFFFFFu;
 // The nl codon ids of two windows, compared one by one.  Only windows whose 128-bit keys are equal get here (i.e. duplicates pay
 // for it, nl x 6 byte loads), and it makes pattern identity exact instead of "equal up to a 128-bit hash collision".
 __device__ __forceinline__ bool same_pattern(const WinSpace &ws, uint32_t w1, uint32_t w2) {
-    int64_t o1, o2;
-    uint32_t s1 = 0, s2 = 0;
-    if (ws.mode == 0) { o1 = ws.c0 + (w1 >> 1); s1 = w1 & 1; o2 = ws.c0 + (w2 >> 1); s2 = w2 & 1; }
-    else { o1 = ws.win_off[w1]; o2 = ws.win_off[w2]; }
+    uint32_t s1, s2;
+    const int64_t o1 = win_column(ws, w1, &s1), o2 = win_column(ws, w2, &s2);
     const uint8_t *p = ws.codes + o1, *q = ws.codes + o2;
     for (int s = 0; s < ws.nl; ++s, p += ws.ld, q += ws.ld) {
         const uint32_t a = s1 ? codon_minus(p[0], p[1], p[2]) : codon_plus(p[0], p[1], p[2]);
@@ -527,9 +535,8 @@ __global__ void __launch_bounds__(PR_THREADS, 1) k_prune(const PruneArgs a) {
                 if (u >= n_unique) u = n_unique - 1;
                 lw = a.uniq[u];
             }
-            int64_t o; uint32_t strand;
-            if (a.ws.mode == 0) { o = a.ws.c0 + (lw >> 1); strand = lw & 1; }
-            else { o = a.ws.win_off[lw]; strand = 0; }
+            uint32_t strand;
+            const int64_t o = win_column(a.ws, lw, &strand);
             s_woff[tid] = (o << 1) | strand;
         }
         named_bar_sync(1, PR_NWARP * 32);

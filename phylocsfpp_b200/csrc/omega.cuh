@@ -72,7 +72,10 @@ __global__ void __launch_bounds__(256) k_omega_counts(WinSpace ws, int n_aln, co
         const int sp = (int)(i / K);
         const int64_t k = i - (int64_t)sp * K;
         const uint8_t *c = ws.codes + (size_t)sp * ws.ld + ws.win_off[w0 + k];
-        const int a = c[0], b = c[1], d = c[2];
+        int a = c[0], b = c[1], d = c[2];
+        if (ws.win_strand && ws.win_strand[w0 + k] && a < 4 && b < 4 && d < 4) {   // '-' window: the complemented, reversed codon
+            const int t = a; a = 3 - d; b = 3 - b; d = 3 - t;
+        }
         if (a < 4 && b < 4 && d < 4) { ++loc[a]; ++loc[4 + b]; ++loc[8 + d]; }
     }
     for (int j = 0; j < 12; ++j) if (loc[j]) atomicAdd(&cnt[j], loc[j]);

@@ -19,6 +19,7 @@
 #include "mle.cuh"
 #include "omega.cuh"
 #include "prune_tc5.cuh"
+#include "regions.cuh"
 #include <nvtx3/nvToolsExt.h>
 
 using namespace pcsf;
@@ -96,6 +97,8 @@ struct pcsf_model {
     int32_t *d_gemm_edges = nullptr;
     // scratch
     DevBuf codes, klo, khi, slot, flag, uniq, pidx, table, bsums, logz, anc, misc, io_in, io_out, perwin, mle;
+    DevBuf rg_units, rg_regions, rg_win;      // pcsf_score_regions: per-(alignment, frame) counts, region lists, region windows
+    std::vector<pcsf_region> regions;         // records of the last pcsf_score_regions call
     int *d_bad = nullptr;
     uint32_t *d_nuniq = nullptr;       // [max chunks]
     int64_t chunk_cols = (int64_t)1 << 21;          // 2 Mi columns: calls of 4 Mi columns and more are pipelined (H2D | compute | D2H per chunk)
@@ -245,7 +248,8 @@ extern "C" void pcsf_model_destroy(pcsf_model *m) {
     for (cudaEvent_t e : m->ev_h2d) cudaEventDestroy(e);
     if (m->ev_chunk) cudaEventDestroy(m->ev_chunk);
     DevBuf *bufs[] = {&m->codes, &m->klo, &m->khi, &m->slot, &m->flag, &m->uniq, &m->pidx, &m->table,
-                      &m->bsums, &m->logz, &m->anc, &m->misc, &m->io_in, &m->io_out, &m->perwin, &m->mle, &m->tc5_ids};
+                      &m->bsums, &m->logz, &m->anc, &m->misc, &m->io_in, &m->io_out, &m->perwin, &m->mle, &m->tc5_ids,
+                      &m->rg_units, &m->rg_regions, &m->rg_win};
     for (DevBuf *b : bufs) b->release();
     for (auto &e : m->ev) if (e) cudaEventDestroy(e);
     delete m;
@@ -667,6 +671,35 @@ extern "C" int pcsf_device_count(void) {
 }
 
 // ---- score-msa -------------------------------------------------------------------------------------
+// The batch side by side ([nl][Ltot], alignment i at col_start[i], two N pad columns behind each) in the handle's page-locked staging
+// (allocated once, re-used by every call: plain DMA, no fresh 100 MB vector per call), copied to the device and packed into m->codes;
+// only the pad columns and the tail are filled with N.
+static pcsf_status stage_and_pack(pcsf_model *m, int32_t n_aln, const uint8_t *seqs, const int64_t *offset, const int64_t *len,
+                                  const int64_t *col_start, int64_t Ltot, cudaStream_t st) {
+    const int nl = m->host.nl;
+    const int64_t ldd = ((Ltot + 15) / 16) * 16;
+    const size_t h_bytes = (size_t)ldd * nl;
+    if (h_bytes > m->h_msa_cap) {
+        if (m->h_msa) cudaFreeHost(m->h_msa);
+        m->h_msa = nullptr;
+        m->h_msa_cap = h_bytes + h_bytes / 4 + 4096;
+        CK(cudaHostAlloc(reinterpret_cast<void **>(&m->h_msa), m->h_msa_cap, cudaHostAllocPortable));
+    }
+    uint8_t *h = m->h_msa;
+    for (int s = 0; s < nl; ++s) {
+        uint8_t *row = h + (size_t)s * ldd;
+        for (int i = 0; i < n_aln; ++i) {
+            memcpy(row + col_start[i], seqs + offset[i] + (size_t)s * len[i], (size_t)len[i]);
+            row[col_start[i] + len[i]] = 'N';
+            row[col_start[i] + len[i] + 1] = 'N';
+        }
+        memset(row + Ltot, 'N', (size_t)(ldd - Ltot));
+    }
+    CK(m->io_in.reserve(h_bytes));
+    CK(cudaMemcpyAsync(m->io_in.p, h, h_bytes, cudaMemcpyHostToDevice, st));
+    return run_pack(m, m->io_in.as<uint8_t>(), Ltot, ldd, st);
+}
+
 extern "C" pcsf_status pcsf_score_msa(pcsf_model *m, pcsf_strategy strategy, int32_t n_aln, const uint8_t *seqs,
                                       const int64_t *offset, const int64_t *len, float *phylo, float *anc, float *bls) {
     if (!m || n_aln < 0 || (n_aln > 0 && (!seqs || !offset || !len)))
@@ -688,33 +721,11 @@ extern "C" pcsf_status pcsf_score_msa(pcsf_model *m, pcsf_strategy strategy, int
     }
     if (Ltot >= ((int64_t)1 << 32) || nwin >= ((int64_t)1 << 31))
         return fail(PCSF_ERR_INVALID, "batch too large: split the call");
-    const int64_t ldd = ((Ltot + 15) / 16) * 16;
-    // the batch side by side in the handle's page-locked staging (allocated once, re-used by every call: plain DMA, no fresh 100 MB
-    // vector per call); only the two pad columns behind every alignment and the tail are filled with N
-    const size_t h_bytes = (size_t)ldd * nl;
-    if (h_bytes > m->h_msa_cap) {
-        if (m->h_msa) cudaFreeHost(m->h_msa);
-        m->h_msa = nullptr;
-        m->h_msa_cap = h_bytes + h_bytes / 4 + 4096;
-        CK(cudaHostAlloc(reinterpret_cast<void **>(&m->h_msa), m->h_msa_cap, cudaHostAllocPortable));
-    }
-    uint8_t *h = m->h_msa;
-    for (int s = 0; s < nl; ++s) {
-        uint8_t *row = h + (size_t)s * ldd;
-        for (int i = 0; i < n_aln; ++i) {
-            memcpy(row + col_start[i], seqs + offset[i] + (size_t)s * len[i], (size_t)len[i]);
-            row[col_start[i] + len[i]] = 'N';
-            row[col_start[i] + len[i] + 1] = 'N';
-        }
-        memset(row + Ltot, 'N', (size_t)(ldd - Ltot));
-    }
     std::vector<uint32_t> win_off((size_t)std::max<int64_t>(nwin, 1));
     for (int i = 0; i < n_aln; ++i)
         for (int64_t k = 0; k < len[i] / 3; ++k) win_off[win_start[i] + k] = (uint32_t)(col_start[i] + 3 * k);
-    CK(m->io_in.reserve(h_bytes));
-    CK(cudaMemcpyAsync(m->io_in.p, h, h_bytes, cudaMemcpyHostToDevice, st));
     pcsf_status rc;
-    if ((rc = run_pack(m, m->io_in.as<uint8_t>(), Ltot, ldd, st))) return rc;
+    if ((rc = stage_and_pack(m, n_aln, seqs, offset, len, col_start.data(), Ltot, st))) return rc;
     // misc: win_off | col_start | win_start | len | outputs
     const size_t o_win = 0, o_cs = o_win + ((win_off.size() * 4 + 15) / 16) * 16, o_ws = o_cs + (size_t)n_aln * 8,
                  o_len = o_ws + (size_t)n_aln * 8, o_out = o_len + (size_t)n_aln * 8, total = o_out + (size_t)n_aln * 12 + 64;
@@ -810,5 +821,181 @@ extern "C" pcsf_status pcsf_score_msa(pcsf_model *m, pcsf_strategy strategy, int
     if (anc && strategy == PCSF_STRATEGY_OMEGA) { for (int i = 0; i < n_aln; ++i) anc[i] = nanf(""); }
     else if (anc) CK(cudaMemcpy(anc, d_anc, (size_t)n_aln * 4, cudaMemcpyDeviceToHost));
     if (bls) CK(cudaMemcpy(bls, d_bls, (size_t)n_aln * 4, cudaMemcpyDeviceToHost));
+    return PCSF_OK;
+}
+
+// ---- score-msa over reading frames / ORFs -----------------------------------------------------------
+static_assert(sizeof(pcsf_region) == 48, "pcsf_region layout is part of the ABI");
+
+extern "C" pcsf_status pcsf_score_regions(pcsf_model *m, pcsf_strategy strategy, int32_t n_aln, const uint8_t *seqs, const int64_t *offset,
+                                          const int64_t *len, const int32_t *ref_row, int32_t frames, pcsf_orf_mode orf, int32_t min_codons,
+                                          int32_t best_only, int32_t want_anc, int32_t want_bls, int64_t *n_regions) {
+    if (!m || !n_regions || n_aln < 0 || (n_aln > 0 && (!seqs || !offset || !len || !ref_row)))
+        return fail(PCSF_ERR_INVALID, "pcsf_score_regions: bad argument");
+    *n_regions = 0;
+    m->regions.clear();
+    if (strategy != PCSF_STRATEGY_FIXED && strategy != PCSF_STRATEGY_MLE && strategy != PCSF_STRATEGY_OMEGA)
+        return fail(PCSF_ERR_INVALID, "pcsf_score_regions: unknown strategy");
+    if (frames != 1 && frames != 3 && frames != 6) return fail(PCSF_ERR_INVALID, "pcsf_score_regions: frames must be 1, 3 or 6");
+    if (orf != PCSF_ORF_ASIS && orf != PCSF_ORF_STOPSTOP && orf != PCSF_ORF_ATGSTOP)
+        return fail(PCSF_ERR_INVALID, "pcsf_score_regions: unknown ORF mode");
+    if (min_codons < 1) return fail(PCSF_ERR_INVALID, "pcsf_score_regions: min_codons must be >= 1");
+    if (want_anc && strategy == PCSF_STRATEGY_OMEGA)
+        return fail(PCSF_ERR_INVALID, "pcsf_score_regions: OMEGA has no ancestral score");
+    const int nl = m->host.nl;
+    std::vector<int64_t> col_start(n_aln);
+    int64_t Ltot = 0;
+    for (int i = 0; i < n_aln; ++i) {
+        if (len[i] < 0) return fail(PCSF_ERR_INVALID, "negative alignment length");
+        if (ref_row[i] < 0 || ref_row[i] >= nl) return fail(PCSF_ERR_INVALID, "pcsf_score_regions: ref_row out of range");
+        col_start[i] = Ltot;
+        Ltot += len[i] + 2;
+    }
+    const int64_t n_units = (int64_t)n_aln * frames;
+    if (Ltot >= ((int64_t)1 << 32) || n_units >= ((int64_t)1 << 31)) return fail(PCSF_ERR_INVALID, "batch too large: split the call");
+    NvtxRange nvtx_("pcsf_score_regions");
+    CK(cudaSetDevice(m->device));
+    if (n_aln == 0) return PCSF_OK;
+    cudaStream_t st = m->own_stream;
+    pcsf_status rc;
+    if ((rc = stage_and_pack(m, n_aln, seqs, offset, len, col_start.data(), Ltot, st))) return rc;
+
+    // per-unit buffers: col_start | len | ref_row | totals | n_reg | n_win | bsums x 2 | off_r | off_w
+    const uint32_t nsb = (uint32_t)((n_units + SCAN_BLOCK - 1) / SCAN_BLOCK);
+    size_t o = 0;
+    auto take = [&](size_t bytes) { const size_t r = o; o += (bytes + 255) / 256 * 256; return r; };
+    const size_t o_cs = take((size_t)n_aln * 8), o_len = take((size_t)n_aln * 8), o_ref = take((size_t)n_aln * 4), o_tot = take(16),
+                 o_nr = take((size_t)n_units * 4), o_nw = take((size_t)n_units * 4), o_br = take((size_t)(nsb + 1) * 4),
+                 o_bw = take((size_t)(nsb + 1) * 4), o_or = take((size_t)(n_units + 1) * 8), o_ow = take((size_t)(n_units + 1) * 8);
+    CK(m->rg_units.reserve(o));
+    unsigned char *ub = m->rg_units.as<unsigned char>();
+    CK(cudaMemcpyAsync(ub + o_cs, col_start.data(), (size_t)n_aln * 8, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(ub + o_len, len, (size_t)n_aln * 8, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(ub + o_ref, ref_row, (size_t)n_aln * 4, cudaMemcpyHostToDevice, st));
+    CK(cudaMemsetAsync(ub + o_tot, 0, 16, st));
+    unsigned long long *d_tot = reinterpret_cast<unsigned long long *>(ub + o_tot);
+    uint32_t *d_nr = reinterpret_cast<uint32_t *>(ub + o_nr), *d_nw = reinterpret_cast<uint32_t *>(ub + o_nw);
+    uint32_t *d_br = reinterpret_cast<uint32_t *>(ub + o_br), *d_bw = reinterpret_cast<uint32_t *>(ub + o_bw);
+    int64_t *d_or = reinterpret_cast<int64_t *>(ub + o_or), *d_ow = reinterpret_cast<int64_t *>(ub + o_ow);
+    RegionUnits U{m->codes.as<uint8_t>(), m->codes_ld, n_aln, frames, (int)orf, min_codons, reinterpret_cast<const int64_t *>(ub + o_cs),
+                  reinterpret_cast<const int64_t *>(ub + o_len), reinterpret_cast<const int32_t *>(ub + o_ref)};
+    const unsigned warp_blocks = (unsigned)((n_units * 32 + 255) / 256);
+    {
+        NvtxRange nvtx_e("pcsf: region enumeration");
+        m->launches += 6;
+        k_orf_count<<<warp_blocks, 256, 0, st>>>(U, n_units, d_nr, d_nw, d_tot);
+        k_scan_blocks<<<nsb, SCAN_THREADS, 0, st>>>(d_nr, (uint32_t)n_units, d_br);
+        k_scan_sums<<<1, 1024, 0, st>>>(d_br, nsb, d_br + nsb);
+        k_scan_blocks<<<nsb, SCAN_THREADS, 0, st>>>(d_nw, (uint32_t)n_units, d_bw);
+        k_scan_sums<<<1, 1024, 0, st>>>(d_bw, nsb, d_bw + nsb);
+        k_unit_offsets<<<(unsigned)((n_units + 1 + 255) / 256), 256, 0, st>>>(n_units, d_nr, d_br, d_nw, d_bw, d_tot, d_or, d_ow);
+        CK(cudaGetLastError());
+    }
+    unsigned long long tot[2] = {0, 0};
+    CK(cudaMemcpyAsync(tot, d_tot, 16, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    // the 32-bit scans above are exact only below 2^32; the window lists (uint32 ids, int counts in the fits) need < 2^31
+    if (tot[0] >= (1ull << 31) || tot[1] >= (1ull << 31)) return fail(PCSF_ERR_INVALID, "too many regions or region codons: split the call");
+    const int64_t nreg = (int64_t)tot[0], nwin = (int64_t)tot[1];
+    const int64_t n_out = best_only ? n_aln : nreg;
+
+    // per-region buffers: aln | fi | k0 | ncod | win_start | slen | phylo | anc | bls | records
+    o = 0;
+    const size_t nr1 = (size_t)std::max<int64_t>(nreg, 1);
+    const size_t o_ra = take(nr1 * 4), o_rf = take(nr1 * 4), o_rk = take(nr1 * 8), o_rn = take(nr1 * 8), o_rw = take(nr1 * 8),
+                 o_rl = take(nr1 * 8), o_ph = take(nr1 * 4), o_an = take(nr1 * 4), o_bl = take(nr1 * 4),
+                 o_rec = take((size_t)std::max<int64_t>(n_out, 1) * sizeof(pcsf_region));
+    CK(m->rg_regions.reserve(o));
+    unsigned char *rb = m->rg_regions.as<unsigned char>();
+    RegionList R{reinterpret_cast<int32_t *>(rb + o_ra), reinterpret_cast<int32_t *>(rb + o_rf), reinterpret_cast<int64_t *>(rb + o_rk),
+                 reinterpret_cast<int64_t *>(rb + o_rn), reinterpret_cast<int64_t *>(rb + o_rw), reinterpret_cast<int64_t *>(rb + o_rl)};
+    float *d_phylo = reinterpret_cast<float *>(rb + o_ph), *d_anc = reinterpret_cast<float *>(rb + o_an),
+          *d_bls = reinterpret_cast<float *>(rb + o_bl);
+    pcsf_region *d_rec = reinterpret_cast<pcsf_region *>(rb + o_rec);
+    CK(m->rg_win.reserve((size_t)std::max<int64_t>(nwin, 1) * 5 + 16));
+    uint32_t *d_woff = m->rg_win.as<uint32_t>();
+    uint8_t *d_wstr = m->rg_win.as<uint8_t>() + (size_t)std::max<int64_t>(nwin, 1) * 4;
+    if (nreg > 0) {
+        NvtxRange nvtx_w("pcsf: region windows");
+        m->launches += 2;
+        k_orf_emit<<<warp_blocks, 256, 0, st>>>(U, n_units, d_or, d_ow, R);
+        k_region_windows<<<(unsigned)std::min<int64_t>((nreg * 32 + 255) / 256, (int64_t)m->sm_count * 32), 256, 0, st>>>(U, nreg, R, d_woff,
+                                                                                                                           d_wstr);
+        CK(cudaGetLastError());
+    }
+    double *d_blraw = nullptr;
+    if (want_bls && nreg > 0) {
+        CK(m->io_out.reserve((size_t)Ltot * 8 + 64));
+        d_blraw = m->io_out.as<double>();
+        if ((rc = run_bls(m, Ltot, 1, d_blraw, st))) return rc;
+    }
+    const unsigned rgrid = (unsigned)((nreg + 127) / 128);
+    WinSpace ws{m->codes.as<uint8_t>(), m->codes_ld, nl, 1, 0, d_woff, d_wstr};
+    if (nreg > 0 && strategy == PCSF_STRATEGY_FIXED) {
+        CK(m->perwin.reserve((size_t)std::max<int64_t>(nwin, 1) * 32));
+        if (nwin > 0) {
+            float t0 = 0, t1 = 0, t2 = 0;
+            if ((rc = dedup_and_prune(m, ws, (uint32_t)nwin, true, want_anc != 0, 0, m->d_nuniq, nullptr, 0, st, &t0, &t1, &t2))) return rc;
+            k_scatter_list<<<(unsigned)((nwin + 255) / 256), 256, 0, st>>>(
+                (uint32_t)nwin, m->pidx.as<uint32_t>(), m->logz.as<double>(), m->logz.as<double>() + nwin,
+                want_anc ? m->anc.as<double>() : nullptr, want_anc ? m->anc.as<double>() + nwin : nullptr, m->perwin.as<double>());
+            CK(cudaGetLastError());
+        }
+        k_region_sums<<<rgrid, 128, 0, st>>>(U, nreg, R, m->perwin.as<double>(), nwin, d_blraw, m->host.bls_all, d_phylo,
+                                             want_anc ? d_anc : nullptr, want_bls ? d_bls : nullptr);
+        CK(cudaGetLastError());
+    } else if (nreg > 0) {
+        if (strategy == PCSF_STRATEGY_OMEGA) {
+            OmegaBatch b{};
+            b.n_aln = (int)nreg;
+            b.d_win_start = R.win_start;
+            b.d_len = R.slen;
+            b.ws = ws;
+            b.nwin = nwin;
+            b.d_phylo = d_phylo;
+            if ((rc = omega_run(m->host, b, m->d_bl, m->d_program, m->d_pi, m->d_logpi, m->mle, m->sm_count, m->prune_smem, m->prune_nwarp, st,
+                                g_err, &m->launches)))
+                return rc;
+        } else {
+            MleBatch b{};
+            b.n_aln = (int)nreg;
+            b.d_win_start = R.win_start;
+            b.d_len = R.slen;
+            b.ws = ws;
+            b.nwin = nwin;
+            b.want_anc = want_anc != 0;
+            b.d_phylo = d_phylo;
+            b.d_anc = want_anc ? d_anc : nullptr;
+            if ((rc = mle_run(m->host, b, m->d_eig, m->d_bl, m->d_program, m->d_pi, m->d_logpi, m->mle, m->sm_count, m->prune_smem,
+                              m->prune_nwarp, st, g_err, &m->launches, &m->msa_stats, m->timing)))
+                return rc;
+        }
+        if (want_bls) {
+            k_region_sums<<<rgrid, 128, 0, st>>>(U, nreg, R, nullptr, 0, d_blraw, m->host.bls_all, nullptr, nullptr, d_bls);
+            CK(cudaGetLastError());
+        }
+    }
+    const float *r_anc = want_anc ? d_anc : nullptr, *r_bls = want_bls ? d_bls : nullptr;
+    if (best_only) {
+        k_best_region<<<(unsigned)(((int64_t)n_aln * 32 + 255) / 256), 256, 0, st>>>(U, R, d_or, d_phylo, r_anc, r_bls, d_rec);
+        CK(cudaGetLastError());
+    } else if (nreg > 0) {
+        k_region_records<<<rgrid, 128, 0, st>>>(U, nreg, R, d_phylo, r_anc, r_bls, d_rec);
+        CK(cudaGetLastError());
+    }
+    CK(cudaStreamSynchronize(st));
+    int bad = 0;
+    CK(cudaMemcpy(&bad, m->d_bad, sizeof(int), cudaMemcpyDeviceToHost));
+    if (bad) return fail(PCSF_ERR_BAD_CHAR, "alignment contains a character outside ACGTacgt.-Nn (reference: exit(37))");
+    m->regions.resize((size_t)n_out);
+    if (n_out > 0) CK(cudaMemcpy(m->regions.data(), d_rec, (size_t)n_out * sizeof(pcsf_region), cudaMemcpyDeviceToHost));
+    *n_regions = n_out;
+    return PCSF_OK;
+}
+
+extern "C" pcsf_status pcsf_score_regions_get(const pcsf_model *m, pcsf_region *out, int64_t n) {
+    if (!m || n < 0 || (n > 0 && !out) || n > (int64_t)m->regions.size())
+        return fail(PCSF_ERR_INVALID, "pcsf_score_regions_get: bad argument (n exceeds the records of the last call)");
+    if (n > 0) memcpy(out, m->regions.data(), (size_t)n * sizeof(pcsf_region));
     return PCSF_OK;
 }

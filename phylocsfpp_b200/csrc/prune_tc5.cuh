@@ -123,9 +123,8 @@ __global__ void __launch_bounds__(128) k_tc5_ids(const WinSpace ws, const uint32
 #pragma unroll
         for (int h = 0; h < 2; ++h) {
             const uint32_t lw = h ? lw1 : lw0;
-            int64_t o; uint32_t strand;
-            if (ws.mode == 0) { o = ws.c0 + (lw >> 1); strand = lw & 1; }
-            else { o = ws.win_off[lw]; strand = 0; }
+            uint32_t strand;
+            const int64_t o = win_column(ws, lw, &strand);
             const uint8_t *p = ws.codes + o;
             for (int s0 = 0; s0 < ws.nl; s0 += 16) {
                 uint32_t v[16][3];

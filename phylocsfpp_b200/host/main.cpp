@@ -592,7 +592,7 @@ int main_build_tracks(int argc, char **argv) {
 // ---------------------------------------------------------------------------------------------- score-msa
 int main_score_msa(int argc, char **argv) {
     const Args a = parse_args(argc, argv, {"strategy", "comp-phylo", "comp-anc", "comp-bls", "threads", "output", "mapping", "species", "gpus",
-                                           "genome-length", "coding-exons", "model-info"});
+                                           "genome-length", "coding-exons", "model-info", "frames", "orf", "min-codons", "all-scores"});
     if (a.has("model-info")) return print_model_info(a.str("model-info"));          // score_msa.hpp:291-295
     if (a.pos.size() < 2) die("usage: phylocsf_b200 score-msa [OPTIONS] <model> <alignments>...");
     const std::string strat = lower(a.str("strategy", "mle"));
@@ -610,6 +610,42 @@ int main_score_msa(int argc, char **argv) {
     const bool comp_phylo = a.boolean("comp-phylo", true), comp_anc = a.boolean("comp-anc", false), comp_bls = true;   // no --comp-bls in the reference
     if (strategy == PCSF_STRATEGY_OMEGA && comp_anc) {          // score_msa.hpp:338-342
         printf("\033[31mThe ancestral sequence composition cannot be computed in the Omega mode!\n\033[0m");
+        return -1;
+    }
+    // reading frames / ORFs (pcsf_score_regions): with --frames 1 --orf asis and without --all-scores the command is the plain
+    // frame +1 score-msa and takes its path unchanged
+    auto strict_int = [&](const char *k, int dflt, int *v) {
+        if (!a.has(k)) { *v = dflt; return true; }
+        const std::string t = a.str(k);
+        char *e = nullptr;
+        const long x = strtol(t.c_str(), &e, 10);
+        if (t.empty() || *e || x < INT32_MIN || x > INT32_MAX) return false;
+        *v = (int)x;
+        return true;
+    };
+    int frames = 1, min_codons = 25;
+    if (!strict_int("frames", 1, &frames) || (frames != 1 && frames != 3 && frames != 6)) {
+        printf("\033[31m--frames must be 1, 3 or 6!\n\033[0m");
+        return -1;
+    }
+    const std::string orf_s = lower(a.str("orf", "asis"));
+    pcsf_orf_mode orf;
+    if (orf_s == "asis") orf = PCSF_ORF_ASIS;
+    else if (orf_s == "stopstop") orf = PCSF_ORF_STOPSTOP;
+    else if (orf_s == "atgstop") orf = PCSF_ORF_ATGSTOP;
+    else { printf("\033[31m--orf must be AsIs, StopStop or ATGStop!\n\033[0m"); return -1; }
+    if (!strict_int("min-codons", 25, &min_codons) || min_codons < 1) {
+        printf("\033[31m--min-codons must be an integer >= 1!\n\033[0m");
+        return -1;
+    }
+    const bool all_scores = a.boolean("all-scores", false);
+    const bool regions = frames != 1 || orf != PCSF_ORF_ASIS || all_scores;
+    if (regions && fixed_mean) {
+        printf("\033[31mFIXED_MEAN cannot be combined with --frames, --orf or --all-scores!\n\033[0m");
+        return -1;
+    }
+    if (regions && !all_scores && !comp_phylo) {
+        printf("\033[31mThe best frame or ORF is chosen by its PhyloCSF score: --comp-phylo 0 needs --all-scores 1!\n\033[0m");
         return -1;
     }
     const int threads = std::max(1, a.integer("threads", (int)std::thread::hardware_concurrency()));
@@ -643,6 +679,7 @@ int main_score_msa(int argc, char **argv) {
         if (!out) die("Error creating file '%s'!", out_path.c_str());
         fprintf(out, "# PhyloCSF scores computed with PhyloCSF++ v1.2.0 (phylocsf_b200, B200-native likelihood core)\n");
         fprintf(out, "seq\tstart\tend\tstrand");
+        if (regions) fprintf(out, "\tframe\torf-start\torf-end");
         if (comp_phylo) fprintf(out, "\tphylocsf-score");
         if (comp_anc) fprintf(out, "\tanc-score");
         if (comp_bls) fprintf(out, "\tbls-score");
@@ -669,11 +706,14 @@ int main_score_msa(int argc, char **argv) {
                     std::vector<uint8_t> blob;
                     std::vector<int64_t> off, len;
                     std::vector<std::string> head;
+                    std::vector<int32_t> ref_row;
+                    std::vector<int64_t> start_pos;
                     const auto p0 = std::chrono::steady_clock::now();
                     for (size_t ci = c0; ci < c1; ++ci) {
                         if (chains[ci].ref_id < 0) continue;
                         maf.read_chain(chains[ci], aln, nullptr);
                         off.push_back((int64_t)blob.size()); len.push_back(aln.L);
+                        ref_row.push_back(chains[ci].ref_id); start_pos.push_back(aln.start_pos);
                         blob.insert(blob.end(), aln.seqs.begin(), aln.seqs.end());
                         char h[600];
                         snprintf(h, sizeof h, "%s\t%" PRId64 "\t%" PRId64 "\t%c", aln.chrom.c_str(), aln.start_pos, aln.start_pos + aln.L - 1, aln.strand);
@@ -684,6 +724,43 @@ int main_score_msa(int argc, char **argv) {
                     if (blob.empty()) blob.push_back('N');
                     const double my_parse = since(p0);
                     const auto g0 = std::chrono::steady_clock::now();
+                    if (regions) {
+                        // one row per region (--all-scores 1) or per alignment (its best region); frame +1..-3 or "." for none,
+                        // ORF columns in the coordinates of start / end
+                        std::vector<pcsf_region> rg;
+                        if (n > 0) {
+                            int64_t nr = 0;
+                            pcsf_status st = pcsf_score_regions(dev[t], strategy, n, blob.data(), off.data(), len.data(), ref_row.data(), frames, orf,
+                                                                min_codons, all_scores ? 0 : 1, comp_anc ? 1 : 0, comp_bls ? 1 : 0, &nr);
+                            if (st == PCSF_ERR_BAD_CHAR) { fprintf(stderr, "%s\n", pcsf_last_error()); exit(37); }
+                            if (st != PCSF_OK) die("pcsf_score_regions: %s", pcsf_last_error());
+                            rg.resize((size_t)nr);
+                            if ((st = pcsf_score_regions_get(dev[t], rg.data(), nr)) != PCSF_OK) die("pcsf_score_regions_get: %s", pcsf_last_error());
+                        }
+                        const double my_gpu = since(g0);
+                        const auto f0 = std::chrono::steady_clock::now();
+                        std::string text;
+                        char v[128];
+                        for (const pcsf_region &r : rg) {
+                            text += head[r.aln];
+                            if (r.frame == 0) text += "\t.\t.\t.";
+                            else {
+                                snprintf(v, sizeof v, "\t%c%d\t%" PRId64 "\t%" PRId64, r.strand > 0 ? '+' : '-', (int)r.frame,
+                                         start_pos[r.aln] + r.col_begin, start_pos[r.aln] + r.col_end - 1);
+                                text += v;
+                            }
+                            if (comp_phylo) { snprintf(v, sizeof v, "\t%.6f", r.phylo); text += v; }
+                            if (comp_anc) { snprintf(v, sizeof v, "\t%.6f", r.anc); text += v; }
+                            if (comp_bls) { snprintf(v, sizeof v, "\t%.6f", r.bls); text += v; }
+                            text += "\n";
+                        }
+                        std::vector<std::string> one(1);
+                        one[0] = std::move(text);
+                        sink.put(bi, std::move(one));
+                        std::lock_guard<std::mutex> g(stat_mu);
+                        t_parse += my_parse; t_gpu += my_gpu; t_format += since(f0); total_aln += n;
+                        continue;
+                    }
                     if (n > 0) {
                         const pcsf_status st = pcsf_score_msa(dev[t], strategy, n, blob.data(), off.data(), len.data(), (comp_phylo || comp_anc) ? phylo.data() : nullptr,
                                                               comp_anc ? anc.data() : nullptr, comp_bls ? bls.data() : nullptr);
@@ -1002,6 +1079,7 @@ int main(int argc, char **argv) {
                "                             [--coding-exons FILE] [--power-threshold FLOAT] [--threads INT] [--gpus INT]\n"
                "                             [--precision f64|tc5] [--output-bigwig BOOL] [--output DIR] [--mapping FILE] [--species LIST] <model> <maf>...\n"
                "  phylocsf_b200 score-msa    [--strategy MLE|FIXED|OMEGA|FIXED_MEAN] [--comp-phylo BOOL] [--comp-anc BOOL] [--threads INT] [--gpus INT]\n"
+               "                             [--frames 1|3|6] [--orf AsIs|StopStop|ATGStop] [--min-codons INT] [--all-scores BOOL]\n"
                "                             [--output DIR] [--mapping FILE] [--species LIST] <model> <maf>...\n"
                "  phylocsf_b200 annotate-with-tracks [--output DIR] <PhyloCSF+1.bw> <gff/gtf>...\n"
                "  phylocsf_b200 wig-to-bigwig [--compress BOOL] <in.wig> <chrom.sizes> <out.bw>\n");

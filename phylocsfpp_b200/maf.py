@@ -37,6 +37,7 @@ class Alignment:
     strand: str = "+"
     chrom: str = ""
     seqs: np.ndarray = field(default_factory=lambda: np.zeros((0, 0), np.uint8))
+    ref_row: int = -1   # model row of the reference species (the first matched species of the first block); -1: none
 
     @property
     def L(self) -> int:
@@ -195,4 +196,5 @@ class MafReader:
         if reached_bp and prev_cum > cum_after_bp + 2:
             mat = mat[:, :cum_after_bp + 2]
         aln.seqs = np.ascontiguousarray(mat)
+        aln.ref_row = ref_seq_id
         return aln
