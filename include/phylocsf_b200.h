@@ -95,6 +95,10 @@ int pcsf_abi_version(void);
 #define PCSF_TRACKS_NO_DEDUP 0x4u  /* prune every window, do not deduplicate site patterns */
 /* 0x8u was PCSF_TRACKS_FP32 (split-TF32 on mma.sync, round 1): superseded by the tcgen05 path and removed from the library */
 #define PCSF_TRACKS_TC5      0x10u /* FP32-class arithmetic on tcgen05/TMEM (5th-gen tensor cores): split TF32 + per-window log-scaling, |delta| <= 1e-3 decibans */
+/* The tcgen05 path holds the tree's codon ids, step program and row sources in one SM's shared memory: every tree of at most 123
+ * leaves fits, trees of 124 to 126 leaves fit depending on their shape (a caterpillar is the largest program for its leaf count),
+ * trees of 127 and 128 leaves never fit.  For a tree that does not fit, pcsf_model_create still succeeds (the FP64 path and score-msa
+ * run on it) and a call with PCSF_TRACKS_TC5 returns PCSF_ERR_UNSUPPORTED. */
 
 typedef struct {
     int64_t n_windows;        /* 2 * max(L-2, 0) */

@@ -195,7 +195,10 @@ extern "C" pcsf_status pcsf_model_create(const pcsf_model_desc *d, int device, p
     if (const char *e = getenv("PCSF_TC5_NSTAGE")) m->tc5_nstage = std::max(2, std::min(m->tc5_nstage, atoi(e)));
     if (const char *e = getenv("PCSF_TC5_NIDS")) m->tc5_nids = std::max(1, std::min(m->tc5_nids, atoi(e)));
     m->prune_tc5_smem = prune_tc5_smem_bytes(m->host.nl, (int)m->host.tc5_steps.size(), (int)m->host.tc5_srcs.size(), m->tc5_nstage, m->tc5_nids);
-    CK(cudaFuncSetAttribute(k_prune_tc5, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)m->prune_tc5_smem));
+    // Trees above the tcgen05 path's budget (127 and 128 leaves always, 124 to 126 depending on the shape) still get a model: the FP64
+    // path and score-msa do not need k_prune_tc5, and pcsf_tracks_device refuses PCSF_TRACKS_TC5 for them with PCSF_ERR_UNSUPPORTED.
+    if (m->prune_tc5_smem <= 227 * 1024)
+        CK(cudaFuncSetAttribute(k_prune_tc5, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)m->prune_tc5_smem));
     if ((st = upload(m->host.bls_short.data(), m->host.bls_short.size() * sizeof(BlsInner), (void **)&m->d_bls_prog))) return st;
     if ((st = upload(m->host.bls_tables.data(), std::max<size_t>(m->host.bls_tables.size(), 1) * sizeof(double), (void **)&m->d_bls_tables))) return st;
     if ((st = upload(m->host.bl.data(), m->host.bl.size() * 4, (void **)&m->d_bl))) return st;
