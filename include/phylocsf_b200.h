@@ -188,7 +188,7 @@ typedef struct {
 pcsf_status pcsf_score_regions(pcsf_model *m, pcsf_strategy strategy, int32_t n_aln, const uint8_t *seqs, const int64_t *offset,
                                const int64_t *len, const int32_t *ref_row, int32_t frames, pcsf_orf_mode orf, int32_t min_codons,
                                int32_t best_only, int32_t want_anc, int32_t want_bls, int64_t *n_regions);
-pcsf_status pcsf_score_regions_get(const pcsf_model *m, pcsf_region *out, int64_t n);   /* results of the last call on this handle */
+pcsf_status pcsf_score_regions_get(const pcsf_model *m, pcsf_region *out, int64_t n);   /* records of the last pcsf_score_regions call on this handle */
 
 /* ---- introspection (used by the parity tests) -------------------------------------------------- */
 

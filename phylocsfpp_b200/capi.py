@@ -212,14 +212,16 @@ class DeviceModel:
             blob = np.zeros(1, np.uint8)
         return n, lens, offs, blob
 
-    def score_msa(self, alignments, strategy: int = STRATEGY_FIXED, comp_anc: bool = True, comp_bls: bool = True):
-        """alignments: list of uint8 ASCII [nl, L_i] matrices.  Returns (phylo, anc, bls) float32 arrays."""
+    def score_msa(self, alignments, strategy: int = STRATEGY_FIXED, comp_phylo: bool = True, comp_anc: bool = True,
+                  comp_bls: bool = True):
+        """alignments: list of uint8 ASCII [nl, L_i] matrices.  Returns (phylo, anc, bls) float32 arrays, None for a score not
+        asked for."""
         n, lens, offs, blob = self._batch(alignments)
-        phylo = np.full(n, np.nan, np.float32)
+        phylo = np.full(n, np.nan, np.float32) if comp_phylo else None
         anc = np.full(n, np.nan, np.float32) if comp_anc else None
         b = np.full(n, np.nan, np.float32) if comp_bls else None
         _check(load().pcsf_score_msa(self.h, strategy, n, blob.ctypes.data, offs.ctypes.data, lens.ctypes.data,
-                                     phylo.ctypes.data, _ptr(anc), _ptr(b)))
+                                     _ptr(phylo), _ptr(anc), _ptr(b)))
         return phylo, anc, b
 
     def score_regions(self, alignments, ref_rows, strategy: int = STRATEGY_FIXED, frames: int = 6, orf: int = ORF_ATGSTOP,

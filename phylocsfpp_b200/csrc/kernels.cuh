@@ -782,30 +782,4 @@ __global__ void __launch_bounds__(BLS_THREADS) k_bls(const uint8_t *__restrict__
     }
 }
 
-// ---------------------------------------------------------------------------------------------------
-// k_aln_sums (score-msa, FIXED): one thread per alignment, sequential sums in the reference's order:
-// lpr += log z per codon (fixed_lik.hpp:431-432), elpr_anc += ... (:440), bl_total += bl (additional_scores.hpp:71).
-__global__ void k_aln_sums(int n_aln, const int64_t *__restrict__ win_start, const int64_t *__restrict__ col_start,
-                           const int64_t *__restrict__ len, const double *__restrict__ perwin /* [4][nwin] */,
-                           int64_t nwin, const double *__restrict__ bl_raw, double bls_all,
-                           float *__restrict__ phylo, float *__restrict__ anc, float *__restrict__ bls) {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n_aln) return;
-    const int64_t K = len[i] / 3, w0 = win_start[i];
-    double lc = 0.0, lnc = 0.0, ac = 0.0, an = 0.0;
-    if (phylo || anc) for (int64_t k = 0; k < K; ++k) {
-        lc = __dadd_rn(lc, perwin[w0 + k]);
-        lnc = __dadd_rn(lnc, perwin[nwin + w0 + k]);
-        ac = __dadd_rn(ac, perwin[2 * nwin + w0 + k]);
-        an = __dadd_rn(an, perwin[3 * nwin + w0 + k]);
-    }
-    if (phylo) phylo[i] = (float)(10.0 * (lc - lnc) / log(10.0));
-    if (anc) anc[i] = (float)(10.0 * (ac - an) / log(10.0));
-    if (bls) {
-        double t = 0.0;
-        for (int64_t c = 0; c < len[i]; ++c) t = __dadd_rn(t, bl_raw[col_start[i] + c]);
-        bls[i] = (float)(t / (bls_all * (double)len[i]));
-    }
-}
-
 }  // namespace pcsf

@@ -64,7 +64,7 @@ struct MleStats {
 
 struct MleBatch {
     int n_aln;
-    const int64_t *d_win_start, *d_col_start, *d_len;
+    const int64_t *d_win_start, *d_len;
     WinSpace ws;
     int64_t nwin;
     bool want_anc;

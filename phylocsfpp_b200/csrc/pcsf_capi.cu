@@ -96,8 +96,8 @@ struct pcsf_model {
     float *d_bl = nullptr;
     int32_t *d_gemm_edges = nullptr;
     // scratch
-    DevBuf codes, klo, khi, slot, flag, uniq, pidx, table, bsums, logz, anc, misc, io_in, io_out, perwin, mle;
-    DevBuf rg_units, rg_regions, rg_win;      // pcsf_score_regions: per-(alignment, frame) counts, region lists, region windows
+    DevBuf codes, klo, khi, slot, flag, uniq, pidx, table, bsums, logz, anc, io_in, io_out, perwin, mle;
+    DevBuf rg_units, rg_regions, rg_win;      // score-msa (both entry points): per-(alignment, frame) counts, region lists, region windows
     std::vector<pcsf_region> regions;         // records of the last pcsf_score_regions call
     int *d_bad = nullptr;
     uint32_t *d_nuniq = nullptr;       // [max chunks]
@@ -251,7 +251,7 @@ extern "C" void pcsf_model_destroy(pcsf_model *m) {
     for (cudaEvent_t e : m->ev_h2d) cudaEventDestroy(e);
     if (m->ev_chunk) cudaEventDestroy(m->ev_chunk);
     DevBuf *bufs[] = {&m->codes, &m->klo, &m->khi, &m->slot, &m->flag, &m->uniq, &m->pidx, &m->table,
-                      &m->bsums, &m->logz, &m->anc, &m->misc, &m->io_in, &m->io_out, &m->perwin, &m->mle, &m->tc5_ids,
+                      &m->bsums, &m->logz, &m->anc, &m->io_in, &m->io_out, &m->perwin, &m->mle, &m->tc5_ids,
                       &m->rg_units, &m->rg_regions, &m->rg_win};
     for (DevBuf *b : bufs) b->release();
     for (auto &e : m->ev) if (e) cudaEventDestroy(e);
@@ -703,6 +703,154 @@ static pcsf_status stage_and_pack(pcsf_model *m, int32_t n_aln, const uint8_t *s
     return run_pack(m, m->io_in.as<uint8_t>(), Ltot, ldd, st);
 }
 
+// One scoring path for reading frames / ORFs (pcsf_score_regions); pcsf_score_msa is its frame +1 as is, one region per alignment.
+static_assert(sizeof(pcsf_region) == 48, "pcsf_region layout is part of the ABI");
+
+// What score_regions_core leaves on the device for its caller (in m->rg_units / m->rg_regions).
+struct ScoredRegions {
+    int64_t nreg = 0;
+    RegionUnits U{};
+    RegionList R{};
+    const int64_t *off_r = nullptr;                           // [n_aln * frames + 1]: first region of each (alignment, frame) unit
+    float *phylo = nullptr, *anc = nullptr, *bls = nullptr;   // [nreg]; phylo if fit, anc / bls if asked for, else null
+    pcsf_region *rec = nullptr;                               // room for max(nreg, n_aln) records
+};
+
+// The scoring path of both entry points: stage and pack the batch, enumerate its regions, score every region as an item of the
+// dedup + prune (FIXED), MLE or OMEGA machinery, synchronise and check for bad characters.  fit = false skips the likelihoods and
+// computes the BLS only.  ref_row may be null for PCSF_ORF_ASIS, which never reads it.
+static pcsf_status score_regions_core(pcsf_model *m, pcsf_strategy strategy, int32_t n_aln, const uint8_t *seqs, const int64_t *offset,
+                                      const int64_t *len, const int64_t *col_start, int64_t Ltot, const int32_t *ref_row, int32_t frames,
+                                      pcsf_orf_mode orf, int32_t min_codons, bool fit, bool want_anc, bool want_bls, ScoredRegions *out) {
+    const int nl = m->host.nl;
+    cudaStream_t st = m->own_stream;
+    pcsf_status rc;
+    if ((rc = stage_and_pack(m, n_aln, seqs, offset, len, col_start, Ltot, st))) return rc;
+
+    // per-unit buffers: col_start | len | ref_row | totals | n_reg | n_win | bsums x 2 | off_r | off_w
+    const int64_t n_units = (int64_t)n_aln * frames;
+    const uint32_t nsb = (uint32_t)((n_units + SCAN_BLOCK - 1) / SCAN_BLOCK);
+    size_t o = 0;
+    auto take = [&](size_t bytes) { const size_t r = o; o += (bytes + 255) / 256 * 256; return r; };
+    const size_t o_cs = take((size_t)n_aln * 8), o_len = take((size_t)n_aln * 8), o_ref = take((size_t)n_aln * 4), o_tot = take(16),
+                 o_nr = take((size_t)n_units * 4), o_nw = take((size_t)n_units * 4), o_br = take((size_t)(nsb + 1) * 4),
+                 o_bw = take((size_t)(nsb + 1) * 4), o_or = take((size_t)(n_units + 1) * 8), o_ow = take((size_t)(n_units + 1) * 8);
+    CK(m->rg_units.reserve(o));
+    unsigned char *ub = m->rg_units.as<unsigned char>();
+    CK(cudaMemcpyAsync(ub + o_cs, col_start, (size_t)n_aln * 8, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(ub + o_len, len, (size_t)n_aln * 8, cudaMemcpyHostToDevice, st));
+    if (ref_row) CK(cudaMemcpyAsync(ub + o_ref, ref_row, (size_t)n_aln * 4, cudaMemcpyHostToDevice, st));
+    CK(cudaMemsetAsync(ub + o_tot, 0, 16, st));
+    unsigned long long *d_tot = reinterpret_cast<unsigned long long *>(ub + o_tot);
+    uint32_t *d_nr = reinterpret_cast<uint32_t *>(ub + o_nr), *d_nw = reinterpret_cast<uint32_t *>(ub + o_nw);
+    uint32_t *d_br = reinterpret_cast<uint32_t *>(ub + o_br), *d_bw = reinterpret_cast<uint32_t *>(ub + o_bw);
+    int64_t *d_or = reinterpret_cast<int64_t *>(ub + o_or), *d_ow = reinterpret_cast<int64_t *>(ub + o_ow);
+    RegionUnits U{m->codes.as<uint8_t>(), m->codes_ld, n_aln, frames, (int)orf, min_codons, reinterpret_cast<const int64_t *>(ub + o_cs),
+                  reinterpret_cast<const int64_t *>(ub + o_len), ref_row ? reinterpret_cast<const int32_t *>(ub + o_ref) : nullptr};
+    const unsigned warp_blocks = (unsigned)((n_units * 32 + 255) / 256);
+    {
+        NvtxRange nvtx_e("pcsf: region enumeration");
+        m->launches += 6;
+        k_orf_count<<<warp_blocks, 256, 0, st>>>(U, n_units, d_nr, d_nw, d_tot);
+        k_scan_blocks<<<nsb, SCAN_THREADS, 0, st>>>(d_nr, (uint32_t)n_units, d_br);
+        k_scan_sums<<<1, 1024, 0, st>>>(d_br, nsb, d_br + nsb);
+        k_scan_blocks<<<nsb, SCAN_THREADS, 0, st>>>(d_nw, (uint32_t)n_units, d_bw);
+        k_scan_sums<<<1, 1024, 0, st>>>(d_bw, nsb, d_bw + nsb);
+        k_unit_offsets<<<(unsigned)((n_units + 1 + 255) / 256), 256, 0, st>>>(n_units, d_nr, d_br, d_nw, d_bw, d_tot, d_or, d_ow);
+        CK(cudaGetLastError());
+    }
+    unsigned long long tot[2] = {0, 0};
+    CK(cudaMemcpyAsync(tot, d_tot, 16, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    // the 32-bit scans above are exact only below 2^32; the window lists (uint32 ids, int counts in the fits) need < 2^31
+    if (tot[0] >= (1ull << 31) || tot[1] >= (1ull << 31)) return fail(PCSF_ERR_INVALID, "too many regions or region codons: split the call");
+    const int64_t nreg = (int64_t)tot[0], nwin = (int64_t)tot[1];
+
+    // per-region buffers: aln | fi | k0 | ncod | win_start | slen | phylo | anc | bls | records
+    o = 0;
+    const size_t nr1 = (size_t)std::max<int64_t>(nreg, 1);
+    const size_t o_ra = take(nr1 * 4), o_rf = take(nr1 * 4), o_rk = take(nr1 * 8), o_rn = take(nr1 * 8), o_rw = take(nr1 * 8),
+                 o_rl = take(nr1 * 8), o_ph = take(nr1 * 4), o_an = take(nr1 * 4), o_bl = take(nr1 * 4),
+                 o_rec = take((size_t)std::max<int64_t>({nreg, n_aln, 1}) * sizeof(pcsf_region));
+    CK(m->rg_regions.reserve(o));
+    unsigned char *rb = m->rg_regions.as<unsigned char>();
+    RegionList R{reinterpret_cast<int32_t *>(rb + o_ra), reinterpret_cast<int32_t *>(rb + o_rf), reinterpret_cast<int64_t *>(rb + o_rk),
+                 reinterpret_cast<int64_t *>(rb + o_rn), reinterpret_cast<int64_t *>(rb + o_rw), reinterpret_cast<int64_t *>(rb + o_rl)};
+    float *d_phylo = reinterpret_cast<float *>(rb + o_ph), *d_anc = reinterpret_cast<float *>(rb + o_an),
+          *d_bls = reinterpret_cast<float *>(rb + o_bl);
+    CK(m->rg_win.reserve((size_t)std::max<int64_t>(nwin, 1) * 5 + 16));
+    uint32_t *d_woff = m->rg_win.as<uint32_t>();
+    // only the minus frames (-1 -2 -3, in six-frame calls) have '-' windows: otherwise the window consumers read no strand at all
+    uint8_t *d_wstr = frames == 6 ? m->rg_win.as<uint8_t>() + (size_t)std::max<int64_t>(nwin, 1) * 4 : nullptr;
+    if (nreg > 0) {
+        NvtxRange nvtx_w("pcsf: region windows");
+        m->launches += 2;
+        k_orf_emit<<<warp_blocks, 256, 0, st>>>(U, n_units, d_or, d_ow, R);
+        k_region_windows<<<(unsigned)std::min<int64_t>((nreg * 32 + 255) / 256, (int64_t)m->sm_count * 32), 256, 0, st>>>(U, nreg, R, d_woff,
+                                                                                                                           d_wstr);
+        CK(cudaGetLastError());
+    }
+    double *d_blraw = nullptr;
+    if (want_bls && nreg > 0) {
+        CK(m->io_out.reserve((size_t)Ltot * 8 + 64));
+        d_blraw = m->io_out.as<double>();
+        if ((rc = run_bls(m, Ltot, 1, d_blraw, st))) return rc;
+    }
+    const unsigned rgrid = (unsigned)((nreg + 127) / 128);
+    WinSpace ws{m->codes.as<uint8_t>(), m->codes_ld, nl, 1, 0, d_woff, d_wstr};
+    if (nreg > 0 && fit && strategy == PCSF_STRATEGY_FIXED) {
+        CK(m->perwin.reserve((size_t)std::max<int64_t>(nwin, 1) * 32));
+        if (nwin > 0) {
+            float t0 = 0, t1 = 0, t2 = 0;
+            if ((rc = dedup_and_prune(m, ws, (uint32_t)nwin, true, want_anc, 0, m->d_nuniq, nullptr, 0, st, &t0, &t1, &t2))) return rc;
+            k_scatter_list<<<(unsigned)((nwin + 255) / 256), 256, 0, st>>>(
+                (uint32_t)nwin, m->pidx.as<uint32_t>(), m->logz.as<double>(), m->logz.as<double>() + nwin,
+                want_anc ? m->anc.as<double>() : nullptr, want_anc ? m->anc.as<double>() + nwin : nullptr, m->perwin.as<double>());
+            CK(cudaGetLastError());
+        }
+        k_region_sums<<<rgrid, 128, 0, st>>>(U, nreg, R, m->perwin.as<double>(), nwin, d_blraw, m->host.bls_all, d_phylo,
+                                             want_anc ? d_anc : nullptr, want_bls ? d_bls : nullptr);
+        CK(cudaGetLastError());
+    } else if (nreg > 0) {
+        if (fit && strategy == PCSF_STRATEGY_OMEGA) {
+            OmegaBatch b{};
+            b.n_aln = (int)nreg;
+            b.d_win_start = R.win_start;
+            b.d_len = R.slen;
+            b.ws = ws;
+            b.nwin = nwin;
+            b.d_phylo = d_phylo;
+            if ((rc = omega_run(m->host, b, m->d_bl, m->d_program, m->d_pi, m->d_logpi, m->mle, m->sm_count, m->prune_smem, m->prune_nwarp, st,
+                                g_err, &m->launches)))
+                return rc;
+        } else if (fit) {
+            MleBatch b{};
+            b.n_aln = (int)nreg;
+            b.d_win_start = R.win_start;
+            b.d_len = R.slen;
+            b.ws = ws;
+            b.nwin = nwin;
+            b.want_anc = want_anc;
+            b.d_phylo = d_phylo;
+            b.d_anc = want_anc ? d_anc : nullptr;
+            if ((rc = mle_run(m->host, b, m->d_eig, m->d_bl, m->d_program, m->d_pi, m->d_logpi, m->mle, m->sm_count, m->prune_smem,
+                              m->prune_nwarp, st, g_err, &m->launches, &m->msa_stats, m->timing)))
+                return rc;
+        }
+        if (want_bls) {
+            k_region_sums<<<rgrid, 128, 0, st>>>(U, nreg, R, nullptr, 0, d_blraw, m->host.bls_all, nullptr, nullptr, d_bls);
+            CK(cudaGetLastError());
+        }
+    }
+    CK(cudaStreamSynchronize(st));
+    int bad = 0;
+    CK(cudaMemcpy(&bad, m->d_bad, sizeof(int), cudaMemcpyDeviceToHost));
+    if (bad) return fail(PCSF_ERR_BAD_CHAR, "alignment contains a character outside ACGTacgt.-Nn (reference: exit(37))");
+    *out = ScoredRegions{nreg, U, R, d_or, fit ? d_phylo : nullptr, want_anc ? d_anc : nullptr, want_bls ? d_bls : nullptr,
+                         reinterpret_cast<pcsf_region *>(rb + o_rec)};
+    return PCSF_OK;
+}
+
 extern "C" pcsf_status pcsf_score_msa(pcsf_model *m, pcsf_strategy strategy, int32_t n_aln, const uint8_t *seqs,
                                       const int64_t *offset, const int64_t *len, float *phylo, float *anc, float *bls) {
     if (!m || n_aln < 0 || (n_aln > 0 && (!seqs || !offset || !len)))
@@ -712,123 +860,28 @@ extern "C" pcsf_status pcsf_score_msa(pcsf_model *m, pcsf_strategy strategy, int
     NvtxRange nvtx_("pcsf_score_msa");
     CK(cudaSetDevice(m->device));
     if (n_aln == 0) return PCSF_OK;
-    const int nl = m->host.nl;
-    cudaStream_t st = m->own_stream;
     // concatenate the alignments along the columns into one [nl][Ltot] matrix (2 pad columns between them)
-    std::vector<int64_t> col_start(n_aln), win_start(n_aln), lens(len, len + n_aln);
+    std::vector<int64_t> col_start(n_aln);
     int64_t Ltot = 0, nwin = 0;
     for (int i = 0; i < n_aln; ++i) {
         if (len[i] < 0) return fail(PCSF_ERR_INVALID, "negative alignment length");
-        col_start[i] = Ltot; win_start[i] = nwin;
+        col_start[i] = Ltot;
         Ltot += len[i] + 2; nwin += len[i] / 3;
     }
     if (Ltot >= ((int64_t)1 << 32) || nwin >= ((int64_t)1 << 31))
         return fail(PCSF_ERR_INVALID, "batch too large: split the call");
-    std::vector<uint32_t> win_off((size_t)std::max<int64_t>(nwin, 1));
-    for (int i = 0; i < n_aln; ++i)
-        for (int64_t k = 0; k < len[i] / 3; ++k) win_off[win_start[i] + k] = (uint32_t)(col_start[i] + 3 * k);
-    pcsf_status rc;
-    if ((rc = stage_and_pack(m, n_aln, seqs, offset, len, col_start.data(), Ltot, st))) return rc;
-    // misc: win_off | col_start | win_start | len | outputs
-    const size_t o_win = 0, o_cs = o_win + ((win_off.size() * 4 + 15) / 16) * 16, o_ws = o_cs + (size_t)n_aln * 8,
-                 o_len = o_ws + (size_t)n_aln * 8, o_out = o_len + (size_t)n_aln * 8, total = o_out + (size_t)n_aln * 12 + 64;
-    CK(m->misc.reserve(total));
-    unsigned char *mb = m->misc.as<unsigned char>();
-    CK(cudaMemcpyAsync(mb + o_win, win_off.data(), win_off.size() * 4, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(mb + o_cs, col_start.data(), (size_t)n_aln * 8, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(mb + o_ws, win_start.data(), (size_t)n_aln * 8, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(mb + o_len, lens.data(), (size_t)n_aln * 8, cudaMemcpyHostToDevice, st));
-    float *d_phylo = reinterpret_cast<float *>(mb + o_out), *d_anc = d_phylo + n_aln, *d_bls = d_anc + n_aln;
-    CK(m->io_out.reserve((size_t)Ltot * 8 + 64));
-    double *d_blraw = m->io_out.as<double>();
-    if (bls) {
-        if ((rc = run_bls(m, Ltot, 1, d_blraw, st))) return rc;
-    }
-    WinSpace ws{m->codes.as<uint8_t>(), m->codes_ld, nl, 1, 0, reinterpret_cast<const uint32_t *>(mb + o_win)};
-    if (!phylo && !anc) {
-        // nothing but the branch length score is asked for: the reference does not call run() at all then (score_msa.hpp:112),
-        // whatever the strategy — no fit, and no way for a failing fit to turn the batch into an error
-        if (bls) {
-            CK(m->perwin.reserve(64));
-            k_aln_sums<<<(n_aln + 127) / 128, 128, 0, st>>>(n_aln, reinterpret_cast<const int64_t *>(mb + o_ws),
-                                                           reinterpret_cast<const int64_t *>(mb + o_cs),
-                                                           reinterpret_cast<const int64_t *>(mb + o_len), m->perwin.as<double>(),
-                                                           0, d_blraw, m->host.bls_all, nullptr, nullptr, d_bls);
-            CK(cudaGetLastError());
-        }
-    } else if (strategy == PCSF_STRATEGY_FIXED) {
-        CK(m->perwin.reserve((size_t)std::max<int64_t>(nwin, 1) * 32));
-        if (nwin > 0) {
-            float t0 = 0, t1 = 0, t2 = 0;
-            if ((rc = dedup_and_prune(m, ws, (uint32_t)nwin, true, anc != nullptr, 0, m->d_nuniq, nullptr, 0, st, &t0, &t1, &t2)))
-                return rc;
-            k_scatter_list<<<(unsigned)((nwin + 255) / 256), 256, 0, st>>>(
-                (uint32_t)nwin, m->pidx.as<uint32_t>(), m->logz.as<double>(), m->logz.as<double>() + nwin,
-                anc ? m->anc.as<double>() : nullptr, anc ? m->anc.as<double>() + nwin : nullptr, m->perwin.as<double>());
-            CK(cudaGetLastError());
-        }
-        k_aln_sums<<<(n_aln + 127) / 128, 128, 0, st>>>(n_aln, reinterpret_cast<const int64_t *>(mb + o_ws),
-                                                       reinterpret_cast<const int64_t *>(mb + o_cs),
-                                                       reinterpret_cast<const int64_t *>(mb + o_len), m->perwin.as<double>(),
-                                                       nwin, d_blraw, m->host.bls_all, phylo ? d_phylo : nullptr,
-                                                       anc ? d_anc : nullptr, bls ? d_bls : nullptr);
-        CK(cudaGetLastError());
-    } else if (strategy == PCSF_STRATEGY_OMEGA) {
-        OmegaBatch b{};
-        b.n_aln = n_aln;
-        b.d_win_start = reinterpret_cast<const int64_t *>(mb + o_ws);
-        b.d_len = reinterpret_cast<const int64_t *>(mb + o_len);
-        b.ws = ws;
-        b.nwin = nwin;
-        b.d_phylo = phylo ? d_phylo : nullptr;
-        if ((rc = omega_run(m->host, b, m->d_bl, m->d_program, m->d_pi, m->d_logpi, m->mle, m->sm_count, m->prune_smem, m->prune_nwarp, st,
-                            g_err, &m->launches)))
-            return rc;
-        if (bls) {
-            CK(m->perwin.reserve(64));
-            k_aln_sums<<<(n_aln + 127) / 128, 128, 0, st>>>(n_aln, reinterpret_cast<const int64_t *>(mb + o_ws),
-                                                           reinterpret_cast<const int64_t *>(mb + o_cs),
-                                                           reinterpret_cast<const int64_t *>(mb + o_len), m->perwin.as<double>(),
-                                                           0, d_blraw, m->host.bls_all, nullptr, nullptr, d_bls);
-            CK(cudaGetLastError());
-        }
-    } else {
-        MleBatch b{};
-        b.n_aln = n_aln;
-        b.d_win_start = reinterpret_cast<const int64_t *>(mb + o_ws);
-        b.d_col_start = reinterpret_cast<const int64_t *>(mb + o_cs);
-        b.d_len = reinterpret_cast<const int64_t *>(mb + o_len);
-        b.ws = ws;
-        b.nwin = nwin;
-        b.want_anc = anc != nullptr;
-        b.d_phylo = phylo ? d_phylo : nullptr;
-        b.d_anc = anc ? d_anc : nullptr;
-        if ((rc = mle_run(m->host, b, m->d_eig, m->d_bl, m->d_program, m->d_pi, m->d_logpi, m->mle, m->sm_count,
-                          m->prune_smem, m->prune_nwarp, st, g_err, &m->launches, &m->msa_stats, m->timing)))
-            return rc;
-        // BLS for MLE uses the same per-alignment sum kernel with phylo/anc disabled
-        if (bls) {
-            CK(m->perwin.reserve(64));
-            k_aln_sums<<<(n_aln + 127) / 128, 128, 0, st>>>(n_aln, reinterpret_cast<const int64_t *>(mb + o_ws),
-                                                           reinterpret_cast<const int64_t *>(mb + o_cs),
-                                                           reinterpret_cast<const int64_t *>(mb + o_len), m->perwin.as<double>(),
-                                                           0, d_blraw, m->host.bls_all, nullptr, nullptr, d_bls);
-            CK(cudaGetLastError());
-        }
-    }
-    CK(cudaStreamSynchronize(st));
-    int bad = 0;
-    CK(cudaMemcpy(&bad, m->d_bad, sizeof(int), cudaMemcpyDeviceToHost));
-    if (bad) return fail(PCSF_ERR_BAD_CHAR, "alignment contains a character outside ACGTacgt.-Nn (reference: exit(37))");
-    if (phylo) CK(cudaMemcpy(phylo, d_phylo, (size_t)n_aln * 4, cudaMemcpyDeviceToHost));
+    // Frame +1 as is: region i is alignment i.  With nothing but the branch length score asked for, the reference does not call run()
+    // at all (score_msa.hpp:112), whatever the strategy — no fit, and no way for a failing fit to turn the batch into an error.
+    ScoredRegions r;
+    pcsf_status rc = score_regions_core(m, strategy, n_aln, seqs, offset, len, col_start.data(), Ltot, nullptr, 1, PCSF_ORF_ASIS, 1,
+                                        phylo || anc, anc && strategy != PCSF_STRATEGY_OMEGA, bls != nullptr, &r);
+    if (rc) return rc;
+    if (phylo) CK(cudaMemcpy(phylo, r.phylo, (size_t)n_aln * 4, cudaMemcpyDeviceToHost));
     if (anc && strategy == PCSF_STRATEGY_OMEGA) { for (int i = 0; i < n_aln; ++i) anc[i] = nanf(""); }
-    else if (anc) CK(cudaMemcpy(anc, d_anc, (size_t)n_aln * 4, cudaMemcpyDeviceToHost));
-    if (bls) CK(cudaMemcpy(bls, d_bls, (size_t)n_aln * 4, cudaMemcpyDeviceToHost));
+    else if (anc) CK(cudaMemcpy(anc, r.anc, (size_t)n_aln * 4, cudaMemcpyDeviceToHost));
+    if (bls) CK(cudaMemcpy(bls, r.bls, (size_t)n_aln * 4, cudaMemcpyDeviceToHost));
     return PCSF_OK;
 }
-
-// ---- score-msa over reading frames / ORFs -----------------------------------------------------------
-static_assert(sizeof(pcsf_region) == 48, "pcsf_region layout is part of the ABI");
 
 extern "C" pcsf_status pcsf_score_regions(pcsf_model *m, pcsf_strategy strategy, int32_t n_aln, const uint8_t *seqs, const int64_t *offset,
                                           const int64_t *len, const int32_t *ref_row, int32_t frames, pcsf_orf_mode orf, int32_t min_codons,
@@ -859,139 +912,22 @@ extern "C" pcsf_status pcsf_score_regions(pcsf_model *m, pcsf_strategy strategy,
     NvtxRange nvtx_("pcsf_score_regions");
     CK(cudaSetDevice(m->device));
     if (n_aln == 0) return PCSF_OK;
+    ScoredRegions r;
+    pcsf_status rc = score_regions_core(m, strategy, n_aln, seqs, offset, len, col_start.data(), Ltot, ref_row, frames, orf, min_codons,
+                                        true, want_anc != 0, want_bls != 0, &r);
+    if (rc) return rc;
     cudaStream_t st = m->own_stream;
-    pcsf_status rc;
-    if ((rc = stage_and_pack(m, n_aln, seqs, offset, len, col_start.data(), Ltot, st))) return rc;
-
-    // per-unit buffers: col_start | len | ref_row | totals | n_reg | n_win | bsums x 2 | off_r | off_w
-    const uint32_t nsb = (uint32_t)((n_units + SCAN_BLOCK - 1) / SCAN_BLOCK);
-    size_t o = 0;
-    auto take = [&](size_t bytes) { const size_t r = o; o += (bytes + 255) / 256 * 256; return r; };
-    const size_t o_cs = take((size_t)n_aln * 8), o_len = take((size_t)n_aln * 8), o_ref = take((size_t)n_aln * 4), o_tot = take(16),
-                 o_nr = take((size_t)n_units * 4), o_nw = take((size_t)n_units * 4), o_br = take((size_t)(nsb + 1) * 4),
-                 o_bw = take((size_t)(nsb + 1) * 4), o_or = take((size_t)(n_units + 1) * 8), o_ow = take((size_t)(n_units + 1) * 8);
-    CK(m->rg_units.reserve(o));
-    unsigned char *ub = m->rg_units.as<unsigned char>();
-    CK(cudaMemcpyAsync(ub + o_cs, col_start.data(), (size_t)n_aln * 8, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(ub + o_len, len, (size_t)n_aln * 8, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(ub + o_ref, ref_row, (size_t)n_aln * 4, cudaMemcpyHostToDevice, st));
-    CK(cudaMemsetAsync(ub + o_tot, 0, 16, st));
-    unsigned long long *d_tot = reinterpret_cast<unsigned long long *>(ub + o_tot);
-    uint32_t *d_nr = reinterpret_cast<uint32_t *>(ub + o_nr), *d_nw = reinterpret_cast<uint32_t *>(ub + o_nw);
-    uint32_t *d_br = reinterpret_cast<uint32_t *>(ub + o_br), *d_bw = reinterpret_cast<uint32_t *>(ub + o_bw);
-    int64_t *d_or = reinterpret_cast<int64_t *>(ub + o_or), *d_ow = reinterpret_cast<int64_t *>(ub + o_ow);
-    RegionUnits U{m->codes.as<uint8_t>(), m->codes_ld, n_aln, frames, (int)orf, min_codons, reinterpret_cast<const int64_t *>(ub + o_cs),
-                  reinterpret_cast<const int64_t *>(ub + o_len), reinterpret_cast<const int32_t *>(ub + o_ref)};
-    const unsigned warp_blocks = (unsigned)((n_units * 32 + 255) / 256);
-    {
-        NvtxRange nvtx_e("pcsf: region enumeration");
-        m->launches += 6;
-        k_orf_count<<<warp_blocks, 256, 0, st>>>(U, n_units, d_nr, d_nw, d_tot);
-        k_scan_blocks<<<nsb, SCAN_THREADS, 0, st>>>(d_nr, (uint32_t)n_units, d_br);
-        k_scan_sums<<<1, 1024, 0, st>>>(d_br, nsb, d_br + nsb);
-        k_scan_blocks<<<nsb, SCAN_THREADS, 0, st>>>(d_nw, (uint32_t)n_units, d_bw);
-        k_scan_sums<<<1, 1024, 0, st>>>(d_bw, nsb, d_bw + nsb);
-        k_unit_offsets<<<(unsigned)((n_units + 1 + 255) / 256), 256, 0, st>>>(n_units, d_nr, d_br, d_nw, d_bw, d_tot, d_or, d_ow);
-        CK(cudaGetLastError());
-    }
-    unsigned long long tot[2] = {0, 0};
-    CK(cudaMemcpyAsync(tot, d_tot, 16, cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
-    // the 32-bit scans above are exact only below 2^32; the window lists (uint32 ids, int counts in the fits) need < 2^31
-    if (tot[0] >= (1ull << 31) || tot[1] >= (1ull << 31)) return fail(PCSF_ERR_INVALID, "too many regions or region codons: split the call");
-    const int64_t nreg = (int64_t)tot[0], nwin = (int64_t)tot[1];
-    const int64_t n_out = best_only ? n_aln : nreg;
-
-    // per-region buffers: aln | fi | k0 | ncod | win_start | slen | phylo | anc | bls | records
-    o = 0;
-    const size_t nr1 = (size_t)std::max<int64_t>(nreg, 1);
-    const size_t o_ra = take(nr1 * 4), o_rf = take(nr1 * 4), o_rk = take(nr1 * 8), o_rn = take(nr1 * 8), o_rw = take(nr1 * 8),
-                 o_rl = take(nr1 * 8), o_ph = take(nr1 * 4), o_an = take(nr1 * 4), o_bl = take(nr1 * 4),
-                 o_rec = take((size_t)std::max<int64_t>(n_out, 1) * sizeof(pcsf_region));
-    CK(m->rg_regions.reserve(o));
-    unsigned char *rb = m->rg_regions.as<unsigned char>();
-    RegionList R{reinterpret_cast<int32_t *>(rb + o_ra), reinterpret_cast<int32_t *>(rb + o_rf), reinterpret_cast<int64_t *>(rb + o_rk),
-                 reinterpret_cast<int64_t *>(rb + o_rn), reinterpret_cast<int64_t *>(rb + o_rw), reinterpret_cast<int64_t *>(rb + o_rl)};
-    float *d_phylo = reinterpret_cast<float *>(rb + o_ph), *d_anc = reinterpret_cast<float *>(rb + o_an),
-          *d_bls = reinterpret_cast<float *>(rb + o_bl);
-    pcsf_region *d_rec = reinterpret_cast<pcsf_region *>(rb + o_rec);
-    CK(m->rg_win.reserve((size_t)std::max<int64_t>(nwin, 1) * 5 + 16));
-    uint32_t *d_woff = m->rg_win.as<uint32_t>();
-    uint8_t *d_wstr = m->rg_win.as<uint8_t>() + (size_t)std::max<int64_t>(nwin, 1) * 4;
-    if (nreg > 0) {
-        NvtxRange nvtx_w("pcsf: region windows");
-        m->launches += 2;
-        k_orf_emit<<<warp_blocks, 256, 0, st>>>(U, n_units, d_or, d_ow, R);
-        k_region_windows<<<(unsigned)std::min<int64_t>((nreg * 32 + 255) / 256, (int64_t)m->sm_count * 32), 256, 0, st>>>(U, nreg, R, d_woff,
-                                                                                                                           d_wstr);
-        CK(cudaGetLastError());
-    }
-    double *d_blraw = nullptr;
-    if (want_bls && nreg > 0) {
-        CK(m->io_out.reserve((size_t)Ltot * 8 + 64));
-        d_blraw = m->io_out.as<double>();
-        if ((rc = run_bls(m, Ltot, 1, d_blraw, st))) return rc;
-    }
-    const unsigned rgrid = (unsigned)((nreg + 127) / 128);
-    WinSpace ws{m->codes.as<uint8_t>(), m->codes_ld, nl, 1, 0, d_woff, d_wstr};
-    if (nreg > 0 && strategy == PCSF_STRATEGY_FIXED) {
-        CK(m->perwin.reserve((size_t)std::max<int64_t>(nwin, 1) * 32));
-        if (nwin > 0) {
-            float t0 = 0, t1 = 0, t2 = 0;
-            if ((rc = dedup_and_prune(m, ws, (uint32_t)nwin, true, want_anc != 0, 0, m->d_nuniq, nullptr, 0, st, &t0, &t1, &t2))) return rc;
-            k_scatter_list<<<(unsigned)((nwin + 255) / 256), 256, 0, st>>>(
-                (uint32_t)nwin, m->pidx.as<uint32_t>(), m->logz.as<double>(), m->logz.as<double>() + nwin,
-                want_anc ? m->anc.as<double>() : nullptr, want_anc ? m->anc.as<double>() + nwin : nullptr, m->perwin.as<double>());
-            CK(cudaGetLastError());
-        }
-        k_region_sums<<<rgrid, 128, 0, st>>>(U, nreg, R, m->perwin.as<double>(), nwin, d_blraw, m->host.bls_all, d_phylo,
-                                             want_anc ? d_anc : nullptr, want_bls ? d_bls : nullptr);
-        CK(cudaGetLastError());
-    } else if (nreg > 0) {
-        if (strategy == PCSF_STRATEGY_OMEGA) {
-            OmegaBatch b{};
-            b.n_aln = (int)nreg;
-            b.d_win_start = R.win_start;
-            b.d_len = R.slen;
-            b.ws = ws;
-            b.nwin = nwin;
-            b.d_phylo = d_phylo;
-            if ((rc = omega_run(m->host, b, m->d_bl, m->d_program, m->d_pi, m->d_logpi, m->mle, m->sm_count, m->prune_smem, m->prune_nwarp, st,
-                                g_err, &m->launches)))
-                return rc;
-        } else {
-            MleBatch b{};
-            b.n_aln = (int)nreg;
-            b.d_win_start = R.win_start;
-            b.d_len = R.slen;
-            b.ws = ws;
-            b.nwin = nwin;
-            b.want_anc = want_anc != 0;
-            b.d_phylo = d_phylo;
-            b.d_anc = want_anc ? d_anc : nullptr;
-            if ((rc = mle_run(m->host, b, m->d_eig, m->d_bl, m->d_program, m->d_pi, m->d_logpi, m->mle, m->sm_count, m->prune_smem,
-                              m->prune_nwarp, st, g_err, &m->launches, &m->msa_stats, m->timing)))
-                return rc;
-        }
-        if (want_bls) {
-            k_region_sums<<<rgrid, 128, 0, st>>>(U, nreg, R, nullptr, 0, d_blraw, m->host.bls_all, nullptr, nullptr, d_bls);
-            CK(cudaGetLastError());
-        }
-    }
-    const float *r_anc = want_anc ? d_anc : nullptr, *r_bls = want_bls ? d_bls : nullptr;
+    const int64_t n_out = best_only ? n_aln : r.nreg;
     if (best_only) {
-        k_best_region<<<(unsigned)(((int64_t)n_aln * 32 + 255) / 256), 256, 0, st>>>(U, R, d_or, d_phylo, r_anc, r_bls, d_rec);
+        k_best_region<<<(unsigned)(((int64_t)n_aln * 32 + 255) / 256), 256, 0, st>>>(r.U, r.R, r.off_r, r.phylo, r.anc, r.bls, r.rec);
         CK(cudaGetLastError());
-    } else if (nreg > 0) {
-        k_region_records<<<rgrid, 128, 0, st>>>(U, nreg, R, d_phylo, r_anc, r_bls, d_rec);
+    } else if (r.nreg > 0) {
+        k_region_records<<<(unsigned)((r.nreg + 127) / 128), 128, 0, st>>>(r.U, r.nreg, r.R, r.phylo, r.anc, r.bls, r.rec);
         CK(cudaGetLastError());
     }
-    CK(cudaStreamSynchronize(st));
-    int bad = 0;
-    CK(cudaMemcpy(&bad, m->d_bad, sizeof(int), cudaMemcpyDeviceToHost));
-    if (bad) return fail(PCSF_ERR_BAD_CHAR, "alignment contains a character outside ACGTacgt.-Nn (reference: exit(37))");
     m->regions.resize((size_t)n_out);
-    if (n_out > 0) CK(cudaMemcpy(m->regions.data(), d_rec, (size_t)n_out * sizeof(pcsf_region), cudaMemcpyDeviceToHost));
+    if (n_out > 0) CK(cudaMemcpyAsync(m->regions.data(), r.rec, (size_t)n_out * sizeof(pcsf_region), cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
     *n_regions = n_out;
     return PCSF_OK;
 }

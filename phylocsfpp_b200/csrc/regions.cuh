@@ -127,7 +127,8 @@ __global__ void __launch_bounds__(256) k_orf_emit(RegionUnits U, int64_t n_units
     orf_walk<true>(U, u, off_r[u], off_w[u], R, nullptr, nullptr);
 }
 
-// One warp per region (grid-stride): window k of region r is codon k0 + k of its frame, at its column in the batch.
+// One warp per region (grid-stride): window k of region r is codon k0 + k of its frame, at its column in the batch.  win_strand is
+// null when no region lies on the '-' strand.
 __global__ void __launch_bounds__(256) k_region_windows(RegionUnits U, int64_t n_reg, RegionList R, uint32_t *__restrict__ win_off,
                                                         uint8_t *__restrict__ win_strand) {
     const int lane = threadIdx.x & 31;
@@ -138,7 +139,7 @@ __global__ void __launch_bounds__(256) k_region_windows(RegionUnits U, int64_t n
         for (int64_t k = lane; k < n; k += 32) {
             const int64_t kk = k0 + k;
             win_off[w0 + k] = (uint32_t)(cs + (minus ? len - 3 - f - 3 * kk : f + 3 * kk));
-            win_strand[w0 + k] = minus ? 1 : 0;
+            if (win_strand) win_strand[w0 + k] = minus ? 1 : 0;
         }
     }
 }
@@ -154,8 +155,9 @@ __device__ __forceinline__ void region_columns(const RegionUnits &U, const Regio
     else { *begin = len - (w + R.slen[r]); *end = len - w; }
 }
 
-// k_aln_sums for regions: lpr / anc in W codon order; BLS over S(r)'s columns in S(r)'s order, i.e. descending original columns on
-// the '-' strand.  The same expressions as k_aln_sums, so a region's floats equal pcsf_score_msa's on the extracted S(r).
+// Per-region sums, one thread per region, sequential in the reference's order: lpr += log z per codon (fixed_lik.hpp:431-432),
+// elpr_anc += ... (:440) in W codon order; bl_total += bl (additional_scores.hpp:71) over S(r)'s columns in S(r)'s order, i.e.
+// descending original columns on the '-' strand.  So a region's floats equal pcsf_score_msa's on the extracted S(r).
 __global__ void k_region_sums(RegionUnits U, int64_t n_reg, RegionList R, const double *__restrict__ perwin /* [4][nwin] */,
                               int64_t nwin, const double *__restrict__ bl_raw, double bls_all, float *__restrict__ phylo,
                               float *__restrict__ anc, float *__restrict__ bls) {

@@ -164,6 +164,20 @@ def test_numeric_violation_gives_nan_rows_and_model_error():
     assert ei.value.status == capi.PCSF_ERR_NUMERIC
 
 
+@pytest.mark.parametrize("strategy", [capi.STRATEGY_FIXED, capi.STRATEGY_MLE, capi.STRATEGY_OMEGA])
+def test_bls_only_call(strategy):
+    """phylo = anc = NULL: the call succeeds without a fit (the reference does not call run() then, score_msa.hpp:112) and its BLS
+    equals the full call's bit for bit."""
+    model = load_model("12flies")
+    dm = capi.DeviceModel(model)
+    alns = [random_alignment(model.nl, L, seed=500 + L, gap=0.2) for L in (0, 1, 2, 3, 5, 30, 61, 150)]
+    phylo, anc, bls = dm.score_msa(alns, strategy, comp_phylo=False, comp_anc=False)
+    assert phylo is None and anc is None
+    _, _, full = dm.score_msa(alns, strategy)
+    assert np.array_equal(bls.view(np.uint32), full.view(np.uint32))
+    dm.close()
+
+
 def test_mle_vs_oracle_random():
     model = load_model("29mammals", "Human,Chimp,Mouse,Dog,Cow,Horse,Elephant,Armadillo,Rat,Rabbit,Cat,Megabat")
     dm = capi.DeviceModel(model)

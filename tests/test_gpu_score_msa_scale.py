@@ -12,7 +12,7 @@ import numpy as np
 import pytest
 
 from oracle import oracle as orc
-from phylocsfpp_b200 import capi
+from phylocsfpp_b200 import capi, orf
 from phylocsfpp_b200.models import load_model
 from tests.util import random_alignment
 
@@ -299,16 +299,44 @@ def test_fixed_config5_size():
     dm.close()
 
 
+def _regions(dm, alns):
+    return dm.score_regions(alns, np.arange(len(alns)) % dm.nl, capi.STRATEGY_MLE, 6, orf.ATGSTOP, 25)
+
+
+def _same_records(x, y):
+    return (len(x) == len(y) and all(np.array_equal(x[k], y[k]) for k in ("aln", "strand", "frame", "col_begin", "col_end", "codons"))
+            and all(_same(x[k], y[k]) for k in ("phylo", "anc", "bls")))
+
+
+def _last_records(dm, n):
+    out = np.zeros(n, capi.REGION_DTYPE)
+    capi._check(capi.load().pcsf_score_regions_get(dm.h, out.ctypes.data if n else None, n))
+    return out
+
+
 def test_handle_reuse_small_large_small():
-    """One handle scores a small batch, a large one (the page-locked staging and the scratch reservation grow), then the small
-    one again; each equals what a fresh handle computes."""
+    """One handle alternates score_msa and six-frame ATG-to-stop score_regions calls (which share the staging and the scratch) on
+    a small batch, a large one (the page-locked staging and the scratch reservations grow), then the small one again; each equals
+    what a fresh handle computes, and a score_msa call leaves the records of the last score_regions call in place."""
     model = load_model("29mammals", SPECIES12)
     small = _batch(model.nl, _lengths(40, 30, 300, 8, tiny=(0, 4)), 800)
     large = _batch(model.nl, _lengths(9000, 30, 600, 9), 900)
+    calls = [("msa", small), ("regions", large), ("msa", small), ("msa", large), ("regions", small), ("msa", small)]
     dm = capi.DeviceModel(model)
-    seq = [dm.score_msa(b, capi.STRATEGY_MLE) for b in (small, large, small)]
+    seq, last = [], None
+    for kind, b in calls:
+        if kind == "msa":
+            seq.append(dm.score_msa(b, capi.STRATEGY_MLE))
+            if last is not None:
+                assert _same_records(_last_records(dm, len(last)), last)
+        else:
+            last = _regions(dm, b)
+            seq.append(last)
     dm.close()
-    for b, got in zip((small, large, small), seq):
+    for (kind, b), got in zip(calls, seq):
         fresh = capi.DeviceModel(model)
-        _assert_same(got, fresh.score_msa(b, capi.STRATEGY_MLE), f"reused handle, batch of {len(b)}")
+        if kind == "msa":
+            _assert_same(got, fresh.score_msa(b, capi.STRATEGY_MLE), f"reused handle, score_msa, batch of {len(b)}")
+        else:
+            assert len(got) > 0 and _same_records(got, _regions(fresh, b)), f"reused handle, score_regions, batch of {len(b)}"
         fresh.close()
