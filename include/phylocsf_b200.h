@@ -45,7 +45,11 @@ typedef enum {
     PCSF_ERR_BAD_CHAR = 37     /* mirrors the reference's exit(37) */
 } pcsf_status;
 
-#define PCSF_MAX_LEAVES 128
+/* Largest species tree pcsf_model_create accepts.  At 512 leaves the FP64 pruning kernel's per-warp stack of sibling partials still
+ * fits one SM's shared memory for every tree shape (a balanced tree is the deepest).  Trees of more than 128 leaves are pruned with
+ * an exact power-of-two rescaling per window, so their likelihoods do not underflow where the reference's unscaled product does, and
+ * they have no tcgen05 path (PCSF_TRACKS_TC5 returns PCSF_ERR_UNSUPPORTED). */
+#define PCSF_MAX_LEAVES 512
 
 /* Flattened species tree + the two empirical codon models: what `struct Model` (src/models.hpp:1742)
  * holds after load_model.  Node ids follow newick_flatten (src/newick.hpp:218): leaves 0..nl-1 in DFS

@@ -464,12 +464,34 @@ __host__ __device__ inline size_t prune_smem_bytes(int nl, int n_ops, int max_st
     b += (size_t)((n_ops * 4 + 15) / 16) * 16;               // program
     b += 4 * 64 * 8;                                         // pi, logpi x 2 models
     b += 2 * PR_NSTAGE * 8;                                  // mbarriers
+    if (nl > SMALL_TREE_MAX_LEAVES) b += (size_t)nwarp * (max_stack > 0 ? max_stack : 1) * 32 * 4;   // exponents of the stack (k_prune_scaled)
     return b;
 }
 
-template <bool PER_TILE>
-__global__ void __launch_bounds__(PR_THREADS, 1) k_prune(const PruneArgs a) {
-    extern __shared__ __align__(128) unsigned char smem[];
+// k_prune_scaled (trees above SMALL_TREE_MAX_LEAVES leaves): an unscaled FP64 likelihood of a few hundred species can fall below the
+// double range.  Every window carries an integer exponent e with true partial = R * 2^-e.  After each step that can shrink the partial
+// (GEMM, leaf or stack Hadamard product), a window whose largest entry is below 2^-512 is multiplied by an exact power of two that brings
+// that entry to [1, 2).  A window that never falls below the threshold keeps e = 0 and the unscaled arithmetic, bit for bit.
+constexpr int PR_RESCALE_BIASED_EXP = 1023 - 512;
+
+__device__ __forceinline__ void prune_rescale(double (&R)[16], int &e) {
+    double mx = R[0];
+#pragma unroll
+    for (int i = 1; i < 16; ++i) mx = fmax(mx, R[i]);
+    mx = fmax(mx, __shfl_xor_sync(0xffffffffu, mx, 1));      // the four lanes of a window
+    mx = fmax(mx, __shfl_xor_sync(0xffffffffu, mx, 2));
+    const int be = (int)((__double_as_longlong(mx) >> 52) & 0x7ff);   // partials are >= 0: biased exponent of the largest
+    if (be < PR_RESCALE_BIASED_EXP && mx > 0.0) {
+        const int k = min(1023 - be, 1022);
+        const double f = __longlong_as_double((long long)(1023 + k) << 52);   // 2^k
+#pragma unroll
+        for (int i = 0; i < 16; ++i) R[i] *= f;
+        e += k;
+    }
+}
+
+template <bool PER_TILE, bool SCALED>
+__device__ __forceinline__ void prune_body(const PruneArgs &a, unsigned char *smem) {
     unsigned char *sp_ = smem;
     const int PR_NWARP = a.nwarp, PR_TILE_W = a.nwarp * 8;
     double *stage_buf = reinterpret_cast<double *>(sp_); sp_ += (size_t)PR_NSTAGE * PR_TILE_BYTES;
@@ -480,6 +502,7 @@ __global__ void __launch_bounds__(PR_THREADS, 1) k_prune(const PruneArgs a) {
     double *s_pi = reinterpret_cast<double *>(sp_); sp_ += 4 * 64 * 8;   // [model][pi 64 | logpi 64]
     uint64_t *full = reinterpret_cast<uint64_t *>(sp_);
     uint64_t *empty = full + PR_NSTAGE;
+    int *estack = reinterpret_cast<int *>(empty + PR_NSTAGE);   // SCALED: [warp][max_stack][lane] exponents of the stacked partials
 
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     if (tid == 0) {
@@ -519,6 +542,7 @@ __global__ void __launch_bounds__(PR_THREADS, 1) k_prune(const PruneArgs a) {
     const int g = lane >> 2, q = lane & 3;
     const int mywin = warp * 8 + g;
     double2 *mystack = stack + (size_t)warp * (a.max_stack > 0 ? a.max_stack : 1) * 256;
+    int *myestack = estack + (size_t)warp * (a.max_stack > 0 ? a.max_stack : 1) * 32 + lane;
     uint32_t use = 0;
     for (uint32_t tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
         // leaf codon ids of this tile's 64 windows
@@ -564,6 +588,7 @@ __global__ void __launch_bounds__(PR_THREADS, 1) k_prune(const PruneArgs a) {
 #pragma unroll
             for (int i = 0; i < 16; ++i) R[i] = 0.0;
             int sp = 0;
+            int e2 = 0;                       // SCALED: exponent of R
             if (idle_warp) {
                 for (int pc = 0; pc < a.n_ops; ++pc) {
                     if ((prog[pc] >> 16) != OP_GEMM) continue;
@@ -587,9 +612,11 @@ __global__ void __launch_bounds__(PR_THREADS, 1) k_prune(const PruneArgs a) {
                     if (code == OP_GATHER_SET) {
 #pragma unroll
                         for (int nt = 0; nt < 8; ++nt) { R[2 * nt] = v[nt].x; R[2 * nt + 1] = v[nt].y; }
+                        if (SCALED) e2 = 0;
                     } else {
 #pragma unroll
                         for (int nt = 0; nt < 8; ++nt) { R[2 * nt] *= v[nt].x; R[2 * nt + 1] *= v[nt].y; }
+                        if (SCALED) prune_rescale(R, e2);
                     }
                 } else if (code == OP_GEMM) {
                     const uint32_t st = use % PR_NSTAGE;
@@ -613,9 +640,11 @@ __global__ void __launch_bounds__(PR_THREADS, 1) k_prune(const PruneArgs a) {
                     ++use;
 #pragma unroll
                     for (int i = 0; i < 16; ++i) R[i] = acc[i];
+                    if (SCALED) prune_rescale(R, e2);
                 } else if (code == OP_PUSH) {
 #pragma unroll
                     for (int nt = 0; nt < 8; ++nt) mystack[(sp * 8 + nt) * 32 + lane] = make_double2(R[2 * nt], R[2 * nt + 1]);
+                    if (SCALED) myestack[sp * 32] = e2;
                     ++sp;
                 } else if (code == OP_POP_MUL) {
                     --sp;
@@ -623,6 +652,10 @@ __global__ void __launch_bounds__(PR_THREADS, 1) k_prune(const PruneArgs a) {
                     for (int nt = 0; nt < 8; ++nt) {
                         const double2 v = mystack[(sp * 8 + nt) * 32 + lane];
                         R[2 * nt] *= v.x; R[2 * nt + 1] *= v.y;
+                    }
+                    if (SCALED) {
+                        e2 += myestack[sp * 32];
+                        prune_rescale(R, e2);
                     }
                 } else {  // OP_END: z = pi . alpha_root; log z; optional ancestral term
                     const double *pi = (PER_TILE && td.pi != nullptr) ? td.pi : s_pi + m * 128, *lpi = s_pi + m * 128 + 64;
@@ -646,15 +679,18 @@ __global__ void __launch_bounds__(PR_THREADS, 1) k_prune(const PruneArgs a) {
                         e += __shfl_xor_sync(0xffffffffu, e, 1);
                         e += __shfl_xor_sync(0xffffffffu, e, 2);
                     }
+                    // the ancestral term is a ratio of the scaled partials: the scale cancels in it, and only log z is corrected
+                    double lz = log(z);
+                    if (SCALED && e2 != 0) lz -= (double)e2 * 0.6931471805599453094;
                     if (PER_TILE) {
                         if (q == 0 && mywin < td.count) {
-                            a.logz[0][td.win0 + mywin] = log(z);
+                            a.logz[0][td.win0 + mywin] = lz;
                             if (a.anc[0] != nullptr) a.anc[0][td.win0 + mywin] = e;
                         }
                     } else {
                         const uint32_t u = tile * PR_TILE_W + mywin;
                         if (q == 0 && u < n_unique) {
-                            a.logz[m][u] = log(z);
+                            a.logz[m][u] = lz;
                             if (a.anc[m] != nullptr) a.anc[m][u] = e;
                         }
                     }
@@ -663,6 +699,22 @@ __global__ void __launch_bounds__(PR_THREADS, 1) k_prune(const PruneArgs a) {
         }
     }
 }
+
+template <bool PER_TILE>
+__global__ void __launch_bounds__(PR_THREADS, 1) k_prune(const PruneArgs a) {
+    extern __shared__ __align__(128) unsigned char smem[];
+    prune_body<PER_TILE, false>(a, smem);
+}
+template <bool PER_TILE>
+__global__ void __launch_bounds__(PR_THREADS, 1) k_prune_scaled(const PruneArgs a) {
+    extern __shared__ __align__(128) unsigned char smem[];
+    prune_body<PER_TILE, true>(a, smem);
+}
+
+// The pruning kernel of a tree of nl leaves: unscaled up to SMALL_TREE_MAX_LEAVES leaves (what the reference computes), rescaled above.
+using PruneKernel = void (*)(PruneArgs);
+template <bool PER_TILE>
+inline PruneKernel prune_kernel(int nl) { return nl > SMALL_TREE_MAX_LEAVES ? k_prune_scaled<PER_TILE> : k_prune<PER_TILE>; }
 
 // ---------------------------------------------------------------------------------------------------
 // k_scatter (tracks): decibans of every window from its pattern's two log-likelihoods (run.hpp:51-54).
@@ -691,31 +743,55 @@ __global__ void k_scatter_list(uint32_t nwin, const uint32_t *__restrict__ pidx,
 }
 
 // ---------------------------------------------------------------------------------------------------
-// k_bls: per-base branch length score.  One thread per column: 128-bit presence mask of the species
-// with A/C/G/T (get_dna_id <= 3, additional_scores.hpp:63), then the post-order BLS program with a
-// per-thread stack in shared memory; summation order (own + left) + right as in
-// newick_sum_branch_lengths (additional_scores.hpp:5-41) => bit-identical doubles.
+// k_bls: per-base branch length score.  One thread per column: presence mask of the species with A/C/G/T (get_dna_id <= 3,
+// additional_scores.hpp:63) in NW 64-bit words (2 for trees of at most 128 leaves, 8 up to 512), then the post-order BLS program
+// with a per-thread stack in shared memory; summation order (own + left) + right as in newick_sum_branch_lengths
+// (additional_scores.hpp:5-41) => bit-identical doubles.
 // raw != 0: write bl(S) itself (score-msa sums it, :71), else bl(S)/bl(all) (:73-74).
 constexpr int BLS_THREADS = 128;
 constexpr int BLS_COLS = 4;            // columns per thread: one 32-bit load per species, four independent evaluations in flight
 
+template <int NW>
 __global__ void __launch_bounds__(BLS_THREADS) k_bls(const uint8_t *__restrict__ codes, int64_t ld, int nl, int64_t L,
-                                                    const BlsInner *__restrict__ prog, int n_prog, int depth,
+                                                    const BlsInnerDev<NW> *__restrict__ prog, int n_prog, int depth,
                                                     const double *__restrict__ tables, double all, int raw, double *__restrict__ out) {
     extern __shared__ double bls_stack[];  // [depth][BLS_COLS][BLS_THREADS]
     const int64_t i0 = ((int64_t)blockIdx.x * BLS_THREADS + threadIdx.x) * BLS_COLS;
     if (i0 >= L) return;
     // presence masks of four consecutive columns (rows are padded with N up to a multiple of 16 columns, so the word load is safe)
-    uint64_t mlo[BLS_COLS] = {0, 0, 0, 0}, mhi[BLS_COLS] = {0, 0, 0, 0};
-    for (int s = 0; s < nl; ++s) {
-        const uint32_t w = __ldg(reinterpret_cast<const uint32_t *>(codes + (int64_t)s * ld + i0));
-        const uint32_t present = ~(w >> 2) & 0x01010101u;          // code <= 3 (A, C, G, T): bit 2 clear
-        if (s < 64) {
+    uint64_t msk[NW][BLS_COLS];
 #pragma unroll
-            for (int j = 0; j < BLS_COLS; ++j) mlo[j] |= (uint64_t)((present >> (8 * j)) & 1u) << s;
-        } else {
+    for (int i = 0; i < NW; ++i)
 #pragma unroll
-            for (int j = 0; j < BLS_COLS; ++j) mhi[j] |= (uint64_t)((present >> (8 * j)) & 1u) << (s - 64);
+        for (int j = 0; j < BLS_COLS; ++j) msk[i][j] = 0;
+    if constexpr (NW == 2) {
+        for (int s = 0; s < nl; ++s) {
+            const uint32_t w = __ldg(reinterpret_cast<const uint32_t *>(codes + (int64_t)s * ld + i0));
+            const uint32_t present = ~(w >> 2) & 0x01010101u;          // code <= 3 (A, C, G, T): bit 2 clear
+            if (s < 64) {
+#pragma unroll
+                for (int j = 0; j < BLS_COLS; ++j) msk[0][j] |= (uint64_t)((present >> (8 * j)) & 1u) << s;
+            } else {
+#pragma unroll
+                for (int j = 0; j < BLS_COLS; ++j) msk[1][j] |= (uint64_t)((present >> (8 * j)) & 1u) << (s - 64);
+            }
+        }
+    } else {
+        // one word at a time into registers, then a static store into its place: the masks never leave registers
+        for (int s0 = 0; s0 < nl; s0 += 64) {
+            uint64_t word[BLS_COLS] = {0, 0, 0, 0};
+            for (int s = s0; s < min(nl, s0 + 64); ++s) {
+                const uint32_t w = __ldg(reinterpret_cast<const uint32_t *>(codes + (int64_t)s * ld + i0));
+                const uint32_t present = ~(w >> 2) & 0x01010101u;
+#pragma unroll
+                for (int j = 0; j < BLS_COLS; ++j) word[j] |= (uint64_t)((present >> (8 * j)) & 1u) << (s - s0);
+            }
+#pragma unroll
+            for (int i = 0; i < NW; ++i)
+                if (64 * i == s0) {
+#pragma unroll
+                    for (int j = 0; j < BLS_COLS; ++j) msk[i][j] = word[j];
+                }
         }
     }
     // inner nodes in post-order; a leaf child contributes its own branch length (no stack traffic), an inner child the value on
@@ -725,15 +801,32 @@ __global__ void __launch_bounds__(BLS_THREADS) k_bls(const uint8_t *__restrict__
     int sp = 0;
     double v[BLS_COLS] = {0.0, 0.0, 0.0, 0.0};
     for (int k = 0; k < n_prog; ++k) {
-        const BlsInner e = prog[k];
+        const BlsInnerDev<NW> e = prog[k];
         if (e.flags & 4) {
-            const int shift = (e.flags >> 8) & 0xff, nbits = (e.flags >> 16) & 0xff;
+            const int nbits = (e.flags >> 16) & 0xff;
 #pragma unroll
             for (int j = 0; j < BLS_COLS; ++j) {
-                const bool arrived = ((mlo[j] & ~e.self_lo) | (mhi[j] & ~e.self_hi)) != 0;
+                uint64_t out_of = 0;
+#pragma unroll
+                for (int i = 0; i < NW; ++i) out_of |= msk[i][j] & ~e.self[i];
+                const bool arrived = out_of != 0;
                 uint64_t bits;
-                if (shift >= 64) bits = mhi[j] >> (shift - 64);
-                else bits = (mlo[j] >> shift) | (shift ? mhi[j] << (64 - shift) : 0ull);
+                if constexpr (NW == 2) {
+                    const int shift = (e.flags >> 8) & 0xff;
+                    if (shift >= 64) bits = msk[1][j] >> (shift - 64);
+                    else bits = (msk[0][j] >> shift) | (shift ? msk[1][j] << (64 - shift) : 0ull);
+                } else {
+                    // first leaf: bits 0-7 in flag bits 8-15, bits 8-15 in flag bits 24-31 (model_prep.hpp: bls_table_flags).  Every
+                    // word shifts its part into place (no indexed access: the masks stay in registers)
+                    const int shift = ((e.flags >> 8) & 0xff) | ((e.flags >> 16) & 0xff00);
+                    bits = 0;
+#pragma unroll
+                    for (int i = 0; i < NW; ++i) {
+                        const int d = 64 * i - shift;   // where word i starts, relative to the first leaf
+                        if (d <= 0 && d > -64) bits |= msk[i][j] >> -d;
+                        else if (d > 0 && d < 64) bits |= msk[i][j] << d;
+                    }
+                }
                 bits &= (1ull << nbits) - 1;
                 v[j] = __ldg(tables + e.tab_off + 2 * bits + (arrived ? 1 : 0));
             }
@@ -757,12 +850,16 @@ __global__ void __launch_bounds__(BLS_THREADS) k_bls(const uint8_t *__restrict__
             }
 #pragma unroll
             for (int j = 0; j < BLS_COLS; ++j) {
-                const bool arrived = ((mlo[j] & ~e.self_lo) | (mhi[j] & ~e.self_hi)) != 0;
-                const bool ol = ((mlo[j] & e.left_lo) | (mhi[j] & e.left_hi)) != 0;
-                const bool orr = ((mlo[j] & e.self_lo & ~e.left_lo) | (mhi[j] & e.self_hi & ~e.left_hi)) != 0;
-                double x = arrived ? e.bl : 0.0;
-                if (ol) x = __dadd_rn(x, l[j]);
-                if (orr) x = __dadd_rn(x, r[j]);
+                uint64_t out_of = 0, in_l = 0, in_r = 0;
+#pragma unroll
+                for (int i = 0; i < NW; ++i) {
+                    out_of |= msk[i][j] & ~e.self[i];
+                    in_l |= msk[i][j] & e.left[i];
+                    in_r |= msk[i][j] & e.self[i] & ~e.left[i];
+                }
+                double x = out_of != 0 ? e.bl : 0.0;
+                if (in_l != 0) x = __dadd_rn(x, l[j]);
+                if (in_r != 0) x = __dadd_rn(x, r[j]);
                 v[j] = x;
             }
         }
@@ -773,8 +870,11 @@ __global__ void __launch_bounds__(BLS_THREADS) k_bls(const uint8_t *__restrict__
 #pragma unroll
     for (int j = 0; j < BLS_COLS; ++j) {
         if (i0 + j >= L) break;
+        int present = 0;
+#pragma unroll
+        for (int i = 0; i < NW; ++i) present += __popcll(msk[i][j]);
         double res = 0.0;
-        if (__popcll(mlo[j]) + __popcll(mhi[j]) >= 2) {          // fewer than two species with a base: 0 (additional_scores.hpp:66-69)
+        if (present >= 2) {          // fewer than two species with a base: 0 (additional_scores.hpp:66-69)
             res = v[j];
             if (!raw) res = __ddiv_rn(res, all);
         }

@@ -493,7 +493,7 @@ inline pcsf_status mle_run(const ModelHost &h, const MleBatch &b, double *const 
         if (ev[0]) MCK(cudaEventRecord(ev[2], st));
         k_mle_expm<<<n_slots * n_br, 128, 0, st>>>(d_slots, n_br, h.nl, d_bl, d_eig[0], d_eig[1], d_e2g, d_p, slot_stride, leaf_off, d_err);
         if (ev[0]) MCK(cudaEventRecord(ev[3], st));
-        k_prune<true><<<sm_count, (prune_nwarp + 1) * 32, prune_smem, st>>>(pa);
+        prune_kernel<true>(h.nl)<<<sm_count, (prune_nwarp + 1) * 32, prune_smem, st>>>(pa);
         MCK(cudaGetLastError());
         if (ev[0]) {
             MCK(cudaEventRecord(ev[4], st));

@@ -11,7 +11,7 @@
 //   * the pruning program: a children-first traversal that finishes the subtree needing more live
 //     partials first (values are order independent, fixed_lik.hpp:135-157), flattened into
 //     GATHER/PUSH/POP/GEMM ops, plus the P matrices of the GEMM edges re-ordered into DMMA fragment order;
-//   * the BLS program: post-order node list with 128-bit "species below" masks and the pointer tree's
+//   * the BLS program: post-order node list with "species below" masks (up to 512 bits) and the pointer tree's
 //     double branch lengths (additional_scores.hpp:5-41).
 #pragma once
 
@@ -25,29 +25,77 @@ namespace pcsf {
 
 constexpr int NS = 64;
 
+// Trees of up to this many leaves run the unscaled FP64 pruning (k_prune), the two-word BLS masks (k_bls<2>) and have a tcgen05
+// program; larger ones (up to PCSF_MAX_LEAVES = 512) run k_prune_scaled and k_bls<8> and have no tcgen05 program (its leaf and
+// source ids are 8-bit, and the tcgen05 kernel's shared memory holds no tree above 126 leaves anyway).
+constexpr int SMALL_TREE_MAX_LEAVES = 128;
+constexpr int BLS_MAX_WORDS = 8;   // 64-bit words of a leaf set: 512 leaves
+
+// A set of leaves (bit l = leaf l), as wide as the largest tree.  The device programs carry only the words their tree needs.
+struct LeafSet {
+    uint64_t w[BLS_MAX_WORDS] = {};
+    LeafSet operator|(const LeafSet &o) const { LeafSet r; for (int i = 0; i < BLS_MAX_WORDS; ++i) r.w[i] = w[i] | o.w[i]; return r; }
+    LeafSet operator&(const LeafSet &o) const { LeafSet r; for (int i = 0; i < BLS_MAX_WORDS; ++i) r.w[i] = w[i] & o.w[i]; return r; }
+    LeafSet operator~() const { LeafSet r; for (int i = 0; i < BLS_MAX_WORDS; ++i) r.w[i] = ~w[i]; return r; }
+    bool any() const { uint64_t x = 0; for (int i = 0; i < BLS_MAX_WORDS; ++i) x |= w[i]; return x != 0; }
+    int count() const { int c = 0; for (int i = 0; i < BLS_MAX_WORDS; ++i) c += __builtin_popcountll(w[i]); return c; }
+    int first() const { for (int i = 0; i < BLS_MAX_WORDS; ++i) if (w[i]) return 64 * i + __builtin_ctzll(w[i]); return -1; }
+    void set(int l) { w[l >> 6] |= 1ull << (l & 63); }
+    static LeafSet all(int nl) { LeafSet r; for (int l = 0; l < nl; ++l) r.set(l); return r; }
+    uint64_t bits(int shift, int nbits) const {   // nbits <= 63 bits starting at leaf `shift`
+        const int i = shift >> 6, o = shift & 63;
+        uint64_t v = w[i] >> o;
+        if (o && i + 1 < BLS_MAX_WORDS) v |= w[i + 1] << (64 - o);
+        return v & ((1ull << nbits) - 1);
+    }
+};
+
 // ---- pruning program ops (int32: code << 16 | arg) -------------------------------------------------
 enum : int32_t { OP_GATHER_SET = 1, OP_GATHER_MUL = 2, OP_PUSH = 3, OP_POP_MUL = 4, OP_GEMM = 5, OP_END = 6 };
 inline int32_t mk_op(int code, int arg) { return (code << 16) | (arg & 0xffff); }
 
 struct BlsNode {            // one post-order entry of the BLS program
     double bl;              // newick_node::branch_length (double)
-    uint64_t self_lo, self_hi;   // leaves below this node
-    uint64_t left_lo, left_hi;   // leaves below the left child (0 for leaves)
+    LeafSet self;           // leaves below this node
+    LeafSet left;           // leaves below the left child (empty for leaves)
     int32_t is_leaf;
-    int32_t pad;
 };
 
 struct BlsInner {           // one INNER node of the BLS program, post-order; leaf children are folded in (their value is their own
     double bl;              // branch length, whatever the presence mask): half of the stack traffic of the node-per-entry program
     double left_bl, right_bl;    // the child's branch length if it is a leaf
-    uint64_t self_lo, self_hi;
-    uint64_t left_lo, left_hi;
+    LeafSet self, left;
     int32_t flags;          // bit 0: left child is a leaf, bit 1: right child is a leaf;
                             // bit 2: TABLE entry — the value of this node for every presence pattern of its (<= BLS_TABLE_BITS, consecutively
                             // numbered) leaves and for arrived = 0 / 1 was tabulated on the host with the very same additions: the device
-                            // pushes tables[tab_off + 2 * pattern + arrived]; bits 8-15: number of the first leaf, bits 16-23: leaf count
+                            // pushes tables[tab_off + 2 * pattern + arrived]; number of the first leaf: bits 0-7 in bits 8-15, bits 8-15 in
+                            // bits 24-31; bits 16-23: leaf count
     int32_t tab_off;
 };
+inline int bls_table_shift(int32_t flags) { return ((flags >> 8) & 0xff) | ((flags >> 16) & 0xff00); }
+inline int32_t bls_table_flags(int shift, int nbits) { return 4 | ((shift & 0xff) << 8) | (nbits << 16) | ((shift >> 8) << 24); }
+
+// The entry k_bls<NW> reads: the BlsInner with its masks cut to NW words (NW = 2 for trees of at most 128 leaves, 8 above).
+template <int NW>
+struct BlsInnerDev {
+    double bl;
+    double left_bl, right_bl;
+    uint64_t self[NW], left[NW];
+    int32_t flags;
+    int32_t tab_off;
+};
+template <int NW>
+inline std::vector<BlsInnerDev<NW>> bls_device_program(const std::vector<BlsInner> &prog) {
+    std::vector<BlsInnerDev<NW>> out(prog.size());
+    for (size_t k = 0; k < prog.size(); ++k) {
+        const BlsInner &e = prog[k];
+        BlsInnerDev<NW> &d = out[k];
+        d.bl = e.bl; d.left_bl = e.left_bl; d.right_bl = e.right_bl;
+        for (int i = 0; i < NW; ++i) { d.self[i] = e.self.w[i]; d.left[i] = e.left.w[i]; }
+        d.flags = e.flags; d.tab_off = e.tab_off;
+    }
+    return out;
+}
 
 struct EcmHost {
     double lambda[NS], SR[NS * NS], SRinv[NS * NS], pi[NS], logpi[NS];
@@ -411,47 +459,46 @@ inline const char *prepare_tc5_program(ModelHost &m) {
     return nullptr;
 }
 
-inline void bls_walk(ModelHost &m, int i, uint64_t &lo, uint64_t &hi, int &depth_out) {
+inline void bls_walk(ModelHost &m, int i, LeafSet &below, int &depth_out) {
     BlsNode e{};
     e.bl = m.bl64[i];
     if (m.child1[i] < 0) {
         e.is_leaf = 1;
-        if (i < 64) e.self_lo = 1ull << i; else e.self_hi = 1ull << (i - 64);
-        lo = e.self_lo; hi = e.self_hi;
+        e.self.set(i);
+        below = e.self;
         depth_out = 1;
         m.bls_prog.push_back(e);
         return;
     }
-    uint64_t llo, lhi, rlo, rhi;
+    LeafSet l, r;
     int dl, dr;
-    bls_walk(m, m.child1[i], llo, lhi, dl);
-    bls_walk(m, m.child2[i], rlo, rhi, dr);
-    e.left_lo = llo; e.left_hi = lhi;
-    e.self_lo = llo | rlo; e.self_hi = lhi | rhi;
-    lo = e.self_lo; hi = e.self_hi;
+    bls_walk(m, m.child1[i], l, dl);
+    bls_walk(m, m.child2[i], r, dr);
+    e.left = l;
+    e.self = l | r;
+    below = e.self;
     depth_out = dl > dr + 1 ? dl : dr + 1;
     m.bls_prog.push_back(e);
     BlsInner in{};
     in.bl = e.bl;
     const int cl = m.child1[i], cr = m.child2[i];
     in.left_bl = m.bl64[cl]; in.right_bl = m.bl64[cr];
-    in.self_lo = e.self_lo; in.self_hi = e.self_hi; in.left_lo = llo; in.left_hi = lhi;
+    in.self = e.self; in.left = l;
     in.flags = (m.child1[cl] < 0 ? 1 : 0) | (m.child1[cr] < 0 ? 2 : 0);
     m.bls_inner.push_back(in);
 }
 }  // namespace detail
 
 // Host restatement of newick_sum_branch_lengths over the BLS program (also what k_bls executes).
-inline double bls_eval_host(const ModelHost &m, uint64_t mlo, uint64_t mhi) {
+inline double bls_eval_host(const ModelHost &m, const LeafSet &mask) {
     std::vector<double> st(m.bls_depth + 2);
     int sp = 0;
     for (const BlsNode &e : m.bls_prog) {
         if (e.is_leaf) { st[sp++] = e.bl; continue; }
         const double r = st[--sp], l = st[--sp];
-        const uint64_t rlo = e.self_lo & ~e.left_lo, rhi = e.self_hi & ~e.left_hi;
-        const bool ol = ((mlo & e.left_lo) | (mhi & e.left_hi)) != 0;
-        const bool orr = ((mlo & rlo) | (mhi & rhi)) != 0;
-        const bool arrived = ((mlo & ~e.self_lo) | (mhi & ~e.self_hi)) != 0;
+        const bool ol = (mask & e.left).any();
+        const bool orr = (mask & e.self & ~e.left).any();
+        const bool arrived = (mask & ~e.self).any();
         double v = arrived ? e.bl : 0.0;
         if (ol) v += l;
         if (orr) v += r;
@@ -461,7 +508,7 @@ inline double bls_eval_host(const ModelHost &m, uint64_t mlo, uint64_t mhi) {
 }
 
 // The inner-node program (what k_bls executed before the tables): value on top of the stack right after entry `upto`.
-inline double bls_eval_inner_host(const std::vector<BlsInner> &prog, int depth, uint64_t mlo, uint64_t mhi, int upto) {
+inline double bls_eval_inner_host(const std::vector<BlsInner> &prog, int depth, const LeafSet &mask, int upto) {
     std::vector<double> st(depth + 2);
     int sp = 0;
     double v = 0.0;
@@ -470,9 +517,9 @@ inline double bls_eval_inner_host(const std::vector<BlsInner> &prog, int depth, 
         double r, l;
         if (e.flags & 2) r = e.right_bl; else r = st[--sp];
         if (e.flags & 1) l = e.left_bl; else l = st[--sp];
-        const bool ol = ((mlo & e.left_lo) | (mhi & e.left_hi)) != 0;
-        const bool orr = ((mlo & e.self_lo & ~e.left_lo) | (mhi & e.self_hi & ~e.left_hi)) != 0;
-        const bool arrived = ((mlo & ~e.self_lo) | (mhi & ~e.self_hi)) != 0;
+        const bool ol = (mask & e.left).any();
+        const bool orr = (mask & e.self & ~e.left).any();
+        const bool arrived = (mask & ~e.self).any();
         v = arrived ? e.bl : 0.0;
         if (ol) v += l;
         if (orr) v += r;
@@ -490,7 +537,6 @@ inline void bls_build_tables(ModelHost &m) {
     m.bls_short.clear();
     m.bls_tables.clear();
     const int n_inner = (int)m.bls_inner.size();
-    auto popcnt = [](uint64_t x) { return __builtin_popcountll(x); };
     // post-order program: the subtree of entry k is a contiguous run of entries ending at k; find its first entry by counting
     std::vector<int> first(n_inner);
     {
@@ -507,33 +553,31 @@ inline void bls_build_tables(ModelHost &m) {
     std::vector<char> is_root(n_inner, 0);
     for (int k = n_inner - 1; k >= 0; --k) {
         const BlsInner &e = m.bls_inner[k];
-        if (popcnt(e.self_lo) + popcnt(e.self_hi) > BLS_TABLE_BITS) continue;
+        if (e.self.count() > BLS_TABLE_BITS) continue;
         bool inside = false;             // already inside a collapsed subtree?
         for (int r = k + 1; r < n_inner && !inside; ++r) inside = is_root[r] && first[r] <= k;
         if (!inside) is_root[k] = 1;
     }
-    const uint64_t alo = m.nl >= 64 ? ~0ull : ((1ull << m.nl) - 1);
-    const uint64_t ahi = m.nl > 64 ? (m.nl >= 128 ? ~0ull : ((1ull << (m.nl - 64)) - 1)) : 0ull;
+    const LeafSet all = LeafSet::all(m.nl);
     for (int k = 0; k < n_inner; ++k) {
         bool dropped = false;
         for (int r = k + 1; r < n_inner && !dropped; ++r) dropped = is_root[r] && first[r] <= k;
         if (dropped) continue;
         BlsInner e = m.bls_inner[k];
         if (is_root[k]) {
-            const int nbits = popcnt(e.self_lo) + popcnt(e.self_hi);
-            const int shift = e.self_lo ? __builtin_ctzll(e.self_lo) : 64 + __builtin_ctzll(e.self_hi);
+            const int nbits = e.self.count();
+            const int shift = e.self.first();
             // one leaf outside the subtree stands for "arrived" (none exists when the subtree is the whole tree: arrived is never set)
-            const uint64_t olo = alo & ~e.self_lo, ohi = ahi & ~e.self_hi;
-            uint64_t wlo = 0, whi = 0;
-            if (olo) wlo = olo & (~olo + 1); else if (ohi) whi = ohi & (~ohi + 1);
-            e.flags = 4 | (shift << 8) | (nbits << 16);
+            const int outside = (all & ~e.self).first();
+            e.flags = bls_table_flags(shift, nbits);
             e.tab_off = (int32_t)m.bls_tables.size();
             for (uint64_t pat = 0; pat < (1ull << nbits); ++pat)
                 for (int arrived = 0; arrived < 2; ++arrived) {
-                    unsigned __int128 bits = (unsigned __int128)pat << shift;
-                    uint64_t mlo = (uint64_t)bits, mhi = (uint64_t)(bits >> 64);
-                    if (arrived) { mlo |= wlo; mhi |= whi; }
-                    m.bls_tables.push_back(bls_eval_inner_host(m.bls_inner, m.bls_depth, mlo, mhi, k));
+                    LeafSet mask;
+                    for (int b = 0; b < nbits; ++b)
+                        if ((pat >> b) & 1) mask.set(shift + b);
+                    if (arrived && outside >= 0) mask.set(outside);
+                    m.bls_tables.push_back(bls_eval_inner_host(m.bls_inner, m.bls_depth, mask, k));
                 }
         }
         m.bls_short.push_back(e);
@@ -550,25 +594,21 @@ inline void bls_build_tables(ModelHost &m) {
 }
 
 // What k_bls executes, on the host (self-check at model creation).
-inline double bls_eval_short_host(const ModelHost &m, uint64_t mlo, uint64_t mhi) {
+inline double bls_eval_short_host(const ModelHost &m, const LeafSet &mask) {
     std::vector<double> st(m.bls_short_depth + 2);
     int sp = 0;
     double v = 0.0;
     for (const BlsInner &e : m.bls_short) {
-        const bool arrived = ((mlo & ~e.self_lo) | (mhi & ~e.self_hi)) != 0;
+        const bool arrived = (mask & ~e.self).any();
         if (e.flags & 4) {
-            const int shift = (e.flags >> 8) & 0xff, nbits = (e.flags >> 16) & 0xff;
-            uint64_t bits;
-            if (shift >= 64) bits = mhi >> (shift - 64);
-            else bits = (mlo >> shift) | (shift ? mhi << (64 - shift) : 0ull);
-            bits &= (1ull << nbits) - 1;
+            const uint64_t bits = mask.bits(bls_table_shift(e.flags), (e.flags >> 16) & 0xff);
             v = m.bls_tables[(size_t)e.tab_off + 2 * bits + (arrived ? 1 : 0)];
         } else {
             double r, l;
             if (e.flags & 2) r = e.right_bl; else r = st[--sp];
             if (e.flags & 1) l = e.left_bl; else l = st[--sp];
-            const bool ol = ((mlo & e.left_lo) | (mhi & e.left_hi)) != 0;
-            const bool orr = ((mlo & e.self_lo & ~e.left_lo) | (mhi & e.self_hi & ~e.left_hi)) != 0;
+            const bool ol = (mask & e.left).any();
+            const bool orr = (mask & e.self & ~e.left).any();
             v = arrived ? e.bl : 0.0;
             if (ol) v += l;
             if (orr) v += r;
@@ -600,30 +640,29 @@ inline std::string prepare_model(ModelHost &m, int nl, const int16_t *c1, const 
     detail::emit_partial(m, m.n - 1, need, sp);
     m.program.push_back(mk_op(OP_END, 0));
     if ((int)m.gemm_edges.size() != nl - 2) return "internal error: GEMM count";
-    if (const char *terr = detail::prepare_tc5_program(m)) return terr;
+    // the tcgen05 program only for trees it can hold (8-bit leaf and source ids; k_prune_tc5 refuses every tree above 126 leaves)
+    if (nl <= SMALL_TREE_MAX_LEAVES)
+        if (const char *terr = detail::prepare_tc5_program(m)) return terr;
     // BLS program
-    uint64_t lo, hi;
+    LeafSet below;
     m.bls_prog.clear();
     m.bls_inner.clear();
-    detail::bls_walk(m, m.n - 1, lo, hi, m.bls_depth);
-    {
-        const uint64_t alo = nl >= 64 ? ~0ull : ((1ull << nl) - 1);
-        const uint64_t ahi = nl > 64 ? (nl >= 128 ? ~0ull : ((1ull << (nl - 64)) - 1)) : 0ull;
-        m.bls_all = bls_eval_host(m, alo, ahi);
-    }
+    detail::bls_walk(m, m.n - 1, below, m.bls_depth);
+    const LeafSet all = LeafSet::all(nl);
+    m.bls_all = bls_eval_host(m, all);
     bls_build_tables(m);
     {   // the collapsed program must give the node-by-node program's doubles, bit for bit
         uint64_t x = 0x9E3779B97F4A7C15ull;
-        const uint64_t alo = nl >= 64 ? ~0ull : ((1ull << nl) - 1);
-        const uint64_t ahi = nl > 64 ? (nl >= 128 ? ~0ull : ((1ull << (nl - 64)) - 1)) : 0ull;
+        auto next = [&x]() { x ^= x << 13; x ^= x >> 7; x ^= x << 17; return x; };
         for (int t = 0; t < 2000; ++t) {
-            x ^= x << 13; x ^= x >> 7; x ^= x << 17;
-            uint64_t mlo = x; x ^= x << 13; x ^= x >> 7; x ^= x << 17;
-            uint64_t mhi = x;
-            if (t % 3 == 1) { x ^= x << 13; x ^= x >> 7; x ^= x << 17; mlo &= x; x ^= x << 13; x ^= x >> 7; x ^= x << 17; mhi &= x; }   // sparse masks
-            if (t % 3 == 2) { x ^= x << 13; x ^= x >> 7; x ^= x << 17; mlo |= x; x ^= x << 13; x ^= x >> 7; x ^= x << 17; mhi |= x; }   // dense masks
-            mlo &= alo; mhi &= ahi;
-            const double a = bls_eval_host(m, mlo, mhi), b = bls_eval_short_host(m, mlo, mhi);
+            LeafSet mask;
+            for (int i = 0; i < BLS_MAX_WORDS; ++i) {
+                mask.w[i] = next();
+                if (t % 3 == 1) mask.w[i] &= next();   // sparse masks
+                if (t % 3 == 2) mask.w[i] |= next();   // dense masks
+            }
+            mask = mask & all;
+            const double a = bls_eval_host(m, mask), b = bls_eval_short_host(m, mask);
             if (memcmp(&a, &b, 8) != 0) return "internal error: BLS tables disagree with the node-by-node program";
         }
     }

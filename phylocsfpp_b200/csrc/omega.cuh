@@ -415,7 +415,7 @@ inline pcsf_status omega_run(const ModelHost &h, const OmegaBatch &b, const floa
         k_mle_plan<<<1, 1024, 0, st>>>(d_slots, n_slots, d_p, slot_stride, leaf_off, tw, d_tiles, reinterpret_cast<uint32_t *>(d_ctr + 2), d_pis);
         k_mle_expm<<<n_slots * n_br, 128, 0, st>>>(d_slots, n_br, h.nl, d_bl, nullptr, nullptr, d_e2g, d_p, slot_stride, leaf_off, d_err,
                                                   d_eig, d_rho);
-        k_prune<true><<<sm_count, (prune_nwarp + 1) * 32, prune_smem, st>>>(pa);
+        prune_kernel<true>(h.nl)<<<sm_count, (prune_nwarp + 1) * 32, prune_smem, st>>>(pa);
         MCK(cudaGetLastError());
         if (launches) *launches += 4;
     }

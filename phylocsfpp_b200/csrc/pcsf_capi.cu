@@ -91,7 +91,7 @@ struct pcsf_model {
     size_t h_msa_cap = 0;
     DevBuf tc5_ids;                      // codon ids of the unique windows, [pairs][2][nl][128] (k_tc5_ids)
     int32_t *d_program = nullptr;
-    BlsInner *d_bls_prog = nullptr;
+    void *d_bls_prog = nullptr;          // BlsInnerDev<2> (trees of at most SMALL_TREE_MAX_LEAVES leaves) or BlsInnerDev<8>
     double *d_bls_tables = nullptr;
     float *d_bl = nullptr;
     int32_t *d_gemm_edges = nullptr;
@@ -129,7 +129,9 @@ extern "C" pcsf_status pcsf_model_create(const pcsf_model_desc *d, int device, p
     if (!d || !out || d->nl < 2 || !d->child1 || !d->child2 || !d->branch_len || !d->branch_len_f64 || !d->ecm_c ||
         !d->freq_c || !d->ecm_nc || !d->freq_nc)
         return fail(PCSF_ERR_INVALID, "pcsf_model_create: null argument or fewer than 2 leaves");
-    if (d->nl > PCSF_MAX_LEAVES) return fail(PCSF_ERR_UNSUPPORTED, "more than 128 leaves are not supported");
+    if (d->nl > PCSF_MAX_LEAVES)
+        return fail(PCSF_ERR_UNSUPPORTED, "tree of " + std::to_string(d->nl) + " leaves: at most " + std::to_string(PCSF_MAX_LEAVES) +
+                                              " leaves (PCSF_MAX_LEAVES) are supported");
     pcsf_model *m = new pcsf_model;
     struct Guard {                       // every early return below releases the handle and what it already owns on the device
         pcsf_model *m;
@@ -172,9 +174,11 @@ extern "C" pcsf_status pcsf_model_create(const pcsf_model_desc *d, int device, p
         if ((st = upload(eig.data(), eig.size() * 8, (void **)&m->d_eig[w]))) return st;
     }
     if ((st = upload(m->host.program.data(), m->host.program.size() * 4, (void **)&m->d_program))) return st;
-    if ((st = upload(m->host.tc5_steps.data(), m->host.tc5_steps.size() * 4, (void **)&m->d_tc5_steps))) return st;
-    CK(cudaMalloc(&m->d_tc5_scratch, (size_t)m->sm_count * 2 * std::max(1, m->host.tc5_max_stack) * T5_STACK_ENTRY_FLOATS * 4));
-    {
+    // Trees above SMALL_TREE_MAX_LEAVES leaves have no tcgen05 program (model_prep.hpp): no row tables, and pcsf_tracks_device refuses
+    // PCSF_TRACKS_TC5 for them.
+    if (m->host.nl <= SMALL_TREE_MAX_LEAVES) {
+        if ((st = upload(m->host.tc5_steps.data(), m->host.tc5_steps.size() * 4, (void **)&m->d_tc5_steps))) return st;
+        CK(cudaMalloc(&m->d_tc5_scratch, (size_t)m->sm_count * 2 * std::max(1, m->host.tc5_max_stack) * T5_STACK_ENTRY_FLOATS * 4));
         // row tables (leaf columns and cherry messages): FP64 on the device from the leaves' columns and the cherry nodes' P, FP32 rows
         const int ns = (int)m->host.tc5_srcs.size();
         if ((st = upload(m->host.tc5_srcs.data(), (size_t)ns * sizeof(Tc5Src), (void **)&m->d_tc5_srcs))) return st;
@@ -190,16 +194,20 @@ extern "C" pcsf_status pcsf_model_create(const pcsf_model_desc *d, int device, p
             cudaFree(d_cp);
             CK(e);
         }
+        prune_tc5_pick_stages(m->host.nl, (int)m->host.tc5_steps.size(), (int)m->host.tc5_srcs.size(), &m->tc5_nstage, &m->tc5_nids);
+        if (const char *e = getenv("PCSF_TC5_NSTAGE")) m->tc5_nstage = std::max(2, std::min(m->tc5_nstage, atoi(e)));
+        if (const char *e = getenv("PCSF_TC5_NIDS")) m->tc5_nids = std::max(1, std::min(m->tc5_nids, atoi(e)));
+        m->prune_tc5_smem = prune_tc5_smem_bytes(m->host.nl, (int)m->host.tc5_steps.size(), (int)m->host.tc5_srcs.size(), m->tc5_nstage, m->tc5_nids);
+        // Trees above the tcgen05 path's budget (127 and 128 leaves always, 124 to 126 depending on the shape) still get a model: the FP64
+        // path and score-msa do not need k_prune_tc5, and pcsf_tracks_device refuses PCSF_TRACKS_TC5 for them with PCSF_ERR_UNSUPPORTED.
+        if (m->prune_tc5_smem <= 227 * 1024)
+            CK(cudaFuncSetAttribute(k_prune_tc5, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)m->prune_tc5_smem));
+        const std::vector<BlsInnerDev<2>> prog = bls_device_program<2>(m->host.bls_short);
+        if ((st = upload(prog.data(), prog.size() * sizeof(prog[0]), &m->d_bls_prog))) return st;
+    } else {
+        const std::vector<BlsInnerDev<8>> prog = bls_device_program<8>(m->host.bls_short);
+        if ((st = upload(prog.data(), prog.size() * sizeof(prog[0]), &m->d_bls_prog))) return st;
     }
-    prune_tc5_pick_stages(m->host.nl, (int)m->host.tc5_steps.size(), (int)m->host.tc5_srcs.size(), &m->tc5_nstage, &m->tc5_nids);
-    if (const char *e = getenv("PCSF_TC5_NSTAGE")) m->tc5_nstage = std::max(2, std::min(m->tc5_nstage, atoi(e)));
-    if (const char *e = getenv("PCSF_TC5_NIDS")) m->tc5_nids = std::max(1, std::min(m->tc5_nids, atoi(e)));
-    m->prune_tc5_smem = prune_tc5_smem_bytes(m->host.nl, (int)m->host.tc5_steps.size(), (int)m->host.tc5_srcs.size(), m->tc5_nstage, m->tc5_nids);
-    // Trees above the tcgen05 path's budget (127 and 128 leaves always, 124 to 126 depending on the shape) still get a model: the FP64
-    // path and score-msa do not need k_prune_tc5, and pcsf_tracks_device refuses PCSF_TRACKS_TC5 for them with PCSF_ERR_UNSUPPORTED.
-    if (m->prune_tc5_smem <= 227 * 1024)
-        CK(cudaFuncSetAttribute(k_prune_tc5, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)m->prune_tc5_smem));
-    if ((st = upload(m->host.bls_short.data(), m->host.bls_short.size() * sizeof(BlsInner), (void **)&m->d_bls_prog))) return st;
     if ((st = upload(m->host.bls_tables.data(), std::max<size_t>(m->host.bls_tables.size(), 1) * sizeof(double), (void **)&m->d_bls_tables))) return st;
     if ((st = upload(m->host.bl.data(), m->host.bl.size() * 4, (void **)&m->d_bl))) return st;
     {
@@ -226,10 +234,10 @@ extern "C" pcsf_status pcsf_model_create(const pcsf_model_desc *d, int device, p
         return fail(PCSF_ERR_UNSUPPORTED, "tree needs more shared memory than one SM has (stack depth " +
                                               std::to_string(m->host.max_stack) + ")");
     }
-    CK(cudaFuncSetAttribute(k_prune<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)m->prune_smem));
-    CK(cudaFuncSetAttribute(k_prune<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)m->prune_smem));
-    CK(cudaFuncSetAttribute(k_bls, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                            std::max(1, m->host.bls_short_depth) * BLS_THREADS * BLS_COLS * 8));
+    CK(cudaFuncSetAttribute(prune_kernel<false>(m->host.nl), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)m->prune_smem));
+    CK(cudaFuncSetAttribute(prune_kernel<true>(m->host.nl), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)m->prune_smem));
+    CK(cudaFuncSetAttribute(m->host.nl <= SMALL_TREE_MAX_LEAVES ? (const void *)k_bls<2> : (const void *)k_bls<8>,
+                            cudaFuncAttributeMaxDynamicSharedMemorySize, std::max(1, m->host.bls_short_depth) * BLS_THREADS * BLS_COLS * 8));
     guard.m = nullptr;
     *out = m;
     return PCSF_OK;
@@ -406,7 +414,7 @@ static pcsf_status dedup_and_prune(pcsf_model *m, const WinSpace &ws, uint32_t n
     const uint32_t tile_w = (uint32_t)m->prune_nwarp * 8;
     const uint32_t max_tiles = (nwin + tile_w - 1) / tile_w;
     const unsigned grid = std::min<uint32_t>((uint32_t)m->sm_count, std::max<uint32_t>(1u, max_tiles));
-    m->launches++; k_prune<false><<<grid, (m->prune_nwarp + 1) * 32, m->prune_smem, st>>>(pa);
+    m->launches++; prune_kernel<false>(m->host.nl)<<<grid, (m->prune_nwarp + 1) * 32, m->prune_smem, st>>>(pa);
     CK(cudaGetLastError());
     if (m->timing) {
         CK(cudaEventRecord(m->ev[3], st));
@@ -433,15 +441,27 @@ static pcsf_status run_pack(pcsf_model *m, const uint8_t *d_seqs, int64_t L, int
     return PCSF_OK;
 }
 
+// k_bls over columns [s0, s0 + n) of m->codes, with the mask width of the tree
+static pcsf_status launch_bls(pcsf_model *m, int64_t s0, int64_t n, int raw, double *d_out, cudaStream_t st) {
+    const size_t sh = (size_t)std::max(1, m->host.bls_short_depth) * BLS_THREADS * BLS_COLS * 8;
+    const unsigned grid = (unsigned)((n + BLS_THREADS * BLS_COLS - 1) / (BLS_THREADS * BLS_COLS));
+    m->launches++;
+    if (m->host.nl <= SMALL_TREE_MAX_LEAVES)
+        k_bls<2><<<grid, BLS_THREADS, sh, st>>>(m->codes.as<uint8_t>() + s0, m->codes_ld, m->host.nl, n,
+                                                static_cast<const BlsInnerDev<2> *>(m->d_bls_prog), (int)m->host.bls_short.size(),
+                                                m->host.bls_short_depth, m->d_bls_tables, m->host.bls_all, raw, d_out);
+    else
+        k_bls<8><<<grid, BLS_THREADS, sh, st>>>(m->codes.as<uint8_t>() + s0, m->codes_ld, m->host.nl, n,
+                                                static_cast<const BlsInnerDev<8> *>(m->d_bls_prog), (int)m->host.bls_short.size(),
+                                                m->host.bls_short_depth, m->d_bls_tables, m->host.bls_all, raw, d_out);
+    CK(cudaGetLastError());
+    return PCSF_OK;
+}
+
 static pcsf_status run_bls(pcsf_model *m, int64_t L, int raw, double *d_out, cudaStream_t st) {
     if (L <= 0) return PCSF_OK;
     NvtxRange nvtx_("pcsf: bls");
-    const size_t sh = (size_t)std::max(1, m->host.bls_short_depth) * BLS_THREADS * BLS_COLS * 8;
-    m->launches++; k_bls<<<(unsigned)((L + BLS_THREADS * BLS_COLS - 1) / (BLS_THREADS * BLS_COLS)), BLS_THREADS, sh, st>>>(
-        m->codes.as<uint8_t>(), m->codes_ld, m->host.nl, L, m->d_bls_prog, (int)m->host.bls_short.size(),
-        m->host.bls_short_depth, m->d_bls_tables, m->host.bls_all, raw, d_out);
-    CK(cudaGetLastError());
-    return PCSF_OK;
+    return launch_bls(m, 0, L, raw, d_out, st);
 }
 
 // Columns [s0, s1) only (s0 a multiple of 16): the pieces of run_pack / run_bls for an input that arrives in segments.
@@ -455,12 +475,7 @@ static pcsf_status run_pack_segment(pcsf_model *m, const uint8_t *d_seqs, int64_
 }
 static pcsf_status run_bls_segment(pcsf_model *m, int64_t s0, int64_t s1, double *d_out, cudaStream_t st) {
     if (s1 <= s0) return PCSF_OK;
-    const size_t sh = (size_t)std::max(1, m->host.bls_short_depth) * BLS_THREADS * BLS_COLS * 8;
-    m->launches++; k_bls<<<(unsigned)((s1 - s0 + BLS_THREADS * BLS_COLS - 1) / (BLS_THREADS * BLS_COLS)), BLS_THREADS, sh, st>>>(
-        m->codes.as<uint8_t>() + s0, m->codes_ld, m->host.nl, s1 - s0, m->d_bls_prog, (int)m->host.bls_short.size(),
-        m->host.bls_short_depth, m->d_bls_tables, m->host.bls_all, 0, d_out + s0);
-    CK(cudaGetLastError());
-    return PCSF_OK;
+    return launch_bls(m, s0, s1 - s0, 0, d_out + s0, st);
 }
 
 extern "C" pcsf_status pcsf_tracks_device(pcsf_model *m, const uint8_t *d_seqs, int64_t L, int64_t ld, uint32_t flags,
@@ -469,6 +484,10 @@ extern "C" pcsf_status pcsf_tracks_device(pcsf_model *m, const uint8_t *d_seqs, 
     if (!m || L < 0 || ld < L || (L > 0 && !d_seqs)) return fail(PCSF_ERR_INVALID, "pcsf_tracks: bad argument");
     if ((flags & PCSF_TRACKS_SCORES) && L > 2 && (!d_plus || !d_minus)) return fail(PCSF_ERR_INVALID, "plus/minus required");
     if ((flags & PCSF_TRACKS_BLS) && L > 0 && !d_bls) return fail(PCSF_ERR_INVALID, "bls required");
+    if ((flags & PCSF_TRACKS_TC5) && m->host.nl > SMALL_TREE_MAX_LEAVES)
+        return fail(PCSF_ERR_UNSUPPORTED, "the tcgen05 path (PCSF_TRACKS_TC5) does not support trees of more than " +
+                                              std::to_string(SMALL_TREE_MAX_LEAVES) + " leaves (this one has " + std::to_string(m->host.nl) +
+                                              "); the FP64 path scores them");
     if ((flags & PCSF_TRACKS_TC5) && m->prune_tc5_smem > 227 * 1024)
         return fail(PCSF_ERR_UNSUPPORTED, "tree too large for the tcgen05 path's shared-memory budget");
     CK(cudaSetDevice(m->device));
