@@ -194,6 +194,17 @@ pcsf_status pcsf_score_regions(pcsf_model *m, pcsf_strategy strategy, int32_t n_
                                int32_t best_only, int32_t want_anc, int32_t want_bls, int64_t *n_regions);
 pcsf_status pcsf_score_regions_get(const pcsf_model *m, pcsf_region *out, int64_t n);   /* records of the last pcsf_score_regions call on this handle */
 
+/*
+ * Scores n_regions column ranges [begin, end) of n_aln alignments (seqs / offset / len as pcsf_score_msa), each in frame +1 from
+ * `begin`.  phylo / anc / bls of region r are bit for bit what pcsf_score_msa returns for the sub-alignment (columns begin..end-1 of
+ * alignment region_aln[r]) extracted on the host.  anc / bls may be NULL.  begin > end, end > len or a bad alignment index:
+ * PCSF_ERR_INVALID.  FP64, all three strategies (OMEGA: anc NaN).  Every alignment is uploaded once, however many of its ranges are
+ * scored (a coding transcript and each of its CDS features).  Does not touch the records pcsf_score_regions_get returns.
+ */
+pcsf_status pcsf_score_given_regions(pcsf_model *m, pcsf_strategy strategy, int32_t n_aln, const uint8_t *seqs, const int64_t *offset,
+                                     const int64_t *len, int64_t n_regions, const int32_t *region_aln, const int64_t *region_begin,
+                                     const int64_t *region_end, float *phylo, float *anc, float *bls);
+
 /* ---- introspection (used by the parity tests) -------------------------------------------------- */
 
 /* What the last pcsf_score_msa call with PCSF_STRATEGY_MLE did on this handle: `evaluations` counts lpr_leaves calls — (alignment,

@@ -45,7 +45,7 @@ EXPORTS = [
     "pcsf_model_create", "pcsf_model_destroy", "pcsf_last_error", "pcsf_abi_version", "pcsf_tracks",
     "pcsf_tracks_device", "pcsf_tracks_device_finish", "pcsf_set_chunk_columns", "pcsf_set_timing",
     "pcsf_score_msa", "pcsf_model_get", "pcsf_alloc_pinned", "pcsf_free_pinned", "pcsf_device_count", "pcsf_score_msa_stats", "pcsf_register_host", "pcsf_unregister_host",
-    "pcsf_score_regions", "pcsf_score_regions_get",
+    "pcsf_score_regions", "pcsf_score_regions_get", "pcsf_score_given_regions",
 ]
 
 
@@ -114,6 +114,8 @@ def load():
     L.pcsf_score_regions.argtypes = [C.c_void_p, C.c_int, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32,
                                      C.c_int, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.POINTER(C.c_int64)]
     L.pcsf_score_regions_get.argtypes = [C.c_void_p, C.c_void_p, C.c_int64]
+    L.pcsf_score_given_regions.argtypes = [C.c_void_p, C.c_int, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p,
+                                           C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     _lib = L
     return L
 
@@ -242,3 +244,22 @@ class DeviceModel:
         out = np.zeros(nreg.value, REGION_DTYPE)
         _check(L.pcsf_score_regions_get(self.h, out.ctypes.data if out.size else None, nreg.value))
         return out
+
+    def score_given_regions(self, alignments, region_aln, region_begin, region_end, strategy: int = STRATEGY_FIXED,
+                            comp_anc: bool = True, comp_bls: bool = True):
+        """Column ranges [region_begin[r], region_end[r]) of alignments[region_aln[r]], each scored in frame +1 from its begin
+        (pcsf_score_given_regions).  Returns (phylo, anc, bls) float32 arrays, None for a score not asked for; bit for bit what
+        score_msa returns for the ranges cut out on the host."""
+        n, lens, offs, blob = self._batch(alignments)
+        ra = np.ascontiguousarray(np.asarray(region_aln, np.int32).reshape(-1))
+        rb = np.ascontiguousarray(np.asarray(region_begin, np.int64).reshape(-1))
+        re_ = np.ascontiguousarray(np.asarray(region_end, np.int64).reshape(-1))
+        if not (ra.size == rb.size == re_.size):
+            raise ValueError("region_aln, region_begin and region_end differ in length")
+        nr = ra.size
+        phylo = np.full(nr, np.nan, np.float32)
+        anc = np.full(nr, np.nan, np.float32) if comp_anc else None
+        b = np.full(nr, np.nan, np.float32) if comp_bls else None
+        _check(load().pcsf_score_given_regions(self.h, strategy, n, blob.ctypes.data, offs.ctypes.data, lens.ctypes.data, nr,
+                                               _ptr(ra), _ptr(rb), _ptr(re_), _ptr(phylo), _ptr(anc), _ptr(b)))
+        return phylo, anc, b

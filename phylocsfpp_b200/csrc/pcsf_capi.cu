@@ -732,39 +732,42 @@ struct ScoredRegions {
     RegionList R{};
     const int64_t *off_r = nullptr;                           // [n_aln * frames + 1]: first region of each (alignment, frame) unit
     float *phylo = nullptr, *anc = nullptr, *bls = nullptr;   // [nreg]; phylo if fit, anc / bls if asked for, else null
-    pcsf_region *rec = nullptr;                               // room for max(nreg, n_aln) records
+    pcsf_region *rec = nullptr;                               // room for max(nreg, unit alignments) records
 };
 
-// The scoring path of both entry points: stage and pack the batch, enumerate its regions, score every region as an item of the
+// The scoring path of all three entry points: stage and pack the batch, enumerate its regions, score every region as an item of the
 // dedup + prune (FIXED), MLE or OMEGA machinery, synchronise and check for bad characters.  fit = false skips the likelihoods and
 // computes the BLS only.  ref_row may be null for PCSF_ORF_ASIS, which never reads it.
+// The frames are read from n_units_aln column ranges of the staged batch, [unit_cs[u], unit_cs[u] + unit_len[u]): the alignments
+// themselves (unit_cs = col_start, unit_len = len), or caller-given ranges inside them (pcsf_score_given_regions, frame +1 as is).
 static pcsf_status score_regions_core(pcsf_model *m, pcsf_strategy strategy, int32_t n_aln, const uint8_t *seqs, const int64_t *offset,
-                                      const int64_t *len, const int64_t *col_start, int64_t Ltot, const int32_t *ref_row, int32_t frames,
-                                      pcsf_orf_mode orf, int32_t min_codons, bool fit, bool want_anc, bool want_bls, ScoredRegions *out) {
+                                      const int64_t *len, const int64_t *col_start, int64_t Ltot, int32_t n_units_aln, const int64_t *unit_cs,
+                                      const int64_t *unit_len, const int32_t *ref_row, int32_t frames, pcsf_orf_mode orf, int32_t min_codons,
+                                      bool fit, bool want_anc, bool want_bls, ScoredRegions *out) {
     const int nl = m->host.nl;
     cudaStream_t st = m->own_stream;
     pcsf_status rc;
     if ((rc = stage_and_pack(m, n_aln, seqs, offset, len, col_start, Ltot, st))) return rc;
 
     // per-unit buffers: col_start | len | ref_row | totals | n_reg | n_win | bsums x 2 | off_r | off_w
-    const int64_t n_units = (int64_t)n_aln * frames;
+    const int64_t n_units = (int64_t)n_units_aln * frames;
     const uint32_t nsb = (uint32_t)((n_units + SCAN_BLOCK - 1) / SCAN_BLOCK);
     size_t o = 0;
     auto take = [&](size_t bytes) { const size_t r = o; o += (bytes + 255) / 256 * 256; return r; };
-    const size_t o_cs = take((size_t)n_aln * 8), o_len = take((size_t)n_aln * 8), o_ref = take((size_t)n_aln * 4), o_tot = take(16),
+    const size_t o_cs = take((size_t)n_units_aln * 8), o_len = take((size_t)n_units_aln * 8), o_ref = take((size_t)n_units_aln * 4), o_tot = take(16),
                  o_nr = take((size_t)n_units * 4), o_nw = take((size_t)n_units * 4), o_br = take((size_t)(nsb + 1) * 4),
                  o_bw = take((size_t)(nsb + 1) * 4), o_or = take((size_t)(n_units + 1) * 8), o_ow = take((size_t)(n_units + 1) * 8);
     CK(m->rg_units.reserve(o));
     unsigned char *ub = m->rg_units.as<unsigned char>();
-    CK(cudaMemcpyAsync(ub + o_cs, col_start, (size_t)n_aln * 8, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(ub + o_len, len, (size_t)n_aln * 8, cudaMemcpyHostToDevice, st));
-    if (ref_row) CK(cudaMemcpyAsync(ub + o_ref, ref_row, (size_t)n_aln * 4, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(ub + o_cs, unit_cs, (size_t)n_units_aln * 8, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(ub + o_len, unit_len, (size_t)n_units_aln * 8, cudaMemcpyHostToDevice, st));
+    if (ref_row) CK(cudaMemcpyAsync(ub + o_ref, ref_row, (size_t)n_units_aln * 4, cudaMemcpyHostToDevice, st));
     CK(cudaMemsetAsync(ub + o_tot, 0, 16, st));
     unsigned long long *d_tot = reinterpret_cast<unsigned long long *>(ub + o_tot);
     uint32_t *d_nr = reinterpret_cast<uint32_t *>(ub + o_nr), *d_nw = reinterpret_cast<uint32_t *>(ub + o_nw);
     uint32_t *d_br = reinterpret_cast<uint32_t *>(ub + o_br), *d_bw = reinterpret_cast<uint32_t *>(ub + o_bw);
     int64_t *d_or = reinterpret_cast<int64_t *>(ub + o_or), *d_ow = reinterpret_cast<int64_t *>(ub + o_ow);
-    RegionUnits U{m->codes.as<uint8_t>(), m->codes_ld, n_aln, frames, (int)orf, min_codons, reinterpret_cast<const int64_t *>(ub + o_cs),
+    RegionUnits U{m->codes.as<uint8_t>(), m->codes_ld, n_units_aln, frames, (int)orf, min_codons, reinterpret_cast<const int64_t *>(ub + o_cs),
                   reinterpret_cast<const int64_t *>(ub + o_len), ref_row ? reinterpret_cast<const int32_t *>(ub + o_ref) : nullptr};
     const unsigned warp_blocks = (unsigned)((n_units * 32 + 255) / 256);
     {
@@ -790,7 +793,7 @@ static pcsf_status score_regions_core(pcsf_model *m, pcsf_strategy strategy, int
     const size_t nr1 = (size_t)std::max<int64_t>(nreg, 1);
     const size_t o_ra = take(nr1 * 4), o_rf = take(nr1 * 4), o_rk = take(nr1 * 8), o_rn = take(nr1 * 8), o_rw = take(nr1 * 8),
                  o_rl = take(nr1 * 8), o_ph = take(nr1 * 4), o_an = take(nr1 * 4), o_bl = take(nr1 * 4),
-                 o_rec = take((size_t)std::max<int64_t>({nreg, n_aln, 1}) * sizeof(pcsf_region));
+                 o_rec = take((size_t)std::max<int64_t>({nreg, n_units_aln, 1}) * sizeof(pcsf_region));
     CK(m->rg_regions.reserve(o));
     unsigned char *rb = m->rg_regions.as<unsigned char>();
     RegionList R{reinterpret_cast<int32_t *>(rb + o_ra), reinterpret_cast<int32_t *>(rb + o_rf), reinterpret_cast<int64_t *>(rb + o_rk),
@@ -892,8 +895,8 @@ extern "C" pcsf_status pcsf_score_msa(pcsf_model *m, pcsf_strategy strategy, int
     // Frame +1 as is: region i is alignment i.  With nothing but the branch length score asked for, the reference does not call run()
     // at all (score_msa.hpp:112), whatever the strategy — no fit, and no way for a failing fit to turn the batch into an error.
     ScoredRegions r;
-    pcsf_status rc = score_regions_core(m, strategy, n_aln, seqs, offset, len, col_start.data(), Ltot, nullptr, 1, PCSF_ORF_ASIS, 1,
-                                        phylo || anc, anc && strategy != PCSF_STRATEGY_OMEGA, bls != nullptr, &r);
+    pcsf_status rc = score_regions_core(m, strategy, n_aln, seqs, offset, len, col_start.data(), Ltot, n_aln, col_start.data(), len, nullptr,
+                                        1, PCSF_ORF_ASIS, 1, phylo || anc, anc && strategy != PCSF_STRATEGY_OMEGA, bls != nullptr, &r);
     if (rc) return rc;
     if (phylo) CK(cudaMemcpy(phylo, r.phylo, (size_t)n_aln * 4, cudaMemcpyDeviceToHost));
     if (anc && strategy == PCSF_STRATEGY_OMEGA) { for (int i = 0; i < n_aln; ++i) anc[i] = nanf(""); }
@@ -932,8 +935,8 @@ extern "C" pcsf_status pcsf_score_regions(pcsf_model *m, pcsf_strategy strategy,
     CK(cudaSetDevice(m->device));
     if (n_aln == 0) return PCSF_OK;
     ScoredRegions r;
-    pcsf_status rc = score_regions_core(m, strategy, n_aln, seqs, offset, len, col_start.data(), Ltot, ref_row, frames, orf, min_codons,
-                                        true, want_anc != 0, want_bls != 0, &r);
+    pcsf_status rc = score_regions_core(m, strategy, n_aln, seqs, offset, len, col_start.data(), Ltot, n_aln, col_start.data(), len, ref_row,
+                                        frames, orf, min_codons, true, want_anc != 0, want_bls != 0, &r);
     if (rc) return rc;
     cudaStream_t st = m->own_stream;
     const int64_t n_out = best_only ? n_aln : r.nreg;
@@ -948,6 +951,51 @@ extern "C" pcsf_status pcsf_score_regions(pcsf_model *m, pcsf_strategy strategy,
     if (n_out > 0) CK(cudaMemcpyAsync(m->regions.data(), r.rec, (size_t)n_out * sizeof(pcsf_region), cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
     *n_regions = n_out;
+    return PCSF_OK;
+}
+
+// Each range is a frame +1 "as is" unit of its own over its columns of the staged batch: it reads exactly the columns, windows and
+// per-column BLS that pcsf_score_msa reads for the extracted sub-alignment, and its sums run in the same order.
+extern "C" pcsf_status pcsf_score_given_regions(pcsf_model *m, pcsf_strategy strategy, int32_t n_aln, const uint8_t *seqs,
+                                                const int64_t *offset, const int64_t *len, int64_t n_regions, const int32_t *region_aln,
+                                                const int64_t *region_begin, const int64_t *region_end, float *phylo, float *anc, float *bls) {
+    if (!m || n_aln < 0 || n_regions < 0 || (n_aln > 0 && (!seqs || !offset || !len)) ||
+        (n_regions > 0 && (!region_aln || !region_begin || !region_end || !phylo)))
+        return fail(PCSF_ERR_INVALID, "pcsf_score_given_regions: bad argument");
+    if (strategy != PCSF_STRATEGY_FIXED && strategy != PCSF_STRATEGY_MLE && strategy != PCSF_STRATEGY_OMEGA)
+        return fail(PCSF_ERR_INVALID, "pcsf_score_given_regions: unknown strategy");
+    if (n_regions >= ((int64_t)1 << 31)) return fail(PCSF_ERR_INVALID, "too many regions: split the call");
+    std::vector<int64_t> col_start(n_aln);
+    int64_t Ltot = 0, nwin = 0;
+    for (int i = 0; i < n_aln; ++i) {
+        if (len[i] < 0) return fail(PCSF_ERR_INVALID, "negative alignment length");
+        col_start[i] = Ltot;
+        Ltot += len[i] + 2;
+    }
+    std::vector<int64_t> unit_cs((size_t)n_regions), unit_len((size_t)n_regions);
+    for (int64_t r = 0; r < n_regions; ++r) {
+        const int32_t a = region_aln[r];
+        if (a < 0 || a >= n_aln) return fail(PCSF_ERR_INVALID, "pcsf_score_given_regions: region " + std::to_string(r) + ": no alignment " + std::to_string(a));
+        if (region_begin[r] < 0 || region_begin[r] > region_end[r] || region_end[r] > len[a])
+            return fail(PCSF_ERR_INVALID, "pcsf_score_given_regions: region " + std::to_string(r) + ": [" + std::to_string(region_begin[r]) + ", " +
+                                              std::to_string(region_end[r]) + ") is not a column range of an alignment of " + std::to_string(len[a]) + " columns");
+        unit_cs[(size_t)r] = col_start[a] + region_begin[r];
+        unit_len[(size_t)r] = region_end[r] - region_begin[r];
+        nwin += unit_len[(size_t)r] / 3;
+    }
+    if (Ltot >= ((int64_t)1 << 32) || nwin >= ((int64_t)1 << 31)) return fail(PCSF_ERR_INVALID, "batch too large: split the call");
+    NvtxRange nvtx_("pcsf_score_given_regions");
+    CK(cudaSetDevice(m->device));
+    if (n_regions == 0) return PCSF_OK;
+    ScoredRegions r;
+    pcsf_status rc = score_regions_core(m, strategy, n_aln, seqs, offset, len, col_start.data(), Ltot, (int32_t)n_regions, unit_cs.data(),
+                                        unit_len.data(), nullptr, 1, PCSF_ORF_ASIS, 1, true, anc && strategy != PCSF_STRATEGY_OMEGA,
+                                        bls != nullptr, &r);
+    if (rc) return rc;
+    CK(cudaMemcpy(phylo, r.phylo, (size_t)n_regions * 4, cudaMemcpyDeviceToHost));
+    if (anc && strategy == PCSF_STRATEGY_OMEGA) { for (int64_t i = 0; i < n_regions; ++i) anc[i] = nanf(""); }
+    else if (anc) CK(cudaMemcpy(anc, r.anc, (size_t)n_regions * 4, cudaMemcpyDeviceToHost));
+    if (bls) CK(cudaMemcpy(bls, r.bls, (size_t)n_regions * 4, cudaMemcpyDeviceToHost));
     return PCSF_OK;
 }
 

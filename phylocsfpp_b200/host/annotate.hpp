@@ -28,6 +28,8 @@ enum class Feature { Transcript, Cds, Other };
 struct GffTranscript {
     std::string chr;
     char strand = '.';
+    uint64_t begin = 0, end = 0;                               // of the `transcript` line
+    std::vector<std::pair<uint64_t, uint64_t>> exons;         // `exon` features [begin, end] in file order (their lines stay Other)
     float score = NAN, power = NAN;
     std::vector<CdsEntry> cds;
     std::vector<std::pair<Feature, std::string>> lines;
@@ -44,12 +46,14 @@ public:
         fclose(f);
     }
     size_t size() const { return text_.size(); }
+    bool ends_with_newline() const { return !text_.empty() && text_.back() == '\n'; }
     size_t pos() const { return pos_; }
 
     bool next(GffTranscript &t) {
         if (pos_ >= text_.size()) return false;
         int transcripts = 0;
         t.cds.clear();
+        t.exons.clear();
         t.lines.clear();
         while (pos_ < text_.size()) {
             size_t le = text_.find('\n', pos_);
@@ -79,9 +83,13 @@ public:
                 f = Feature::Transcript;
                 t.chr = chr;
                 t.strand = strand;
+                t.begin = begin;
+                t.end = end;
             } else if (feature == "CDS") {
                 f = Feature::Cds;
                 t.cds.push_back(CdsEntry{begin, end, (uint8_t)(phase - '0')});
+            } else if (feature == "exon") {
+                t.exons.emplace_back(begin, end);
             }
             t.lines.emplace_back(f, text_.substr(pos_, le - pos_));
             pos_ = le + 1;

@@ -102,7 +102,10 @@ public:
         int ref_id = -1;
     };
 
-    MafFile(const std::string &path, const Model &model, bool concatenate, int threads) : model_(model), concatenate_(concatenate) {
+    // minus_ref (with concatenate): a chain whose reference row is on '-' is kept as a chain of strand '-' instead of stopping the
+    // program, for callers that skip such chains (annotate-with-maf); a block on the other strand than its chain starts a new chain.
+    MafFile(const std::string &path, const Model &model, bool concatenate, int threads, bool minus_ref = false)
+        : model_(model), concatenate_(concatenate), minus_ref_(minus_ref) {
         fd_ = open(path.c_str(), O_RDONLY);
         if (fd_ < 0) die("Cannot open %s", path.c_str());
         size_ = (size_t)lseek(fd_, 0, SEEK_END);
@@ -421,7 +424,7 @@ private:
                     if (!first_block) {
                         for (const PreLine &pl : b.pre)
                             if (!contiguous(pl.start0, pl.chrom, pl.chrom_len)) { aborted = true; break; }
-                        if (!aborted && b.has_ref && !contiguous(b.start0, b.chrom, b.chrom_len)) aborted = true;
+                        if (!aborted && b.has_ref && (!contiguous(b.start0, b.chrom, b.chrom_len) || (minus_ref_ && b.strand != c.strand))) aborted = true;
                     }
                     if (aborted) {
                         abort_next = true;
@@ -431,7 +434,7 @@ private:
                             c.start_pos = b.start0 + 1; c.chrom.assign(b.chrom, (size_t)b.chrom_len); c.chrom_len = b.src_size; c.strand = b.strand;
                             c.ref_id = b.ref_id;
                             prev_cum = b.size;
-                            if (b.strand != '+' && concatenate_) die("Reference sequence is not on the + strand (%s at position %ld)!", who.c_str(), (long)b.start0);
+                            if (b.strand != '+' && concatenate_ && !minus_ref_) die("Reference sequence is not on the + strand (%s at position %ld)!", who.c_str(), (long)b.start0);
                             const int64_t prev_end = c.start_pos, new_end = c.start_pos + b.size;
                             if (!reached_bp && prev_end / BREAKPOINT_POS < new_end / BREAKPOINT_POS) { reached_bp = true; cum_after_bp = prev_cum; }
                         } else if (!first_block) {
@@ -440,7 +443,7 @@ private:
                             if (!reached_bp && prev_end / BREAKPOINT_POS < new_end / BREAKPOINT_POS) { reached_bp = true; cum_after_bp = prev_cum; }
                             if (c.ref_id != (int)b.ref_id)
                                 die("Encountered an alignment block that didn't start with the reference species: %s at position %ld!", who.c_str(), (long)b.start0);
-                            if (b.strand != '+' && concatenate_) die("Reference sequence is not on the + strand (%s at position %ld)!", who.c_str(), (long)b.start0);
+                            if (b.strand != '+' && concatenate_ && !minus_ref_) die("Reference sequence is not on the + strand (%s at position %ld)!", who.c_str(), (long)b.start0);
                         }
                         c.blocks.push_back(bi);
                     } else {
@@ -459,7 +462,7 @@ private:
     }
 
     const Model &model_;
-    bool concatenate_;
+    bool concatenate_, minus_ref_;
     int fd_ = -1;
     size_t size_ = 0;
     const char *mem_ = nullptr;

@@ -19,6 +19,7 @@
 #include "annotate.hpp"
 #include "hmm.hpp"
 #include "maf.hpp"
+#include "transcripts.hpp"
 
 using namespace host;
 
@@ -944,6 +945,250 @@ int main_annotate_with_tracks(int argc, char **argv) {
     return 0;
 }
 
+// annotate-with-maf: PhyloCSF scores of the CDS (and of the coding transcripts as a whole) of GFF/GTF files, from spliced alignments
+// cut out of whole-genome MAF files (transcripts.hpp); with --find-orf 1, the best ATG-to-stop ORF of every transcript without CDS.
+// Every input line is copied; transcript and CDS lines get attributes in the file's syntax.  Batches of transcripts are scored by
+// score-msa's worker pattern (one device model per worker, thread t on GPU t mod --gpus) and written in file order.
+int main_annotate_with_maf(int argc, char **argv) {
+    const Args a = parse_args(argc, argv, {"output", "strategy", "comp-anc", "find-orf", "min-codons", "species", "mapping", "threads", "gpus"});
+    if (a.pos.size() < 3)
+        die("usage: phylocsf_b200 annotate-with-maf [OPTIONS] <model> <alignments.maf[,more.maf...]> <gff/gtf files>...");
+    const std::string strat = lower(a.str("strategy", "mle"));
+    pcsf_strategy strategy;
+    if (strat == "mle") strategy = PCSF_STRATEGY_MLE;
+    else if (strat == "fixed") strategy = PCSF_STRATEGY_FIXED;
+    else if (strat == "omega") strategy = PCSF_STRATEGY_OMEGA;
+    else { printf("\033[31mPlease choose a valid strategy (MLE, FIXED or OMEGA)!\n\033[0m"); return -1; }
+    const bool comp_anc = a.boolean("comp-anc", false), find_orf = a.boolean("find-orf", false);
+    if (strategy == PCSF_STRATEGY_OMEGA && comp_anc) {
+        printf("\033[31mThe ancestral sequence composition cannot be computed in the Omega mode!\n\033[0m");
+        return -1;
+    }
+    const std::string mc = a.str("min-codons", "25");
+    char *mc_end = nullptr;
+    const long min_codons = strtol(mc.c_str(), &mc_end, 10);
+    if (mc.empty() || *mc_end || min_codons < 1 || min_codons > INT32_MAX) {
+        printf("\033[31m--min-codons must be an integer >= 1!\n\033[0m");
+        return -1;
+    }
+    const int threads = std::max(1, a.integer("threads", (int)std::thread::hardware_concurrency()));
+    const int gpus = std::max(1, a.integer("gpus", default_gpus()));
+    const int workers_n = std::min(threads, 2 * gpus);
+    Model model;
+    load_model(model, a.pos[0], a.str("species"), a.str("mapping"));
+    const auto t_start = std::chrono::steady_clock::now();
+    auto since = [](std::chrono::steady_clock::time_point t) { return std::chrono::duration<double>(std::chrono::steady_clock::now() - t).count(); };
+    std::vector<pcsf_model *> dev(workers_n);
+    std::thread model_maker([&] {
+        std::vector<std::thread> th;
+        for (int t = 0; t < workers_n; ++t) th.emplace_back([&, t] { dev[t] = create_device_model(model, t % gpus); });
+        for (auto &x : th) x.join();
+    });
+    const ChainIndex idx(split(a.pos[1], ','), model, threads);
+    for (const auto &maf : idx.mafs()) warn_unresolved(*maf);
+    if (idx.minus_chains())
+        printf("\033[33mWARNING: %" PRId64 " alignment chains with the reference on the '-' strand are not used.\033[0m\n", idx.minus_chains());
+    const double t_scan = since(t_start);
+
+    struct GffFile { std::string out_path; bool newline_at_end; std::vector<GffTranscript> recs; };
+    std::vector<GffFile> files;
+    const std::string out_dir = a.str("output");
+    if (!out_dir.empty()) create_directory(out_dir);
+    for (size_t i = 2; i < a.pos.size(); ++i) {
+        const std::string &path = a.pos[i];
+        const size_t slash = path.find_last_of('/');
+        std::string out = out_dir.empty() ? path : out_dir + "/" + (slash == std::string::npos ? path : path.substr(slash + 1));
+        const size_t dot = out.find_last_of('.');
+        if (dot == std::string::npos || (out.find_last_of('/') != std::string::npos && dot < out.find_last_of('/'))) out += ".PhyloCSF++maf";
+        else out.insert(dot, ".PhyloCSF++maf");
+        GffReader reader(path);
+        GffFile f{out, reader.ends_with_newline(), {}};
+        GffTranscript t;
+        while (reader.next(t)) f.recs.push_back(t);
+        files.push_back(std::move(f));
+    }
+    struct Batch { size_t file, r0, r1; };
+    const size_t BATCH = getenv("PCSF_HOST_MAF_BATCH") ? std::max<size_t>(1, (size_t)atoll(getenv("PCSF_HOST_MAF_BATCH"))) : 4096;
+    std::vector<Batch> batches;
+    for (size_t fi = 0; fi < files.size(); ++fi)
+        for (size_t r0 = 0; r0 < files[fi].recs.size(); r0 += BATCH) batches.push_back(Batch{fi, r0, std::min(files[fi].recs.size(), r0 + BATCH)});
+    const double t_read = since(t_start) - t_scan;
+    model_maker.join();
+
+    OrderedSink sink;
+    sink.resize(batches.size());
+    std::atomic<size_t> next{0};
+    std::mutex stat_mu;
+    double t_extract = 0.0, t_gpu = 0.0, t_format = 0.0;
+    int64_t n_coding = 0, n_orf = 0;
+    std::vector<std::thread> workers;
+    for (int w = 0; w < workers_n; ++w)
+        workers.emplace_back([&, w] {
+            ChainCache cache(idx);
+            for (size_t bi = next++; bi < batches.size(); bi = next++) {
+                const Batch &bt = batches[bi];
+                const std::vector<GffTranscript> &recs = files[bt.file].recs;
+                const auto p0 = std::chrono::steady_clock::now();
+                // coding transcripts: one alignment each, its regions through pcsf_score_given_regions; the others (--find-orf 1): one
+                // alignment each through pcsf_score_regions, best ATG-to-stop ORF of frames +1..+3
+                std::vector<TxAlignment> tx(bt.r1 - bt.r0);
+                std::vector<char> scored(tx.size(), 0);
+                std::vector<uint8_t> cblob, oblob;
+                std::vector<int64_t> coff, clen, ooff, olen, rbeg, rend;
+                std::vector<int32_t> raln, oref;
+                std::vector<int64_t> first_region(tx.size(), -1), orf_index(tx.size(), -1);
+                // extracted in genomic order: the transcripts of a batch then share the chains the cache holds, however the file is sorted
+                std::vector<size_t> by_pos(tx.size());
+                for (size_t k = 0; k < tx.size(); ++k) by_pos[k] = k;
+                std::stable_sort(by_pos.begin(), by_pos.end(), [&](size_t i, size_t j) {
+                    const GffTranscript &a = recs[bt.r0 + i], &b = recs[bt.r0 + j];
+                    return a.chr != b.chr ? a.chr < b.chr : a.begin < b.begin;
+                });
+                for (size_t k : by_pos) {
+                    TxAlignment &x = tx[k];
+                    if (!extract_transcript(idx, cache, recs[bt.r0 + k], find_orf, x)) continue;
+                    scored[k] = 1;
+                    if (x.coding) {
+                        first_region[k] = (int64_t)rbeg.size();
+                        for (size_t r = 0; r < x.reg_begin.size(); ++r) {
+                            raln.push_back((int32_t)coff.size()); rbeg.push_back(x.reg_begin[r]); rend.push_back(x.reg_end[r]);
+                        }
+                        coff.push_back((int64_t)cblob.size()); clen.push_back(x.L);
+                        cblob.insert(cblob.end(), x.seqs.begin(), x.seqs.end());
+                    } else if (x.ref_row >= 0) {
+                        orf_index[k] = (int64_t)ooff.size();
+                        ooff.push_back((int64_t)oblob.size()); olen.push_back(x.L); oref.push_back(x.ref_row);
+                        oblob.insert(oblob.end(), x.seqs.begin(), x.seqs.end());
+                    }
+                    std::vector<uint8_t>().swap(x.seqs);
+                }
+                const double my_extract = since(p0);
+                const auto g0 = std::chrono::steady_clock::now();
+                const int64_t nr = (int64_t)rbeg.size();
+                std::vector<float> phylo(nr, NAN), anc(nr, NAN), bls(nr, NAN);
+                if (nr > 0) {
+                    const pcsf_status st = pcsf_score_given_regions(dev[w], strategy, (int32_t)coff.size(), cblob.data(), coff.data(), clen.data(), nr,
+                                                                    raln.data(), rbeg.data(), rend.data(), phylo.data(), comp_anc ? anc.data() : nullptr,
+                                                                    bls.data());
+                    if (st == PCSF_ERR_BAD_CHAR) { fprintf(stderr, "%s\n", pcsf_last_error()); exit(37); }
+                    if (st != PCSF_OK) die("pcsf_score_given_regions: %s", pcsf_last_error());
+                }
+                std::vector<pcsf_region> orfs(ooff.size());
+                if (!ooff.empty()) {
+                    int64_t n = 0;
+                    pcsf_status st = pcsf_score_regions(dev[w], strategy, (int32_t)ooff.size(), oblob.data(), ooff.data(), olen.data(), oref.data(), 3,
+                                                        PCSF_ORF_ATGSTOP, (int32_t)min_codons, 1, 0, 1, &n);
+                    if (st == PCSF_ERR_BAD_CHAR) { fprintf(stderr, "%s\n", pcsf_last_error()); exit(37); }
+                    if (st != PCSF_OK) die("pcsf_score_regions: %s", pcsf_last_error());
+                    if ((st = pcsf_score_regions_get(dev[w], orfs.data(), n)) != PCSF_OK) die("pcsf_score_regions_get: %s", pcsf_last_error());
+                }
+                const double my_gpu = since(g0);
+                const auto f0 = std::chrono::steady_clock::now();
+                std::string text;
+                char v[160];
+                auto attr = [&](bool gff, const char *key, const char *val) {
+                    if (gff) snprintf(v, sizeof v, ";%s=%s", key, val);
+                    else snprintf(v, sizeof v, " %s \"%s\";", key, val);
+                    text += v;
+                };
+                auto num = [](char *buf, size_t n, float f) { snprintf(buf, n, "%.6f", std::isnan(f) ? NAN : f); };
+                for (size_t k = 0; k < tx.size(); ++k) {
+                    const GffTranscript &t = recs[bt.r0 + k];
+                    const TxAlignment &x = tx[k];
+                    bool first = true, gff = true;
+                    size_t cds_id = 0;
+                    for (const auto &ln : t.lines) {
+                        text += ln.second;
+                        const bool tx_line = ln.first == Feature::Transcript;
+                        if (scored[k] && (tx_line || (x.coding && ln.first == Feature::Cds))) {
+                            if (first) { first = false; gff = is_gff_line(ln.second); }
+                            char s[64];
+                            if (x.coding) {
+                                const int64_t r = first_region[k] + (tx_line ? 0 : (int64_t)(1 + cds_id++));
+                                num(s, sizeof s, phylo[r]); attr(gff, "phylocsf_score", s);
+                                if (comp_anc) { num(s, sizeof s, anc[r]); attr(gff, "phylocsf_anc", s); }
+                                num(s, sizeof s, bls[r]); attr(gff, "phylocsf_bls", s);
+                                snprintf(s, sizeof s, "%" PRId64, (rend[r] - rbeg[r]) / 3); attr(gff, "phylocsf_codons", s);
+                            } else {
+                                const pcsf_region *o = orf_index[k] >= 0 ? &orfs[(size_t)orf_index[k]] : nullptr;
+                                const bool found = o && o->frame != 0;
+                                num(s, sizeof s, found ? o->phylo : NAN); attr(gff, "phylocsf_orf_score", s);
+                                if (found) {
+                                    const uint64_t g0p = genomic_position(x, o->col_begin), g1p = genomic_position(x, o->col_end - 1);
+                                    snprintf(s, sizeof s, "%" PRIu64, std::min(g0p, g1p)); attr(gff, "phylocsf_orf_start", s);
+                                    snprintf(s, sizeof s, "%" PRIu64, std::max(g0p, g1p)); attr(gff, "phylocsf_orf_end", s);
+                                    snprintf(s, sizeof s, "%" PRId64, o->codons); attr(gff, "phylocsf_orf_codons", s);
+                                } else {
+                                    attr(gff, "phylocsf_orf_start", "."); attr(gff, "phylocsf_orf_end", "."); attr(gff, "phylocsf_orf_codons", ".");
+                                }
+                                num(s, sizeof s, found ? o->bls : NAN); attr(gff, "phylocsf_orf_bls", s);
+                            }
+                        }
+                        text += '\n';
+                    }
+                }
+                std::vector<std::string> one(1);
+                one[0] = std::move(text);
+                sink.put(bi, std::move(one));
+                std::lock_guard<std::mutex> g(stat_mu);
+                t_extract += my_extract; t_gpu += my_gpu; t_format += since(f0);
+                n_coding += (int64_t)coff.size(); n_orf += (int64_t)ooff.size();
+            }
+        });
+    double t_write = 0.0;
+    size_t bi = 0;
+    for (const GffFile &f : files) {
+        FILE *fo = fopen(f.out_path.c_str(), "w");
+        if (!fo) die("Error creating file %s!", f.out_path.c_str());
+        for (; bi < batches.size() && batches[bi].file == (size_t)(&f - files.data()); ++bi) {
+            std::string text = sink.take(bi)[0];
+            const auto w0 = std::chrono::steady_clock::now();
+            if (batches[bi].r1 == f.recs.size() && !f.newline_at_end && !text.empty()) text.pop_back();          // the input's last line had none
+            fwrite(text.data(), 1, text.size(), fo);
+            t_write += since(w0);
+        }
+        fclose(fo);
+    }
+    for (auto &w : workers) w.join();
+    printf("\33[2K\rDone!\n");
+    if (getenv("PCSF_HOST_STATS"))
+        printf("{\"transcripts\": %" PRId64 ", \"coding\": %" PRId64 ", \"orf_searched\": %" PRId64 ", \"seconds\": %.3f, \"scan_seconds\": %.3f, "
+               "\"gff_read_seconds\": %.3f, \"extract_seconds_sum\": %.3f, \"gpu_call_seconds_sum\": %.3f, \"format_seconds_sum\": %.3f, "
+               "\"write_seconds\": %.3f, \"workers\": %d}\n",
+               n_coding + n_orf, n_coding, n_orf, since(t_start), t_scan, t_read, t_extract, t_gpu, t_format, t_write, workers_n);
+    for (pcsf_model *m : dev) pcsf_model_destroy(m);
+    return 0;
+}
+
+// Test hook (no GPU needed): the alignments annotate-with-maf scores.  One line per coding transcript and per CDS region, and one per
+// transcript without CDS (its exon alignment and the reference row of its chains): file, record, kind, columns, region, FNV-1a hash.
+int main_dump_transcripts(int argc, char **argv) {
+    const Args a = parse_args(argc, argv, {"threads", "mapping", "species"});
+    if (a.pos.size() < 3) die("usage: phylocsf_b200 dump-transcripts [--threads INT] <model> <alignments.maf[,more.maf...]> <gff/gtf files>...");
+    Model model;
+    load_model(model, a.pos[0], a.str("species"), a.str("mapping"));
+    const int nl = model.nl();
+    const ChainIndex idx(split(a.pos[1], ','), model, std::max(1, a.integer("threads", 4)));
+    printf("# minus_chains %" PRId64 "\n", idx.minus_chains());
+    ChainCache cache(idx);
+    for (size_t fi = 2; fi < a.pos.size(); ++fi) {
+        GffReader reader(a.pos[fi]);
+        GffTranscript t;
+        TxAlignment x;
+        for (size_t rec = 0; reader.next(t); ++rec) {
+            if (!extract_transcript(idx, cache, t, true, x)) continue;
+            if (!x.coding) {
+                printf("%zu\t%zu\texons\t%" PRId64 "\t0\t%" PRId64 "\t%016" PRIx64 "\t%d\n", fi - 2, rec, x.L, x.L, region_hash(x, nl, 0, x.L), x.ref_row);
+                continue;
+            }
+            for (size_t r = 0; r < x.reg_begin.size(); ++r)
+                printf("%zu\t%zu\t%s\t%" PRId64 "\t%" PRId64 "\t%" PRId64 "\t%016" PRIx64 "\t.\n", fi - 2, rec, r == 0 ? "transcript" : "CDS", x.L,
+                       x.reg_begin[r], x.reg_end[r], region_hash(x, nl, x.reg_begin[r], x.reg_end[r]));
+        }
+    }
+    return 0;
+}
+
 // wig-to-bigwig: the step the reference leaves to UCSC's wigToBigWig (README: "wigToBigWig PhyloCSF+1.wig chrom.sizes PhyloCSF+1.bw").
 int main_wig_to_bigwig(int argc, char **argv) {
     const Args a = parse_args(argc, argv, {"compress"});
@@ -1082,6 +1327,8 @@ int main(int argc, char **argv) {
                "                             [--frames 1|3|6] [--orf AsIs|StopStop|ATGStop] [--min-codons INT] [--all-scores BOOL]\n"
                "                             [--output DIR] [--mapping FILE] [--species LIST] <model> <maf>...\n"
                "  phylocsf_b200 annotate-with-tracks [--output DIR] <PhyloCSF+1.bw> <gff/gtf>...\n"
+               "  phylocsf_b200 annotate-with-maf [--output DIR] [--strategy MLE|FIXED|OMEGA] [--comp-anc BOOL] [--find-orf BOOL] [--min-codons INT]\n"
+               "                             [--species LIST] [--mapping FILE] [--threads INT] [--gpus INT] <model> <maf[,maf...]> <gff/gtf>...\n"
                "  phylocsf_b200 wig-to-bigwig [--compress BOOL] <in.wig> <chrom.sizes> <out.bw>\n");
         return argc < 2 ? 1 : 0;
     }
@@ -1094,7 +1341,9 @@ int main(int argc, char **argv) {
     if (tool == "matrix-to-maf") return main_matrix_to_maf(argc, argv);
     if (tool == "parse-bench") return main_parse_bench(argc, argv);
     if (tool == "annotate-with-tracks") return main_annotate_with_tracks(argc, argv);
+    if (tool == "annotate-with-maf") return main_annotate_with_maf(argc, argv);
+    if (tool == "dump-transcripts") return main_dump_transcripts(argc, argv);
     if (tool == "wig-to-bigwig") return main_wig_to_bigwig(argc, argv);
     if (tool == "bigwig-dump") return main_bigwig_dump(argc, argv);
-    die("unknown tool '%s' (build-tracks, score-msa, annotate-with-tracks and wig-to-bigwig are available)", tool.c_str());
+    die("unknown tool '%s' (build-tracks, score-msa, annotate-with-tracks, annotate-with-maf and wig-to-bigwig are available)", tool.c_str());
 }

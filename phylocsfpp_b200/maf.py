@@ -51,7 +51,9 @@ def _atoi(tok: bytes) -> int:
 
 class MafReader:
     def __init__(self, path: str, seqid_to_phyloid: Dict[str, int], nl: int, concatenate: bool,
-                 warn=True):
+                 warn=True, minus_ref=False):
+        """minus_ref (with concatenate): a chain whose reference row is on '-' is returned with strand '-' instead of raising, and
+        a block on the other strand than its chain starts a new chain (annotate-with-maf skips such chains)."""
         opener = gzip.open if path.endswith(".gz") else open
         with opener(path, "rb") as fh:
             data = fh.read()
@@ -65,6 +67,7 @@ class MafReader:
         self.unresolved = set()
         self.species_seen = np.zeros(nl, bool)
         self.warn = warn
+        self.minus_ref = minus_ref
         # constructor (:321-343): start at the first "a " line
         self.pos = 0
         while self.pos < self.nlines and not self.lines[self.pos].startswith(b"a "):
@@ -147,7 +150,7 @@ class MafReader:
                     aln.strand = strand
                     ref_seq_id = alnid
                     prev_cum = size
-                    if strand != "+" and not single_block_scoring:
+                    if strand != "+" and not single_block_scoring and not self.minus_ref:
                         raise ValueError(f"Reference sequence is not on the + strand ({species}.{chrom} at position {start0})!")
                     prev_end = aln.start_pos
                     new_end = aln.start_pos + size
@@ -155,6 +158,9 @@ class MafReader:
                         reached_bp = True
                         cum_after_bp = prev_cum
                 elif ref_seq_id_sub == -1 and not first_block:
+                    if self.minus_ref and strand != aln.strand:
+                        abort_next = True
+                        break
                     ref_seq_id_sub = alnid
                     prev_end = aln.start_pos + prev_cum
                     new_end = aln.start_pos + prev_cum + size
@@ -165,7 +171,7 @@ class MafReader:
                     if ref_seq_id != ref_seq_id_sub:
                         raise ValueError(f"Encountered an alignment block that didn't start with the reference species: "
                                          f"{species}.{chrom} at position {start0}!")
-                    if strand != "+" and not single_block_scoring:
+                    if strand != "+" and not single_block_scoring and not self.minus_ref:
                         raise ValueError(f"Reference sequence is not on the + strand ({species}.{chrom} at position {start0})!")
 
                 rows[alnid].append(seq)
