@@ -132,7 +132,10 @@ pcsf_status pcsf_tracks(pcsf_model *m, const uint8_t *seqs, int64_t L, int64_t l
 pcsf_status pcsf_tracks_device(pcsf_model *m, const uint8_t *d_seqs, int64_t L, int64_t ld, uint32_t flags,
                                double *d_plus, double *d_minus, double *d_bls, uint32_t *d_pattern_index,
                                void *cuda_stream);
-/* Synchronises the stream, checks the bad-character flag and fills stats. */
+/* Synchronises the stream, reads and clears the bad-character flag and fills stats.  The flag covers every pcsf_tracks_device call
+ * since the last finish: PCSF_ERR_BAD_CHAR if any of them read a character outside "ACGTacgt.-Nn" in its columns [0, L) (bytes in
+ * [L, ld) are never read).  stats describe the last of those calls.  pcsf_tracks ends with a finish of its own (its flag is cleared
+ * also when it fails); pcsf_score_msa and the region calls have a flag of their own and leave this one alone. */
 pcsf_status pcsf_tracks_device_finish(pcsf_model *m, void *cuda_stream, pcsf_tracks_stats *stats);
 
 /* Maximum number of columns per dedup chunk (default 1<<21); 0 restores the default. */

@@ -99,6 +99,8 @@ struct pcsf_model {
     DevBuf codes, klo, khi, slot, flag, uniq, pidx, table, bsums, logz, anc, io_in, io_out, perwin, mle;
     DevBuf rg_units, rg_regions, rg_win;      // score-msa (both entry points): per-(alignment, frame) counts, region lists, region windows
     std::vector<pcsf_region> regions;         // records of the last pcsf_score_regions call
+    // Bad-character flags, raised by k_pack.  [0]: every pcsf_tracks_device call since the last pcsf_tracks_device_finish, which reads
+    // and clears it (a flag cleared by each call would hide a bad call queued before a good one).  [1]: the score-msa call in flight.
     int *d_bad = nullptr;
     uint32_t *d_nuniq = nullptr;       // [max chunks]
     int64_t chunk_cols = (int64_t)1 << 21;          // 2 Mi columns: calls of 4 Mi columns and more are pipelined (H2D | compute | D2H per chunk)
@@ -214,8 +216,8 @@ extern "C" pcsf_status pcsf_model_create(const pcsf_model_desc *d, int device, p
         std::vector<int32_t> ge(m->host.gemm_edges.begin(), m->host.gemm_edges.end());
         if ((st = upload(ge.data(), ge.size() * 4, (void **)&m->d_gemm_edges))) return st;
     }
-    CK(cudaMalloc(&m->d_bad, sizeof(int)));
-    CK(cudaMemset(m->d_bad, 0, sizeof(int)));
+    CK(cudaMalloc(&m->d_bad, 2 * sizeof(int)));
+    CK(cudaMemset(m->d_bad, 0, 2 * sizeof(int)));
     if (!getenv("PCSF_LEGACY_STREAM")) {
         CK(cudaStreamCreateWithFlags(&m->own_stream, cudaStreamNonBlocking));
         CK(cudaStreamCreateWithFlags(&m->copy_stream, cudaStreamNonBlocking));
@@ -427,16 +429,16 @@ static pcsf_status dedup_and_prune(pcsf_model *m, const WinSpace &ws, uint32_t n
     return PCSF_OK;
 }
 
-static pcsf_status run_pack(pcsf_model *m, const uint8_t *d_seqs, int64_t L, int64_t ld, cudaStream_t st) {
+// k_pack raises *d_bad (m->d_bad or m->d_bad + 1) on a character outside the alphabet; it never lowers it.
+static pcsf_status run_pack(pcsf_model *m, const uint8_t *d_seqs, int64_t L, int64_t ld, int *d_bad, cudaStream_t st) {
     const int nl = m->host.nl;
     m->codes_ld = ((L + 16 + 15) / 16) * 16;
     CK(m->codes.reserve((size_t)m->codes_ld * nl));
-    CK(cudaMemsetAsync(m->d_bad, 0, sizeof(int), st));
     const int64_t nvec = m->codes_ld / 16;
     // a few fat blocks per SM with grid-stride loops (four vectors in flight per thread) instead of one block per 4 KB of a row
     dim3 grid((unsigned)std::max<int64_t>(1, std::min<int64_t>((nvec + 255) / 256, ((int64_t)m->sm_count * 16 + nl - 1) / nl)), nl);
     NvtxRange nvtx_("pcsf: pack");
-    m->launches++; k_pack<<<grid, 256, 0, st>>>(d_seqs, L, ld, nl, m->codes.as<uint8_t>(), m->codes_ld, m->codes_ld, m->d_bad);
+    m->launches++; k_pack<<<grid, 256, 0, st>>>(d_seqs, L, ld, nl, m->codes.as<uint8_t>(), m->codes_ld, m->codes_ld, d_bad);
     CK(cudaGetLastError());
     return PCSF_OK;
 }
@@ -510,12 +512,13 @@ extern "C" pcsf_status pcsf_tracks_device(pcsf_model *m, const uint8_t *d_seqs, 
         const int64_t c1 = std::min(W_all, (c + 1) * m->chunk_cols);
         return std::min<int64_t>(L, ((c1 + 2 + 15) / 16) * 16);
     };
+    // refused before any work is queued: nothing of a refused call reaches the bad-character flag
+    if ((flags & PCSF_TRACKS_SCORES) && nchunks_all > MAX_CHUNKS) return fail(PCSF_ERR_INVALID, "too many chunks; raise pcsf_set_chunk_columns");
     NvtxRange nvtx_("pcsf_tracks_device");
     if (seg) {
         NvtxRange nvtx_h2d("pcsf: H2D segments");
         m->codes_ld = ((L + 16 + 15) / 16) * 16;
         CK(m->codes.reserve((size_t)m->codes_ld * m->host.nl));
-        CK(cudaMemsetAsync(m->d_bad, 0, sizeof(int), st));
         while ((int64_t)m->ev_h2d.size() < nchunks_all) {
             cudaEvent_t e;
             CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
@@ -530,7 +533,7 @@ extern "C" pcsf_status pcsf_tracks_device(pcsf_model *m, const uint8_t *d_seqs, 
         }
     }
     if (m->timing) CK(cudaEventRecord(m->ev[4], st));
-    if (!seg && (rc = run_pack(m, d_seqs, L, ld, st))) return rc;
+    if (!seg && (rc = run_pack(m, d_seqs, L, ld, m->d_bad, st))) return rc;
     if (m->timing) CK(cudaEventRecord(m->ev[5], st));
     if ((flags & PCSF_TRACKS_BLS) && !seg) {
         if ((rc = run_bls(m, L, 0, d_bls, st))) return rc;
@@ -548,8 +551,7 @@ extern "C" pcsf_status pcsf_tracks_device(pcsf_model *m, const uint8_t *d_seqs, 
     }
     const int64_t W = L - 2;
     if ((flags & PCSF_TRACKS_SCORES) && W > 0) {
-        const int64_t nchunks = (W + m->chunk_cols - 1) / m->chunk_cols;
-        if (nchunks > MAX_CHUNKS) return fail(PCSF_ERR_INVALID, "too many chunks; raise pcsf_set_chunk_columns");
+        const int64_t nchunks = nchunks_all;
         for (int64_t c = 0; c < nchunks; ++c) {
             const int64_t c0 = c * m->chunk_cols, c1 = std::min(W, c0 + m->chunk_cols);
             const uint32_t nwin = (uint32_t)(2 * (c1 - c0));
@@ -608,6 +610,7 @@ extern "C" pcsf_status pcsf_tracks_device_finish(pcsf_model *m, void *cuda_strea
     cudaStream_t st = (cudaStream_t)cuda_stream;
     int bad = 0;
     CK(cudaMemcpyAsync(&bad, m->d_bad, sizeof(int), cudaMemcpyDeviceToHost, st));
+    CK(cudaMemsetAsync(m->d_bad, 0, sizeof(int), st));      // read and cleared in stream order: the next call starts a new batch
     CK(cudaStreamSynchronize(st));
     m->last.n_windows = m->last_nwin;
     m->last.n_chunks = m->last_chunks;
@@ -634,6 +637,13 @@ extern "C" pcsf_status pcsf_tracks(pcsf_model *m, const uint8_t *seqs, int64_t L
     const int nl = m->host.nl;
     const int64_t W = std::max<int64_t>(L - 2, 0);
     const int64_t ldd = ((L + 15) / 16) * 16;
+    // This call ends with its own pcsf_tracks_device_finish, which reads and clears the bad-character flag; a return before that point
+    // clears it here, so that a failed call leaves no stale bad character for the next one to report.
+    struct BadFlagGuard {
+        pcsf_model *m;
+        bool armed = true;
+        ~BadFlagGuard() { if (armed) { cudaMemsetAsync(m->d_bad, 0, sizeof(int), m->own_stream); cudaStreamSynchronize(m->own_stream); } }
+    } bad_guard{m};
     CK(m->io_in.reserve((size_t)ldd * nl));
     const size_t out_bytes = (size_t)W * 16 + (size_t)L * 8 + (pattern_index ? (size_t)W * 8 : 0) + 64;
     CK(m->io_out.reserve(out_bytes));
@@ -666,6 +676,7 @@ extern "C" pcsf_status pcsf_tracks(pcsf_model *m, const uint8_t *seqs, int64_t L
         if (flags & PCSF_TRACKS_BLS) CK(cudaMemcpyAsync(bls, d_bls, (size_t)L * 8, cudaMemcpyDeviceToHost, st));
     }
     rc = pcsf_tracks_device_finish(m, st, stats);
+    bad_guard.armed = false;
     if (piped && cudaStreamSynchronize(m->copy_stream) != cudaSuccess && rc == PCSF_OK) rc = fail(PCSF_ERR_CUDA, "copy stream failed");
     return rc;
 }
@@ -719,7 +730,10 @@ static pcsf_status stage_and_pack(pcsf_model *m, int32_t n_aln, const uint8_t *s
     }
     CK(m->io_in.reserve(h_bytes));
     CK(cudaMemcpyAsync(m->io_in.p, h, h_bytes, cudaMemcpyHostToDevice, st));
-    return run_pack(m, m->io_in.as<uint8_t>(), Ltot, ldd, st);
+    // The score-msa calls are synchronous and own m->d_bad[1] from here to score_regions_core's read: whatever a failed call left in it
+    // goes, and the tracks flag m->d_bad[0] of queued pcsf_tracks_device calls is not touched.
+    CK(cudaMemsetAsync(m->d_bad + 1, 0, sizeof(int), st));
+    return run_pack(m, m->io_in.as<uint8_t>(), Ltot, ldd, m->d_bad + 1, st);
 }
 
 // One scoring path for reading frames / ORFs (pcsf_score_regions); pcsf_score_msa is its frame +1 as is, one region per alignment.
@@ -864,9 +878,10 @@ static pcsf_status score_regions_core(pcsf_model *m, pcsf_strategy strategy, int
             CK(cudaGetLastError());
         }
     }
-    CK(cudaStreamSynchronize(st));
     int bad = 0;
-    CK(cudaMemcpy(&bad, m->d_bad, sizeof(int), cudaMemcpyDeviceToHost));
+    CK(cudaMemcpyAsync(&bad, m->d_bad + 1, sizeof(int), cudaMemcpyDeviceToHost, st));
+    CK(cudaMemsetAsync(m->d_bad + 1, 0, sizeof(int), st));
+    CK(cudaStreamSynchronize(st));
     if (bad) return fail(PCSF_ERR_BAD_CHAR, "alignment contains a character outside ACGTacgt.-Nn (reference: exit(37))");
     *out = ScoredRegions{nreg, U, R, d_or, fit ? d_phylo : nullptr, want_anc ? d_anc : nullptr, want_bls ? d_bls : nullptr,
                          reinterpret_cast<pcsf_region *>(rb + o_rec)};
